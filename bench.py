@@ -57,7 +57,17 @@ def parse():
     ap.add_argument("--gather", default="auto", choices=["auto", "p2p", "nccl"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the sparse/crowd/strong-scaling sub-measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the last timed step's outputs, float32: DIR/rows.npy (world, batch, max_det, 6), slots past "
+                         "an image's count zeroed, and DIR/counts.npy (world, batch), -1 = no candidate.  Above 64 MB a "
+                         "fixed, seeded sample of k images: rows (k, max_det, 6), counts (k,), their flat image indices "
+                         "in DIR/images.npy.  Inputs are seeded: two builds run with the same arguments can be compared "
+                         "output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     cfg = CONFIGS[args.config]
     args.family = args.family or cfg["family"]
     args.img = args.img or cfg["img"]
@@ -78,6 +88,28 @@ def workload_config(args, world, batch=None, dist_name=None):
         "parallelism": f"image-sharded x{world}" + (", kept detections all-gathered (rows stored into every peer's slot by the NMS kernel)" if world > 1 else ""),
         "l2": "inputs per step exceed the 126 MB L2 (548 MB at 64 v5s images) and are streamed once per step",
     }
+
+
+DUMP_CAP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, rows, counts):
+    """Writes what a caller of ShardedPostProcessor.gathered() receives for one step: rows.npy (world, batch, max_det, 6)
+    with the slots past each image's count zeroed, and counts.npy (world, batch; -1: no candidate passed the filter), both
+    float32.  Beyond DUMP_CAP_BYTES a fixed, seeded sample of the images is written instead, their flat indices in
+    images.npy."""
+    import numpy as np
+    rows, counts = rows.cpu().numpy(), counts.cpu().numpy()
+    rows = np.where((np.arange(rows.shape[2]) < counts[..., None])[..., None], rows, np.float32(0))
+    os.makedirs(out_dir, exist_ok=True)
+    per_image = rows[0, 0].nbytes + 4
+    n = counts.size
+    if n * per_image > DUMP_CAP_BYTES:
+        images = np.sort(np.random.default_rng(0).choice(n, DUMP_CAP_BYTES // per_image, replace=False))
+        rows, counts = rows.reshape(n, *rows.shape[2:])[images], counts.reshape(n)[images]
+        np.save(os.path.join(out_dir, "images.npy"), images.astype(np.float64))
+    np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float32))
+    np.save(os.path.join(out_dir, "counts.npy"), counts.astype(np.float32))
 
 
 def bench_hyp(family="yolov5"):
@@ -369,7 +401,7 @@ def run_ours(args):
             e_beg.record(stream)
             self.fork()
             for k in range(steps):
-                spp.submit(self.heads, events=evs[k] if evs else None, sync_input=False)
+                self.last_lane = spp.submit(self.heads, events=evs[k] if evs else None, sync_input=False)
             spp.drain()
             e_end.record(stream)
             sync_all()
@@ -419,6 +451,11 @@ def run_ours(args):
     graphed = main.spp.graph
     timed = main.measure(args.steps, args.warmup, events=not graphed)
     total_ms = timed["total_ms"]
+    last_out = None
+    if args.dump_outputs and rank == 0:
+        # copied on the device before the hold steps reuse the lane's buffers; written to disk once the sampler is off
+        last_out = [t.clone() for t in main.spp.gathered(main.last_lane)]
+        stream.synchronize()
     # Keep the identical load running ~1.5 s so NVML (10 ms period) sees the clocks this workload runs at; the step count
     # is derived from the all-reduced step time, so every rank issues the same sequence.
     hold_steps = int(min(200000, max(100, 1500.0 / max(total_ms / args.steps, 1e-3))))
@@ -432,6 +469,9 @@ def run_ours(args):
     torch.cuda.synchronize()
     if sampler:
         sampler.arm(False)
+    if last_out is not None:
+        dump_outputs(args.dump_outputs, *last_out)
+        del last_out
     sync_all()
     main.spp.check()
     iso_ms = main.filter_alone_ms()

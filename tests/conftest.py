@@ -69,8 +69,12 @@ def full_size_golden(name):
         heads = None
     decoded = None
     if "decoded_rows" in g:
+        # stored: box + objectness of every survivor and its largest class probability; the single-label path reads
+        # nothing else of the class columns, so the others stay zero
         decoded = np.zeros(tuple(int(x) for x in g["decoded_shape"]), dtype=np.float32)
-        decoded[0, g["decoded_index"]] = g["decoded_rows"]
+        idx = g["decoded_index"]
+        decoded[0, idx, :5] = g["decoded_rows"]
+        decoded[0, idx, 5 + g["decoded_cls_id"]] = g["decoded_cls_max"]
     return g, heads, decoded
 
 

@@ -6,6 +6,9 @@ byte-for-byte copy baseline/_ref/:
           8c, the end-to-end bit-exact oracle for kept indices;
   mode A  hyp['device'] = 'cpu': the path the goldens were generated with (CPU ATen sigmoid/exp differ from CUDA's by an
           ulp, so score bits may differ; every disagreement is counted and attributed to its stage, oracle/parity.py).
+Without the upstream sources these tests skip.  test_fused_path_vs_oracle_* then make the same comparisons against the
+oracle (oracle/, pinned to upstream by the fixtures under tests/golden), less the two checks that would compare the
+oracle or the engine with itself there (_oracle_runs).
 Sizes: BASELINE C1 (YOLOv5s 640^2, 25 200 candidates, dense/sparse/crowd), YOLOX-s 8 400, YOLOv7, YOLOv8, RetinaNet,
 FCOS at sizes the reference's O(K*M) loop finishes in seconds, and the 1280^2 crowd case.
 """
@@ -14,7 +17,6 @@ import json
 import os
 import subprocess
 import sys
-import tempfile
 
 import numpy as np
 import pytest
@@ -52,14 +54,75 @@ CASES = [
 ]
 
 
+def _numpy(x):
+    return x.numpy() if isinstance(x, torch.Tensor) else type(x)(_numpy(v) for v in x)
+
+
+def _oracle_decode(fam, heads, img):
+    import oracle
+    h = _numpy(heads)
+    if fam == "yolov5":
+        return oracle.decode_yolov5(h)
+    if fam == "yolov7":
+        return oracle.decode_yolov7(h)
+    if fam == "yolox":
+        return oracle.decode_yolox(h, img)
+    if fam == "yolov8":
+        return oracle.decode_yolov8(h, img)
+    if fam in ("retinanet", "retinanet_exp"):
+        return oracle.decode_retinanet(h[0], h[1], img, img)
+    return oracle.decode_fcos(h[0], h[1], h[2], img)
+
+
+def _oracle_runs(tmp):
+    """The reference side of CASES from the oracle (oracle/), pinned to upstream outputs stored
+    in tests/golden -- on upstream's decoded tensors its NMS reproduces upstream's rows bit for bit, and its decode is
+    within 1e-5 of upstream's CPU decode.  One npz per case and mode, in the format of baseline/ref_worker.py:
+      mode A  the oracle's numpy decode (upstream's CPU path restated) -> oracle NMS;
+      mode B  the engine's CUDA decode -> oracle NMS: kept rows and candidate indices are held bit-exact given the same
+              CUDA decode, as upstream's CUDA-decode mode held them; the decode itself is held to 1e-5 by mode A."""
+    import oracle
+    from oracle import refharness
+    from yoloseries_b200 import synth
+    from yoloseries_b200.engine import PostProcessor
+    out = {mode: os.path.join(tmp, mode) for mode in ("A", "B")}
+    for d in out.values():
+        os.makedirs(d)
+    for case in CASES:
+        fam, img = case["family"], case["img"]
+        meta = {k: v for k, v in refharness.reference_hyp((img, img), **case.get("hyp", {})).items()
+                if isinstance(v, (int, float, bool, str))}
+        hyp = _hyp(meta)
+        heads = synth.make_heads(fam, case["batch"], img, img, 80, case["dist"], case["seed"], "cpu")
+        anchors = torch.tensor(synth.V5_ANCHORS_PX) if fam in ("yolov5", "yolov7") else None
+        decoded = {"A": _oracle_decode(fam, heads, img),
+                   "B": PostProcessor(fam, hyp, anchors=anchors).decode(_engine_outputs(case), img, img).cpu().numpy()}
+        for mode, dec in decoded.items():
+            res = oracle.evaluator_nms(fam, dec, hyp)
+            rows = np.zeros((len(res), max([1] + [r.rows.shape[0] for r in res if r.rows is not None]), 6), np.float32)
+            counts = np.full(len(res), -1, np.int32)
+            for i, r in enumerate(res):
+                if r.rows is not None:
+                    counts[i] = r.rows.shape[0]
+                    rows[i, :counts[i]] = r.rows
+            np.savez(os.path.join(out[mode], case["name"] + ".npz"), decoded=dec, rows=rows, counts=counts,
+                     meta=np.array(repr(meta)))
+    return out
+
+
 @pytest.fixture(scope="module")
-def reference_runs():
+def oracle_runs(tmp_path_factory):
+    return _oracle_runs(str(tmp_path_factory.mktemp("oracle")))
+
+
+@pytest.fixture(scope="module")
+def reference_runs(tmp_path_factory):
     """Runs the unmodified reference over CASES once per mode (two child processes side by side)."""
     sys.path.insert(0, ROOT)
     from oracle import refharness
     if not (refharness.available() or os.path.isdir(os.path.join(refharness.STAGED_ROOT, "trainer"))):
-        pytest.skip("neither /root/reference nor the staged copy baseline/_ref is present")
-    tmp = tempfile.mkdtemp(prefix="ysb_ref_")
+        pytest.skip("the upstream YOLOSeries sources are not present (test_fused_path_vs_oracle_* run without them)")
+    tmp = str(tmp_path_factory.mktemp("reference"))
     spec = os.path.join(tmp, "spec.json")
     with open(spec, "w") as f:
         json.dump(CASES, f)
@@ -146,14 +209,15 @@ def _dump(tag, case, summary, reps):
                                 "images": [r for r in reps if r["stage"] != "ok"]}) + "\n")
 
 
-@pytest.mark.parametrize("case", CASES, ids=[c["name"] for c in CASES])
-def test_fused_path_vs_reference_cuda_mode_b(case, reference_runs):
-    """Mode B: kept rows and kept candidate indices bit-exact against the reference run with hyp['device']='cuda'
-    (RetinaNet's merged boxes: 1e-5, the reference's own sgemm order is unspecified)."""
-    dec, ref_dec, reps, summary = _report(case, reference_runs["B"])
-    _dump("B", case, summary, reps)
-    assert summary["oracle_reproduces_reference"], summary
-    assert _decode_ok(case["family"], dec, ref_dec, case["img"]), "decoded tensor beyond 1e-5 of the reference's"
+def _check_cuda_decode(case, ref_dir, tag, upstream):
+    """Kept rows and kept candidate indices bit-exact (RetinaNet's merged boxes: 1e-5, the reference's own sgemm order is
+    unspecified).  ``upstream``: the rows and the decoded tensor come from an upstream run, so the oracle's reproduction
+    of those rows and the decode are checked too; otherwise the rows are the oracle's own, on the engine's decode."""
+    dec, ref_dec, reps, summary = _report(case, ref_dir)
+    _dump(tag, case, summary, reps)
+    if upstream:
+        assert summary["oracle_reproduces_reference"], summary
+        assert _decode_ok(case["family"], dec, ref_dec, case["img"]), "decoded tensor beyond 1e-5 of the reference's"
     fam = case["family"]
     for r in reps:
         if fam.startswith("retinanet") or fam == "yolov8":
@@ -165,17 +229,42 @@ def test_fused_path_vs_reference_cuda_mode_b(case, reference_runs):
             assert r["stage"] == "ok" and r["rows_bit_exact"], (r, summary)
 
 
-@pytest.mark.parametrize("case", CASES, ids=[c["name"] for c in CASES])
-def test_fused_path_vs_reference_cpu_mode_a(case, reference_runs):
-    """Mode A (CPU ATen decode): decoded tensors within 1e-5; kept rows compared and every disagreement attributed.  A
-    disagreement is accepted only when it is explained by differing score bits (CPU vs CUDA sigmoid/exp ulps) or by an
-    IoU within 1e-6 of the threshold -- never by the NMS stage on identical inputs."""
-    dec, ref_dec, reps, summary = _report(case, reference_runs["A"])
-    _dump("A", case, summary, reps)
-    assert summary["oracle_reproduces_reference"], summary
+def _check_cpu_decode(case, ref_dir, tag, upstream):
+    """Decoded tensors within 1e-5; kept rows compared and every disagreement attributed.  A disagreement is accepted only
+    when it is explained by differing score bits (CPU vs CUDA sigmoid/exp ulps) or by an IoU within 1e-6 of the
+    threshold -- never by the NMS stage on identical inputs.  ``upstream``: see _check_cuda_decode."""
+    dec, ref_dec, reps, summary = _report(case, ref_dir)
+    _dump(tag, case, summary, reps)
+    if upstream:
+        assert summary["oracle_reproduces_reference"], summary
     assert _decode_ok(case["family"], dec, ref_dec, case["img"]), "decoded tensor beyond 1e-5 of the reference's"
     for r in reps:
         if r["stage"] == "nms":
             assert r.get("iou_within_eps_of_threshold", 0) > 0 or r.get("score_bits_differ", 0) > 0, (r, summary)
         if r["stage"] in ("ok", "rows"):
             assert r.get("rows_max_rel_err", 0.0) <= 1e-5, (r, summary)
+
+
+@pytest.mark.parametrize("case", CASES, ids=[c["name"] for c in CASES])
+def test_fused_path_vs_reference_cuda_mode_b(case, reference_runs):
+    """Mode B: against the reference run with hyp['device']='cuda'."""
+    _check_cuda_decode(case, reference_runs["B"], "B", upstream=True)
+
+
+@pytest.mark.parametrize("case", CASES, ids=[c["name"] for c in CASES])
+def test_fused_path_vs_reference_cpu_mode_a(case, reference_runs):
+    """Mode A: against the reference run with hyp['device']='cpu' (CPU ATen decode)."""
+    _check_cpu_decode(case, reference_runs["A"], "A", upstream=True)
+
+
+@pytest.mark.parametrize("case", CASES, ids=[c["name"] for c in CASES])
+def test_fused_path_vs_oracle_cuda_decode(case, oracle_runs):
+    """The oracle's NMS on the engine's own CUDA decode: the select, sort, NMS and post-filter kernels at full size."""
+    _check_cuda_decode(case, oracle_runs["B"], "oracle-B", upstream=False)
+
+
+@pytest.mark.parametrize("case", CASES, ids=[c["name"] for c in CASES])
+def test_fused_path_vs_oracle_cpu_decode(case, oracle_runs):
+    """The oracle's numpy decode (upstream's CPU path restated) and its NMS: the engine's decode within 1e-5 of it and
+    every disagreement in the kept rows attributed."""
+    _check_cpu_decode(case, oracle_runs["A"], "oracle-A", upstream=False)
