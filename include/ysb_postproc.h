@@ -44,7 +44,7 @@
 extern "C" {
 #endif
 
-#define YSB_ABI_VERSION 5
+#define YSB_ABI_VERSION 6
 #define YSB_MAX_LEVELS 8
 #define YSB_MAX_ANCHORS 9
 #define YSB_MAX_PASSES 4             /* test-time-augmentation passes merged by ysb_postprocess_tta */
@@ -73,6 +73,14 @@ typedef enum ysb_family {
     YSB_RETINANET_EXP = 5, /* heads: reg (b, N, 5), cls (b, N, C)                 trainer/eval_retinanet_experiment.py */
     YSB_FCOS = 6           /* heads: L x cls (b,C,H,W), L x reg (b,4,H,W), L x ctr (b,1,H,W)  trainer/eval_fcos.py */
 } ysb_family;
+
+/* Element type of the raw head tensors.  16-bit heads are widened to float32 right after every load (exact): all
+ * arithmetic and every output stay float32, bit-identical to a float32 call on the widened heads. */
+typedef enum ysb_dtype {
+    YSB_F32 = 0,
+    YSB_F16 = 1,   /* IEEE binary16 (torch.float16) */
+    YSB_BF16 = 2   /* bfloat16 (torch.bfloat16) */
+} ysb_dtype;
 
 typedef enum ysb_input_kind {
     YSB_INPUT_RAW_HEADS = 0,   /* raw model outputs; decode is fused into the filter/NMS kernels */
@@ -137,6 +145,10 @@ typedef struct ysb_params {
      * output).  Same arithmetic as ysb_undo_letterbox; applied after NMS, the postprocess_bbox count filter and
      * remove_small_boxes, which all see the un-mapped boxes exactly like the reference. */
     const float *d_letterbox;
+    /* ysb_dtype of every tensor in d_heads (RAW_HEADS input; one type per call, every TTA pass the same).  0 = float32,
+     * so a zero-filled struct keeps the float32 behaviour.  DECODED_ROWS input is float32 only: another value there, an
+     * unknown value or passes of different types return YSB_ERR_BAD_ARG. */
+    int32_t head_dtype;
 } ysb_params;
 
 int ysb_abi_version(void);

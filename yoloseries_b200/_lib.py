@@ -20,11 +20,13 @@ YOLOV5, YOLOV7, YOLOX, YOLOV8, RETINANET, RETINANET_EXP, FCOS = range(7)
 FAMILY_IDS = {"yolov5": YOLOV5, "yolov7": YOLOV7, "yolox": YOLOX, "yolov8": YOLOV8, "retinanet": RETINANET,
               "retinanet_exp": RETINANET_EXP, "fcos": FCOS}
 INPUT_RAW_HEADS, INPUT_DECODED_ROWS = 0, 1
+# enum ysb_dtype (element type of the raw heads)
+DTYPE_F32, DTYPE_F16, DTYPE_BF16 = 0, 1, 2
 IOU_NUMBA_F64MIX, IOU_F32, GIOU, DIOU, CIOU = range(5)
 IOU_KIND_IDS = {"numba": IOU_NUMBA_F64MIX, "iou": IOU_F32, "giou": GIOU, "diou": DIOU, "ciou": CIOU}
 CMP_GE, CMP_GT = 0, 1
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 YSB_MAX_PASSES = 4
 YSB_MAX_PEERS = 16
 YSB_IPC_HANDLE_BYTES = 64
@@ -65,6 +67,7 @@ class YsbParams(ctypes.Structure):
         ("tta_img_h", ctypes.c_int32),
         ("tta_img_w", ctypes.c_int32),
         ("d_letterbox", ctypes.c_void_p),
+        ("head_dtype", ctypes.c_int32),
     ]
 
 

@@ -9,19 +9,21 @@
 #include "ysb_internal.cuh"
 
 namespace ysb {
+// dtype: ysb_dtype of the heads the Plan points at
 cudaError_t launch_filter(const Plan &P, int vec, uint64_t *d_keys, int64_t key_cap, int32_t *d_counts, cudaStream_t stream,
-                          bool zero_counts);
+                          bool zero_counts, int dtype);
 cudaError_t launch_select_nms(const Plan &P, const uint64_t *d_keys, int64_t key_cap, const int32_t *d_counts,
                               float *d_dets, int32_t *d_det_idx, int32_t *d_det_cnt, cudaStream_t stream,
-                              const GatherSink *sink = nullptr);
+                              const GatherSink *sink, int dtype);
 bool make_gather_sink(const ysb_gather *g, int slot, GatherSink *out);
 bool gather_valid(const ysb_gather *g, int slot);
 cudaError_t launch_gather_begin(const ysb_gather *g, int slot, int32_t *d_counts, int64_t n_counts, cudaStream_t stream);
 cudaError_t launch_gather_wait(const ysb_gather *g, int slot, cudaStream_t stream);
 cudaError_t launch_select_nms_tta(const Plan &P, const ExtraPasses &X, const uint64_t *d_keys, int64_t key_cap,
                                   const int32_t *d_counts, float *d_dets, int32_t *d_det_idx, int32_t *d_det_cnt,
-                                  cudaStream_t stream);
-cudaError_t launch_decode(const Plan &P, float *d_out, int64_t rows_total, int64_t row_offset, cudaStream_t stream);
+                                  cudaStream_t stream, int dtype);
+cudaError_t launch_decode(const Plan &P, float *d_out, int64_t rows_total, int64_t row_offset, cudaStream_t stream,
+                          int dtype);
 cudaError_t launch_array_nms(const float *d_boxes, const float *d_scores, int64_t m, double iou_thr, int cmp, int iou_kind,
                              int64_t max_keep, void *ws, int32_t *d_keep, int32_t *d_keep_cnt, cudaStream_t stream);
 size_t array_nms_workspace_bytes(int64_t m);
@@ -68,9 +70,12 @@ static int64_t key_slots(const Plan &P) { return static_cast<int64_t>(P.N) * (P.
 
 struct Built {
     Plan plan;
-    int vec;  // 128-bit loads possible for the planes kernel
+    int vec;  // 4-element vector loads possible for the planes kernel
     int heads_expected;
+    int dtype;  // ysb_dtype of the heads
 };
+
+static size_t dtype_bytes(int dtype) { return dtype == YSB_F32 ? 4 : 2; }
 
 static int expected_heads(const ysb_params *p)
 {
@@ -89,6 +94,8 @@ static int build_plan(const ysb_params *p, const void *const *d_heads, int num_h
     if (!p || !out) return YSB_ERR_BAD_ARG;
     if (p->family < YSB_YOLOV5 || p->family > YSB_FCOS) return YSB_ERR_BAD_ARG;
     if (p->input_kind != YSB_INPUT_RAW_HEADS && p->input_kind != YSB_INPUT_DECODED_ROWS) return YSB_ERR_BAD_ARG;
+    if (p->head_dtype != YSB_F32 && p->head_dtype != YSB_F16 && p->head_dtype != YSB_BF16) return YSB_ERR_BAD_ARG;
+    if (p->head_dtype != YSB_F32 && p->input_kind == YSB_INPUT_DECODED_ROWS) return YSB_ERR_BAD_ARG;  // decoded rows: float32
     if (p->batch < 0 || p->num_classes <= 0 || p->num_levels <= 0 || p->num_levels > YSB_MAX_LEVELS) return YSB_ERR_BAD_ARG;
     if (p->anchors_per_cell <= 0 || p->anchors_per_cell > YSB_MAX_ANCHORS) return YSB_ERR_BAD_ARG;
     if (p->num_classes > YSB_MAX_CLASSES) return YSB_ERR_LIMIT;
@@ -211,11 +218,16 @@ static int build_plan(const ysb_params *p, const void *const *d_heads, int num_h
     if (P.layout == LAYOUT_ROWS && static_cast<size_t>(128) * (P.row_w_in | 1) * sizeof(float) > 227u * 1024u) return YSB_ERR_LIMIT;
 
     out->heads_expected = expected_heads(p);
+    out->dtype = p->head_dtype;
+    const size_t esize = dtype_bytes(p->head_dtype);
     out->vec = 1;
     if (P.layout == LAYOUT_PLANES) {
+        // a unit of 4 positions is one 16-byte (float32) or 8-byte (16-bit) load: plane starts stay aligned to it when
+        // the tensor base is and H*W % 4 == 0
         bool aligned = true;
         if (d_heads)
-            for (int i = 0; i < num_heads; ++i) aligned = aligned && ((reinterpret_cast<uintptr_t>(d_heads[i]) & 15u) == 0);
+            for (int i = 0; i < num_heads; ++i)
+                aligned = aligned && ((reinterpret_cast<uintptr_t>(d_heads[i]) & (4 * esize - 1)) == 0);
         int n4 = 0, units = 0;
         for (int l = 0; l < L; ++l) {
             P.lv[l].vec = (aligned && P.lv[l].hw % 4 == 0) ? 4 : 1;  // e.g. FCOS' 5x5 level falls back to scalar units
@@ -254,7 +266,9 @@ static int build_plan(const ysb_params *p, const void *const *d_heads, int num_h
     case YSB_RETINANET:
     case YSB_RETINANET_EXP:
         for (int l = 0; l < L; ++l) {
-            P.lv[l].p0 = static_cast<const float *>(d_heads[1]) + static_cast<size_t>(P.lv[l].cand_off) * C;
+            // (the Plan's pointers are typed float; the kernels reinterpret them as the head element type)
+            P.lv[l].p0 = reinterpret_cast<const float *>(static_cast<const char *>(d_heads[1]) +
+                                                         static_cast<size_t>(P.lv[l].cand_off) * C * esize);
             P.lv[l].p1 = static_cast<const float *>(d_heads[0]);
         }
         break;
@@ -312,7 +326,7 @@ int ysb_decode(const ysb_params *p, const void *const *d_heads, int num_heads, f
     Built b;
     const int st = build_plan(p, d_heads, num_heads, &b);
     if (st != YSB_OK) return st;
-    return cuda_status(launch_decode(b.plan, d_decoded, b.plan.N, 0, static_cast<cudaStream_t>(stream)));
+    return cuda_status(launch_decode(b.plan, d_decoded, b.plan.N, 0, static_cast<cudaStream_t>(stream), b.dtype));
 }
 
 int ysb_decode_into(const ysb_params *p, const void *const *d_heads, int num_heads, float *d_decoded, int64_t rows_total,
@@ -324,7 +338,7 @@ int ysb_decode_into(const ysb_params *p, const void *const *d_heads, int num_hea
     const int st = build_plan(p, d_heads, num_heads, &b);
     if (st != YSB_OK) return st;
     if (row_offset < 0 || rows_total < row_offset + b.plan.N) return YSB_ERR_BAD_ARG;
-    return cuda_status(launch_decode(b.plan, d_decoded, rows_total, row_offset, static_cast<cudaStream_t>(stream)));
+    return cuda_status(launch_decode(b.plan, d_decoded, rows_total, row_offset, static_cast<cudaStream_t>(stream), b.dtype));
 }
 
 int ysb_filter_candidates(const ysb_params *p, const void *const *d_heads, int num_heads, uint64_t *d_keys,
@@ -335,7 +349,8 @@ int ysb_filter_candidates(const ysb_params *p, const void *const *d_heads, int n
     const int st = build_plan(p, d_heads, num_heads, &b);
     if (st != YSB_OK) return st;
     if (key_capacity < key_slots(b.plan)) return YSB_ERR_WORKSPACE;
-    return cuda_status(launch_filter(b.plan, b.vec, d_keys, key_capacity, d_counts, static_cast<cudaStream_t>(stream), true));
+    return cuda_status(launch_filter(b.plan, b.vec, d_keys, key_capacity, d_counts, static_cast<cudaStream_t>(stream), true,
+                                     b.dtype));
 }
 
 int ysb_select_nms(const ysb_params *p, const void *const *d_heads, int num_heads, const uint64_t *d_keys,
@@ -348,7 +363,7 @@ int ysb_select_nms(const ysb_params *p, const void *const *d_heads, int num_head
     if (st != YSB_OK) return st;
     if (key_capacity < key_slots(b.plan)) return YSB_ERR_WORKSPACE;
     return cuda_status(launch_select_nms(b.plan, d_keys, key_capacity, d_counts, d_dets, d_det_idx, d_det_cnt,
-                                         static_cast<cudaStream_t>(stream)));
+                                         static_cast<cudaStream_t>(stream), nullptr, b.dtype));
 }
 
 // ---- multi-GPU detection gather (gather_kernels.cu) ------------------------------------------------------------------
@@ -445,7 +460,7 @@ int ysb_select_nms_gather(const ysb_params *p, const void *const *d_heads, int n
     if (!make_gather_sink(g, slot, &sink)) return YSB_ERR_BAD_ARG;
     if (g->batch != b.plan.batch || g->max_det != b.plan.max_det) return YSB_ERR_BAD_ARG;
     return cuda_status(launch_select_nms(b.plan, d_keys, key_capacity, d_counts, nullptr, d_det_idx, nullptr,
-                                         static_cast<cudaStream_t>(stream), &sink));
+                                         static_cast<cudaStream_t>(stream), &sink, b.dtype));
 }
 
 int ysb_gather_wait(const ysb_gather *g, int slot, void *stream)
@@ -491,9 +506,9 @@ int ysb_postprocess(const ysb_params *p, const void *const *d_heads, int num_hea
     const int64_t slots = key_slots(b.plan);
     int32_t *d_counts = reinterpret_cast<int32_t *>(base + align256(sizeof(uint64_t) * static_cast<size_t>(slots) * b.plan.batch));
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    st = cuda_status(launch_filter(b.plan, b.vec, d_keys, slots, d_counts, s, true));
+    st = cuda_status(launch_filter(b.plan, b.vec, d_keys, slots, d_counts, s, true, b.dtype));
     if (st != YSB_OK) return st;
-    return cuda_status(launch_select_nms(b.plan, d_keys, slots, d_counts, d_dets, d_det_idx, d_det_cnt, s));
+    return cuda_status(launch_select_nms(b.plan, d_keys, slots, d_counts, d_dets, d_det_idx, d_det_cnt, s, nullptr, b.dtype));
 }
 
 // ---- test-time augmentation: several passes, one merged candidate space -------------------------------------------
@@ -520,7 +535,7 @@ static int build_passes(const ysb_params *passes, int num_passes, const void *co
             p->iou_thr != q->iou_thr || p->max_det != q->max_det || p->class_aware != q->class_aware ||
             p->multi_label != q->multi_label || p->postprocess_bbox != q->postprocess_bbox ||
             p->min_box_wh != q->min_box_wh || p->pre_nms_topk != q->pre_nms_topk ||
-            p->thresh_with_ctr != q->thresh_with_ctr)
+            p->thresh_with_ctr != q->thresh_with_ctr || p->head_dtype != q->head_dtype)
             return YSB_ERR_BAD_ARG;
         const int nh = d_heads ? heads_per_pass[i] : 0;
         const int st = build_plan(p, d_heads ? d_heads + head0 : nullptr, nh, &out->b[i]);
@@ -565,7 +580,7 @@ int ysb_postprocess_tta(const ysb_params *passes, int num_passes, const void *co
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     // every pass appends its survivors to the same per-image key list (the counters are zeroed by the first pass only)
     for (int i = 0; i < num_passes; ++i) {
-        st = cuda_status(launch_filter(bp.b[i].plan, bp.b[i].vec, d_keys, bp.slots, d_counts, s, i == 0));
+        st = cuda_status(launch_filter(bp.b[i].plan, bp.b[i].vec, d_keys, bp.slots, d_counts, s, i == 0, bp.b[i].dtype));
         if (st != YSB_OK) return st;
     }
     ExtraPasses X;
@@ -575,7 +590,8 @@ int ysb_postprocess_tta(const ysb_params *passes, int num_passes, const void *co
         X.base[i - 1] = static_cast<int>(bp.base[i]);
         X.p[i - 1] = bp.b[i].plan;
     }
-    return cuda_status(launch_select_nms_tta(bp.b[0].plan, X, d_keys, bp.slots, d_counts, d_dets, d_det_idx, d_det_cnt, s));
+    return cuda_status(launch_select_nms_tta(bp.b[0].plan, X, d_keys, bp.slots, d_counts, d_dets, d_det_idx, d_det_cnt, s,
+                                             bp.b[0].dtype));
 }
 
 int ysb_nms_workspace_bytes(int64_t m, size_t *bytes_out)

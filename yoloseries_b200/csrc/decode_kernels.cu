@@ -8,6 +8,7 @@
 // A CTA owns 32 consecutive candidates of one image; sigmoid/exp values are produced into a shared-memory tile
 // [32][C'] and written out with fully coalesced stores (32 rows of one image are contiguous in the output).
 // Planes heads are read coalesced along positions (lane = candidate), rows heads along the row (lane = column).
+// Templated on the head element type T: 16-bit heads are widened as they are loaded, the rows are float32.
 #include "ysb_internal.cuh"
 
 namespace ysb {
@@ -23,38 +24,40 @@ constexpr int kDecInFlightRows = 10;
 
 // Address of class logit 0 of a candidate and the stride between consecutive classes (hoisted out of the class loop:
 // the level lookup and the two integer divisions are per candidate, not per element).
+template <typename T>
 struct CandAddr {
-    const float *cls;
+    const T *cls;
     size_t cstride;
-    const float *obj;  // objectness / centerness / conf logit, nullptr when the family has none
+    const T *obj;  // objectness / centerness / conf logit, nullptr when the family has none
 };
 
-__device__ __forceinline__ CandAddr cand_addr(const Plan &P, int img, int cand)
+template <typename T>
+__device__ __forceinline__ CandAddr<T> cand_addr(const Plan &P, int img, int cand)
 {
-    CandAddr c;
+    CandAddr<T> c;
     const int l = find_level(P, cand);
     const LevelDesc &lv = P.lv[l];
     const int r = cand - lv.cand_off;
     c.obj = nullptr;
     if (P.layout == LAYOUT_PLANES) {
         const int a = r / lv.hw, pos = r - a * lv.hw;
-        c.cls = lv.p0 + (static_cast<size_t>(img * P.A + a) * P.cls_nch + P.cls_ch) * lv.hw + pos;
+        c.cls = head_ptr<T>(lv.p0) + (static_cast<size_t>(img * P.A + a) * P.cls_nch + P.cls_ch) * lv.hw + pos;
         c.cstride = static_cast<size_t>(lv.hw);
         if (P.obj_col >= 0)
-            c.obj = (P.obj_src == 2 ? lv.p2 : lv.p0) + (static_cast<size_t>(img * P.A + a) * P.obj_nch + P.obj_ch) * lv.hw + pos;
+            c.obj = head_ptr<T>(P.obj_src == 2 ? lv.p2 : lv.p0) + (static_cast<size_t>(img * P.A + a) * P.obj_nch + P.obj_ch) * lv.hw + pos;
     } else {
-        const float *row = lv.p0 + (static_cast<size_t>(img) * lv.img_rows + r) * P.row_w_in;
+        const T *row = head_ptr<T>(lv.p0) + (static_cast<size_t>(img) * lv.img_rows + r) * P.row_w_in;
         c.cls = row + P.cls_col_in;
         c.cstride = 1;
         if (P.obj_col >= 0)
-            c.obj = P.obj_src == 1 ? P.lv[0].p1 + (static_cast<size_t>(img) * P.N + cand) * P.reg_row_w + 4 : row + P.obj_col_in;
+            c.obj = P.obj_src == 1 ? head_ptr<T>(P.lv[0].p1) + (static_cast<size_t>(img) * P.N + cand) * P.reg_row_w + 4 : row + P.obj_col_in;
     }
     return c;
 }
 
 // ROWS = candidates per CTA: 32 for channels-last heads (their rows are contiguous anyway), 128 for NCHW planes so that
 // every plane access of a CTA covers 512 contiguous bytes.
-template <int ROWS>
+template <int ROWS, typename T>
 __global__ void __launch_bounds__(kDecThreads) k_decode_rows(const __grid_constant__ Plan P, float *__restrict__ out,
                                                               int64_t rows_total, int64_t row_offset)
 {
@@ -69,19 +72,19 @@ __global__ void __launch_bounds__(kDecThreads) k_decode_rows(const __grid_consta
         constexpr int kPhases = kDecThreads / ROWS;  // 2 for ROWS = 128
         const int rr = threadIdx.x % ROWS, ph = threadIdx.x / ROWS;
         if (rr < nrows) {
-            const CandAddr ca = cand_addr(P, img, c0 + rr);
+            const CandAddr<T> ca = cand_addr<T>(P, img, c0 + rr);
             float *tc = tile + rr * rw + P.cls_col;
             const size_t step = static_cast<size_t>(kPhases) * ca.cstride;
             // kDecInFlight independent loads per thread before the first sigmoid: the kernel is bound by memory-level
             // parallelism, not by instruction issue (4 loads in flight left DRAM at 37 % of peak)
-            const float ov = (ph == 0 && ca.obj) ? __ldg(ca.obj) : 0.0f;
-            const float *src = ca.cls + static_cast<size_t>(ph) * ca.cstride;
+            const float ov = (ph == 0 && ca.obj) ? ldg_head(ca.obj) : 0.0f;
+            const T *src = ca.cls + static_cast<size_t>(ph) * ca.cstride;
             int k = ph;
             // whole batches need no per-load bounds test (80 classes: four of them)
             for (; k + (kDecInFlight - 1) * kPhases < P.C; k += kDecInFlight * kPhases, src += kDecInFlight * step) {
                 float v[kDecInFlight];
 #pragma unroll
-                for (int u = 0; u < kDecInFlight; ++u) v[u] = __ldg(src + u * step);
+                for (int u = 0; u < kDecInFlight; ++u) v[u] = ldg_head(src + u * step);
                 bool redo = false;
 #pragma unroll
                 for (int u = 0; u < kDecInFlight; ++u) tc[k + u * kPhases] = sigmoid_fast(v[u], redo);
@@ -93,7 +96,7 @@ __global__ void __launch_bounds__(kDecThreads) k_decode_rows(const __grid_consta
             if (k < P.C) {
                 float v[kDecInFlight];
 #pragma unroll
-                for (int u = 0; u < kDecInFlight; ++u) v[u] = (k + u * kPhases < P.C) ? __ldg(src + u * step) : 0.0f;
+                for (int u = 0; u < kDecInFlight; ++u) v[u] = (k + u * kPhases < P.C) ? ldg_head(src + u * step) : 0.0f;
 #pragma unroll
                 for (int u = 0; u < kDecInFlight; ++u)
                     if (k + u * kPhases < P.C) tc[k + u * kPhases] = sigmoid_ref(v[u]);
@@ -105,7 +108,7 @@ __global__ void __launch_bounds__(kDecThreads) k_decode_rows(const __grid_consta
             for (int base = 0; base < nrows; base += kDecThreads / 4) {
                 const int r4 = base + (threadIdx.x >> 2), side = threadIdx.x & 3;
                 float sv = 0.0f;
-                if (r4 < nrows) sv = v8_side_value(P, img, c0 + r4, side);
+                if (r4 < nrows) sv = v8_side_value<T>(P, img, c0 + r4, side);
                 const unsigned qb = lane & ~3u;
                 const float s0 = __shfl_sync(0xffffffffu, sv, qb), s1 = __shfl_sync(0xffffffffu, sv, qb + 1);
                 const float s2 = __shfl_sync(0xffffffffu, sv, qb + 2), s3 = __shfl_sync(0xffffffffu, sv, qb + 3);
@@ -117,7 +120,7 @@ __global__ void __launch_bounds__(kDecThreads) k_decode_rows(const __grid_consta
             }
         } else if (threadIdx.x >= kDecThreads - ROWS && threadIdx.x - (kDecThreads - ROWS) < nrows) {
             const int rb = threadIdx.x - (kDecThreads - ROWS);
-            const float4 b = tta_undo(P, decode_box_cols(P, img, c0 + rb));
+            const float4 b = tta_undo(P, decode_box_cols<T>(P, img, c0 + rb));
             float *t = tile + rb * rw + P.box_col;
             t[0] = b.x; t[1] = b.y; t[2] = b.z; t[3] = b.w;
         }
@@ -126,13 +129,13 @@ __global__ void __launch_bounds__(kDecThreads) k_decode_rows(const __grid_consta
         // fetched sector fully used; kDecInFlightRows loads in flight per thread.  Lane-per-candidate box / objectness decode.
         const int r = threadIdx.x >> 3, q = threadIdx.x & 7;
         if (r < nrows) {
-            const CandAddr ca = cand_addr(P, img, c0 + r);
+            const CandAddr<T> ca = cand_addr<T>(P, img, c0 + r);
             float *tc = tile + r * rw + P.cls_col;
             int k = q;
             for (; k + 8 * (kDecInFlightRows - 1) < P.C; k += 8 * kDecInFlightRows) {
                 float v[kDecInFlightRows];
 #pragma unroll
-                for (int u = 0; u < kDecInFlightRows; ++u) v[u] = __ldg(ca.cls + k + 8 * u);
+                for (int u = 0; u < kDecInFlightRows; ++u) v[u] = ldg_head(ca.cls + k + 8 * u);
                 bool redo = false;
 #pragma unroll
                 for (int u = 0; u < kDecInFlightRows; ++u) tc[k + 8 * u] = sigmoid_fast(v[u], redo);
@@ -144,7 +147,7 @@ __global__ void __launch_bounds__(kDecThreads) k_decode_rows(const __grid_consta
             if (k < P.C) {
                 float v[kDecInFlightRows];
 #pragma unroll
-                for (int u = 0; u < kDecInFlightRows; ++u) v[u] = (k + 8 * u < P.C) ? __ldg(ca.cls + k + 8 * u) : 0.0f;
+                for (int u = 0; u < kDecInFlightRows; ++u) v[u] = (k + 8 * u < P.C) ? ldg_head(ca.cls + k + 8 * u) : 0.0f;
 #pragma unroll
                 for (int u = 0; u < kDecInFlightRows; ++u)
                     if (k + 8 * u < P.C) tc[k + 8 * u] = sigmoid_ref(v[u]);
@@ -152,12 +155,12 @@ __global__ void __launch_bounds__(kDecThreads) k_decode_rows(const __grid_consta
         }
         if (warp == 0 && lane < nrows) {
             const int cand = c0 + lane;
-            const float4 b = tta_undo(P, decode_box_cols(P, img, cand));
+            const float4 b = tta_undo(P, decode_box_cols<T>(P, img, cand));
             float *t = tile + lane * rw + P.box_col;
             t[0] = b.x; t[1] = b.y; t[2] = b.z; t[3] = b.w;
             if (P.obj_col >= 0) {
-                const CandAddr ca = cand_addr(P, img, cand);
-                t[P.obj_col - P.box_col] = sigmoid_ref(__ldg(ca.obj));
+                const CandAddr<T> ca = cand_addr<T>(P, img, cand);
+                t[P.obj_col - P.box_col] = sigmoid_ref(ldg_head(ca.obj));
             }
         }
     }
@@ -174,27 +177,38 @@ __global__ void __launch_bounds__(kDecThreads) k_decode_rows(const __grid_consta
     }
 }
 
-template <int ROWS>
+template <int ROWS, typename T>
 static cudaError_t launch_decode_t(const Plan &P, float *d_out, int64_t rows_total, int64_t row_offset, cudaStream_t stream)
 {
     const size_t smem = static_cast<size_t>(ROWS) * P.row_w * sizeof(float);
     if (smem > 200 * 1024) return cudaErrorInvalidValue;
     if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(k_decode_rows<ROWS>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
+        cudaError_t e = cudaFuncSetAttribute(k_decode_rows<ROWS, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
         if (e != cudaSuccess) return e;
     }
     const dim3 grid((P.N + ROWS - 1) / ROWS, P.batch);
-    k_decode_rows<ROWS><<<grid, kDecThreads, smem, stream>>>(P, d_out, rows_total, row_offset);
+    k_decode_rows<ROWS, T><<<grid, kDecThreads, smem, stream>>>(P, d_out, rows_total, row_offset);
     return cudaGetLastError();
 }
 
+template <typename T>
+static cudaError_t launch_decode_dt(const Plan &P, float *d_out, int64_t rows_total, int64_t row_offset, cudaStream_t stream)
+{
+    if (P.layout == LAYOUT_PLANES && static_cast<size_t>(128) * P.row_w * sizeof(float) <= 100 * 1024)
+        return launch_decode_t<128, T>(P, d_out, rows_total, row_offset, stream);
+    return launch_decode_t<32, T>(P, d_out, rows_total, row_offset, stream);
+}
+
 // rows_total / row_offset: the pass fills rows [row_offset, row_offset + N) of a (batch, rows_total, C') tensor
-cudaError_t launch_decode(const Plan &P, float *d_out, int64_t rows_total, int64_t row_offset, cudaStream_t stream)
+cudaError_t launch_decode(const Plan &P, float *d_out, int64_t rows_total, int64_t row_offset, cudaStream_t stream,
+                          int dtype)
 {
     if (P.batch == 0 || P.N == 0) return cudaSuccess;
-    if (P.layout == LAYOUT_PLANES && static_cast<size_t>(128) * P.row_w * sizeof(float) <= 100 * 1024)
-        return launch_decode_t<128>(P, d_out, rows_total, row_offset, stream);
-    return launch_decode_t<32>(P, d_out, rows_total, row_offset, stream);
+    switch (dtype) {
+    case YSB_F16: return launch_decode_dt<__half>(P, d_out, rows_total, row_offset, stream);
+    case YSB_BF16: return launch_decode_dt<__nv_bfloat16>(P, d_out, rows_total, row_offset, stream);
+    default: return launch_decode_dt<float>(P, d_out, rows_total, row_offset, stream);
+    }
 }
 
 // Self-test: the spelled-out reciprocal of sigmoid_ref / sigmoid_fast against __frcp_rn for EVERY float in [1, +inf]

@@ -14,6 +14,10 @@
 // Output: one 64-bit sort key per survivor, written with warp-aggregated atomics (order inside an image is
 // irrelevant: the key carries the candidate index, see pack_key).
 //
+// Every kernel is templated on the head element type T (float, __half, __nv_bfloat16): values are widened to float32 as
+// they are loaded, so survivors, scores and classes are those of the float32 path on the widened heads.  The float
+// instantiations are the kernels of the float32-only engine, unchanged.
+//
 // Kernels in this file (dispatch: launch_filter at the bottom):
 //   k_filter_planes_v4     NCHW heads whose levels are all 128-bit loadable (YOLOv5 / YOLOX / YOLOv8)   -- product path
 //   k_filter_planes        NCHW heads with levels that are not (FCOS' 5x5 map); generic                   -- product path
@@ -56,10 +60,67 @@ __device__ __forceinline__ float ldg_stream1(const float *p)
     return v;
 }
 
+// 16-bit heads: four consecutive values are one 64-bit load (a warp reads 256 contiguous bytes per class plane), widened
+// to the float4 the float32 kernels work on.  Element 0 is the low half of the first word (little endian).
+__device__ __forceinline__ float4 widen4(uint2 r, const __half *)
+{
+    return make_float4(__half2float(__ushort_as_half(static_cast<unsigned short>(r.x & 0xffffu))),
+                       __half2float(__ushort_as_half(static_cast<unsigned short>(r.x >> 16))),
+                       __half2float(__ushort_as_half(static_cast<unsigned short>(r.y & 0xffffu))),
+                       __half2float(__ushort_as_half(static_cast<unsigned short>(r.y >> 16))));
+}
+__device__ __forceinline__ float4 widen4(uint2 r, const __nv_bfloat16 *)
+{
+    return make_float4(__uint_as_float(r.x << 16), __uint_as_float(r.x & 0xffff0000u), __uint_as_float(r.y << 16),
+                       __uint_as_float(r.y & 0xffff0000u));
+}
+template <typename T>
+__device__ __forceinline__ float4 ldg_stream4(const T *p)
+{
+    uint2 r;
+    asm volatile("ld.global.nc.L1::no_allocate.v2.u32 {%0,%1}, [%2];" : "=r"(r.x), "=r"(r.y) : "l"(p));
+    return widen4(r, p);
+}
+template <typename T>
+__device__ __forceinline__ float4 ldg_stream4_256(const T *p)
+{
+    uint2 r;
+    asm volatile("ld.global.nc.L1::no_allocate.L2::256B.v2.u32 {%0,%1}, [%2];" : "=r"(r.x), "=r"(r.y) : "l"(p));
+    return widen4(r, p);
+}
+// one raw 16-bit element (staged unconverted into the rows kernel's tile)
+template <typename T>
+__device__ __forceinline__ T ldg_stream1_raw(const T *p)
+{
+    unsigned short v;
+    asm volatile("ld.global.nc.L1::no_allocate.u16 %0, [%1];" : "=h"(v) : "l"(p));
+    return *reinterpret_cast<const T *>(&v);
+}
+__device__ __forceinline__ float ldg_stream1_raw(const float *p) { return ldg_stream1(p); }
+template <typename T>
+__device__ __forceinline__ float ldg_stream1(const T *p) { return widen(ldg_stream1_raw(p)); }
+
 __device__ __forceinline__ void top2_update(float c, int k, float &m1, float &m2, int &k0)
 {
     m2 = fmaxf(m2, fminf(m1, c));
     k0 = (c > m1) ? k : k0;
+    m1 = fmaxf(m1, c);
+}
+// 16-bit heads: exact ties of the largest logit are common (bfloat16 keeps 8 significant bits: ~1.5 % of dense
+// candidates), and with the update above every tie takes the literal re-evaluation (80 scattered re-reads), which halved
+// the bfloat16 throughput.  Here m2 is the largest value STRICTLY below m1 and k0 the lowest index holding m1 in any
+// visiting order.  Same result: when m2 < guard_lo every class value in the guard band equals m1, so the literal path
+// would score exactly those classes, all alike, and keep the lowest index -- k0, with score and smax of the fast path.
+// Distinct values inside the band still take the literal path.
+template <typename T>
+__device__ __forceinline__ void top2_update_t(float c, int k, float &m1, float &m2, int &k0)
+{
+    if (sizeof(T) == 4) {
+        top2_update(c, k, m1, m2, k0);
+        return;
+    }
+    m2 = (c < m1) ? fmaxf(m2, c) : ((c > m1) ? m1 : m2);
+    k0 = (c > m1 || (c == m1 && k < k0)) ? k : k0;
     m1 = fmaxf(m1, c);
 }
 
@@ -179,7 +240,7 @@ __device__ __forceinline__ void emit_keys(const uint64_t (&k)[VEC], unsigned okm
 // planes layout (NCHW heads: YOLOv5, YOLOX, YOLOv8, FCOS).  One thread = VEC consecutive positions of one
 // (image, anchor); per class plane a warp reads 32*VEC*4 contiguous bytes (512 B with 128-bit loads).
 // -------------------------------------------------------------------------------------------------------
-template <int VEC, int U = 8, int THREADS = 256, int MINB = 1, int HINT = 0, int PROBE = 0>
+template <typename T, int VEC, int U = 8, int THREADS = 256, int MINB = 1, int HINT = 0, int PROBE = 0>
 __global__ void __launch_bounds__(THREADS, MINB) k_filter_planes(const __grid_constant__ Plan P, uint64_t *__restrict__ keys,
                                                                  int64_t key_cap, int32_t *__restrict__ counts)
 {
@@ -201,7 +262,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_filter_planes(const __grid_co
         for (int i = 1; i < YSB_MAX_LEVELS; ++i)
             if (i < P.L && u >= P.lv[i].unit_off) l = i;
         const LevelDesc &lv = P.lv[l];
-        const bool vec4 = VEC == 4 && lv.vec == 4;  // levels whose planes are not 16-byte sized use one position per unit
+        const bool vec4 = VEC == 4 && lv.vec == 4;  // levels whose planes are not 4-element sized use one position per unit
         const int upos = vec4 ? 4 : 1;
         const int upa = lv.hw / upos;  // units per anchor
         const int ru = u - lv.unit_off;
@@ -209,7 +270,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_filter_planes(const __grid_co
         const int pos = (ru - a * upa) * upos;
         const int cand0 = lv.cand_off + a * lv.hw + pos;
         const size_t hw = static_cast<size_t>(lv.hw);
-        const float *cls = lv.p0 + (static_cast<size_t>(img * P.A + a) * P.cls_nch + P.cls_ch) * hw + pos;
+        const T *cls = head_ptr<T>(lv.p0) + (static_cast<size_t>(img * P.A + a) * P.cls_nch + P.cls_ch) * hw + pos;
 
         float m1[VEC], m2[VEC];
         int k0[VEC];
@@ -236,7 +297,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_filter_planes(const __grid_co
 #pragma unroll
                 for (int j = 0; j < VEC; ++j) {
                     if (PROBE) m1[j] = fmaxf(m1[j], v[q][j]);  // profiling aid: same loads, 1 ALU op per logit
-                    else top2_update(v[q][j], k + q, m1[j], m2[j], k0[j]);
+                    else top2_update_t<T>(v[q][j], k + q, m1[j], m2[j], k0[j]);
                 }
         }
         for (; k < P.C; ++k) {
@@ -250,14 +311,14 @@ __global__ void __launch_bounds__(THREADS, MINB) k_filter_planes(const __grid_co
                 for (int j = 1; j < VEC; ++j) v[j] = -INFINITY;
             }
 #pragma unroll
-            for (int j = 0; j < VEC; ++j) top2_update(v[j], k, m1[j], m2[j], k0[j]);
+            for (int j = 0; j < VEC; ++j) top2_update_t<T>(v[j], k, m1[j], m2[j], k0[j]);
         }
         float objv[VEC];
 #pragma unroll
         for (int j = 0; j < VEC; ++j) objv[j] = 0.0f;
         if (P.use_obj) {
-            const float *ob = (P.obj_src == 2 ? lv.p2 : lv.p0) +
-                              (static_cast<size_t>(img * P.A + a) * P.obj_nch + P.obj_ch) * hw + pos;
+            const T *ob = head_ptr<T>(P.obj_src == 2 ? lv.p2 : lv.p0) +
+                          (static_cast<size_t>(img * P.A + a) * P.obj_nch + P.obj_ch) * hw + pos;
             if (vec4) {
                 const float4 t = ldg_stream4(ob);
                 objv[0] = t.x; objv[1 % VEC] = t.y; objv[2 % VEC] = t.z; objv[3 % VEC] = t.w;
@@ -271,9 +332,9 @@ __global__ void __launch_bounds__(THREADS, MINB) k_filter_planes(const __grid_co
             float score;
             int c;
             bool pre;
-            const float *cj = cls + j;
+            const T *cj = cls + j;
             const bool ok = decide_candidate<false>(
-                P, m1[j], m2[j], k0[j], objv[j], [&](int kk) { return __ldg(cj + static_cast<size_t>(kk) * hw); },
+                P, m1[j], m2[j], k0[j], objv[j], [&](int kk) { return ldg_head(cj + static_cast<size_t>(kk) * hw); },
                 score, c, pre);
             npre += pre ? 1 : 0;
             if (ok) {
@@ -296,11 +357,11 @@ __global__ void __launch_bounds__(THREADS, MINB) k_filter_planes(const __grid_co
 //   * the last C % U class planes and the objectness plane are ONE batch of independent loads (the generic kernel walks
 //     the remainder one dependent load at a time and fetches objectness after the whole class scan).
 // -------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void prefetch_l2(const float *p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
+__device__ __forceinline__ void prefetch_l2(const void *p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 
 // PF > 0: while the loads of batch b are in flight, the lines of batch b + PF are requested into L2 with prefetch
 // instructions (no registers held): the demand loads of later batches then hit L2 instead of waiting a DRAM round trip.
-template <int U, int THREADS, int MINB, int PF = 0>
+template <typename T, int U, int THREADS, int MINB, int PF = 0>
 __global__ void __launch_bounds__(THREADS, MINB) k_filter_planes_v4(const __grid_constant__ Plan P, uint64_t *__restrict__ keys,
                                                                     int64_t key_cap, int32_t *__restrict__ counts)
 {
@@ -323,7 +384,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_filter_planes_v4(const __grid
         const int a = ru / upa;
         const int pos = (ru - a * upa) << 2;
         const int cand0 = lv.cand_off + a * lv.hw + pos;
-        const float *cls = lv.p0 + (static_cast<size_t>(img * P.A + a) * P.cls_nch + P.cls_ch) * hw + pos;
+        const T *cls = head_ptr<T>(lv.p0) + (static_cast<size_t>(img * P.A + a) * P.cls_nch + P.cls_ch) * hw + pos;
         const int C = P.C;
 
         float m1[4], m2[4], objv[4];
@@ -332,7 +393,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_filter_planes_v4(const __grid
         for (int j = 0; j < 4; ++j) { m1[j] = -INFINITY; m2[j] = -INFINITY; k0[j] = 0; objv[j] = 0.0f; }
 
         int k = 0;
-        uint32_t off = 0;  // k * hw, in elements: an (image, anchor) block is far below 2^32 floats
+        uint32_t off = 0;  // k * hw, in elements: an (image, anchor) block is far below 2^32 elements
         if (PF > 0 && (threadIdx.x & 7) == 0) {
             // prime the pipeline: batches 1 .. PF (8 lanes share a 128-byte line; one of them asks for it)
 #pragma unroll
@@ -350,14 +411,14 @@ __global__ void __launch_bounds__(THREADS, MINB) k_filter_planes_v4(const __grid
                     if (kk < C) prefetch_l2(cls + (off + ((PF + 1) * U + q) * hw));
                 }
                 if (P.use_obj && k == 0)
-                    prefetch_l2((P.obj_src == 2 ? lv.p2 : lv.p0) + (static_cast<size_t>(img * P.A + a) * P.obj_nch + P.obj_ch) * hw + pos);
+                    prefetch_l2(head_ptr<T>(P.obj_src == 2 ? lv.p2 : lv.p0) + (static_cast<size_t>(img * P.A + a) * P.obj_nch + P.obj_ch) * hw + pos);
             }
 #pragma unroll
             for (int q = 0; q < U; ++q) {
-                top2_update(v[q].x, k + q, m1[0], m2[0], k0[0]);
-                top2_update(v[q].y, k + q, m1[1], m2[1], k0[1]);
-                top2_update(v[q].z, k + q, m1[2], m2[2], k0[2]);
-                top2_update(v[q].w, k + q, m1[3], m2[3], k0[3]);
+                top2_update_t<T>(v[q].x, k + q, m1[0], m2[0], k0[0]);
+                top2_update_t<T>(v[q].y, k + q, m1[1], m2[1], k0[1]);
+                top2_update_t<T>(v[q].z, k + q, m1[2], m2[2], k0[2]);
+                top2_update_t<T>(v[q].w, k + q, m1[3], m2[3], k0[3]);
             }
         }
         {
@@ -366,8 +427,8 @@ __global__ void __launch_bounds__(THREADS, MINB) k_filter_planes_v4(const __grid
             float4 v[U];
             float4 ov = make_float4(0.f, 0.f, 0.f, 0.f);
             if (P.use_obj) {
-                const float *ob = (P.obj_src == 2 ? lv.p2 : lv.p0) +
-                                  (static_cast<size_t>(img * P.A + a) * P.obj_nch + P.obj_ch) * hw + pos;
+                const T *ob = head_ptr<T>(P.obj_src == 2 ? lv.p2 : lv.p0) +
+                              (static_cast<size_t>(img * P.A + a) * P.obj_nch + P.obj_ch) * hw + pos;
                 ov = ldg_stream4_256(ob);
             }
 #pragma unroll
@@ -376,10 +437,10 @@ __global__ void __launch_bounds__(THREADS, MINB) k_filter_planes_v4(const __grid
 #pragma unroll
             for (int q = 0; q < U - 1; ++q)
                 if (q < rem) {
-                    top2_update(v[q].x, k + q, m1[0], m2[0], k0[0]);
-                    top2_update(v[q].y, k + q, m1[1], m2[1], k0[1]);
-                    top2_update(v[q].z, k + q, m1[2], m2[2], k0[2]);
-                    top2_update(v[q].w, k + q, m1[3], m2[3], k0[3]);
+                    top2_update_t<T>(v[q].x, k + q, m1[0], m2[0], k0[0]);
+                    top2_update_t<T>(v[q].y, k + q, m1[1], m2[1], k0[1]);
+                    top2_update_t<T>(v[q].z, k + q, m1[2], m2[2], k0[2]);
+                    top2_update_t<T>(v[q].w, k + q, m1[3], m2[3], k0[3]);
                 }
             objv[0] = ov.x; objv[1] = ov.y; objv[2] = ov.z; objv[3] = ov.w;
         }
@@ -388,9 +449,9 @@ __global__ void __launch_bounds__(THREADS, MINB) k_filter_planes_v4(const __grid
             float score;
             int c;
             bool pre;
-            const float *cj = cls + j;
+            const T *cj = cls + j;
             const bool ok = decide_candidate<false>(
-                P, m1[j], m2[j], k0[j], objv[j], [&](int kk) { return __ldg(cj + static_cast<size_t>(kk) * hw); }, score, c, pre);
+                P, m1[j], m2[j], k0[j], objv[j], [&](int kk) { return ldg_head(cj + static_cast<size_t>(kk) * hw); }, score, c, pre);
             npre += pre ? 1 : 0;
             if (ok) {
                 out[j] = pack_key(score, static_cast<uint32_t>(P.cand_base + cand0 + j), static_cast<uint32_t>(c));
@@ -462,12 +523,18 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst_smem, const void *src_gmem
 // aligned individually, but the tile is contiguous and 16-byte aligned), then one thread scans one row: 128-bit shared
 // loads when the class run of every row is 16-byte aligned, else scalar loads; rows with an even stride are walked with
 // a per-thread rotation so that the rows a warp scans sit in different banks.
+// 16-bit heads are staged as they are (rows of 170 B / 160 B, 2-byte aligned) and widened as the scan reads them.  The
+// copy engines move 16-byte multiples from 16-byte aligned addresses, so a tile takes the bulk path when its first
+// element is 16-byte aligned and its length is a multiple of 16 bytes (8 elements here, 4 for float32): true for every
+// full tile of both layouts (128 rows x 170 B = 1360 x 16 B) and for every tail at a 640x640 input;
+// anything else is staged with scalar loads.
 // -------------------------------------------------------------------------------------------------------
 constexpr int kRowsTile = 128;
 
 // One thread scans one staged row (thread t of the tile -> row r0 + t of level lv), decides it and the warp appends the
 // survivors.  Every thread of the warp must call (rows beyond nrows contribute nothing).
-__device__ __forceinline__ void rows_scan_emit(const Plan &P, const LevelDesc &lv, int img, const float *tile, int sstride,
+template <typename T>
+__device__ __forceinline__ void rows_scan_emit(const Plan &P, const LevelDesc &lv, int img, const T *tile, int sstride,
                                                int nrows, int r0, int t, uint64_t *__restrict__ keys, int64_t key_cap,
                                                int32_t *__restrict__ counts, bool vec4 = false, const uint2 *ext_seen = nullptr)
 {
@@ -476,14 +543,14 @@ __device__ __forceinline__ void rows_scan_emit(const Plan &P, const LevelDesc &l
     int npre = 0;
     uint32_t smax_bits = 0u, smin_inv = 0u;
     if (t < nrows) {
-        const float *row = tile + t * sstride;
-        const float *cls = row + P.cls_col_in;
+        const T *row = tile + t * sstride;
+        const T *cls = row + P.cls_col_in;
         float m1 = -INFINITY, m2 = -INFINITY;
         int k0 = 0;
         // thread t reads word sstride*t + k: conflict-free when sstride is odd; otherwise start the walk at column t so
         // that the 32 lanes hit (sstride+1)*t + k.  The visiting order is irrelevant: a unique maximum has a unique
         // index, and equal maxima force m2 == m1, i.e. the literal path, which walks in index order.
-        if (vec4 && ((sstride | P.cls_col_in | P.C) & 3) == 0) {
+        if (sizeof(T) == 4 && vec4 && ((sstride | P.cls_col_in | P.C) & 3) == 0) {
             // 16-byte aligned class runs (RetinaNet's 80-float rows, 84-float decoded rows): 128-bit shared loads, four
             // independent (max, runner-up, position) chains -- one per float4 component -- that share the float4's
             // position, merged at the end.  A quarter-warp reads 8 float4 per wavefront: with an even number of float4 per
@@ -517,7 +584,7 @@ __device__ __forceinline__ void rows_scan_emit(const Plan &P, const LevelDesc &l
         } else if (sstride & 1) {
             // odd stride (YOLOv7's 85-float rows): already conflict-free, a straight run without the wrap test
 #pragma unroll 8
-            for (int k = 0; k < P.C; ++k) top2_update(cls[k], k, m1, m2, k0);
+            for (int k = 0; k < P.C; ++k) top2_update_t<T>(widen(cls[k]), k, m1, m2, k0);
         } else {
             // rotated walk: lane l starts at column l, i.e. reads word sstride*tid + l + t = (sstride + 1)*l + t (mod 32)
             // -- an odd multiplier, conflict-free.  Every lane runs the same C iterations (two straight runs per lane
@@ -526,18 +593,18 @@ __device__ __forceinline__ void rows_scan_emit(const Plan &P, const LevelDesc &l
             if (P.C >= 32) {
                 const int straight = P.C - 32;
 #pragma unroll 8
-                for (int t = 0; t < straight; ++t) top2_update(cls[t + lane], t + lane, m1, m2, k0);
+                for (int t = 0; t < straight; ++t) top2_update_t<T>(widen(cls[t + lane]), t + lane, m1, m2, k0);
                 int k = straight + lane;
 #pragma unroll 8
                 for (int t = 0; t < 32; ++t) {
                     if (k >= P.C) k -= P.C;
-                    top2_update(cls[k], k, m1, m2, k0);
+                    top2_update_t<T>(widen(cls[k]), k, m1, m2, k0);
                     ++k;
                 }
             } else {
                 int k = lane % P.C;
                 for (int t = 0; t < P.C; ++t) {
-                    top2_update(cls[k], k, m1, m2, k0);
+                    top2_update_t<T>(widen(cls[k]), k, m1, m2, k0);
                     if (++k == P.C) k = 0;
                 }
             }
@@ -546,17 +613,17 @@ __device__ __forceinline__ void rows_scan_emit(const Plan &P, const LevelDesc &l
         float objv = 0.0f;
         if (P.use_obj) {
             if (P.obj_src == 1)  // RetinaNet-exp: conf logit is the last column of the reg tensor
-                objv = __ldg(P.lv[0].p1 + (static_cast<size_t>(img) * P.N + cand) * P.reg_row_w + 4);
+                objv = ldg_head(head_ptr<T>(P.lv[0].p1) + (static_cast<size_t>(img) * P.N + cand) * P.reg_row_w + 4);
             else
-                objv = row[P.obj_col_in];
+                objv = widen(row[P.obj_col_in]);
         }
         float score;
         int c;
         bool pre, ok;
         if (P.input_kind == YSB_INPUT_DECODED_ROWS)
-            ok = decide_candidate<true>(P, m1, m2, k0, objv, [&](int kk) { return cls[kk]; }, score, c, pre);
+            ok = decide_candidate<true>(P, m1, m2, k0, objv, [&](int kk) { return widen(cls[kk]); }, score, c, pre);
         else
-            ok = decide_candidate<false>(P, m1, m2, k0, objv, [&](int kk) { return cls[kk]; }, score, c, pre);
+            ok = decide_candidate<false>(P, m1, m2, k0, objv, [&](int kk) { return widen(cls[kk]); }, score, c, pre);
         npre = pre ? 1 : 0;
         if (ok) {
             out[0] = pack_key(score, static_cast<uint32_t>(P.cand_base + cand), static_cast<uint32_t>(c));
@@ -569,10 +636,13 @@ __device__ __forceinline__ void rows_scan_emit(const Plan &P, const LevelDesc &l
                  counts + img * 4, P.pre_kind == PRE_ANY_GT, ext_seen);
 }
 
+template <typename T>
 __global__ void __launch_bounds__(kRowsTile) k_filter_rows(const __grid_constant__ Plan P, uint64_t *__restrict__ keys,
                                                            int64_t key_cap, int32_t *__restrict__ counts, int flags)
 {
-    extern __shared__ __align__(128) float tile[];
+    extern __shared__ __align__(128) float tile_f[];
+    T *tile = reinterpret_cast<T *>(tile_f);
+    constexpr int kVecShift = sizeof(T) == 4 ? 2 : 3;   // log2 of the elements in 16 bytes
     const int img = blockIdx.x;  // image fastest: see k_filter_planes
     const int t = blockIdx.y;
     int l = 0;
@@ -584,7 +654,7 @@ __global__ void __launch_bounds__(kRowsTile) k_filter_rows(const __grid_constant
     const int r0 = (t - lv.unit_off) * kRowsTile;
     const int nrows = min(kRowsTile, rows_l - r0);
     const int rw = P.row_w_in;
-    const float *src = lv.p0 + (static_cast<size_t>(img) * lv.img_rows + r0) * rw;
+    const T *src = head_ptr<T>(lv.p0) + (static_cast<size_t>(img) * lv.img_rows + r0) * rw;
     const int nfl = nrows * rw;
     // the image's running score extrema, read now so that the load hides behind the staging copy (see emit_keys)
     const volatile unsigned int *ext_p = reinterpret_cast<const volatile unsigned int *>(counts + img * 4 + 2);
@@ -592,12 +662,12 @@ __global__ void __launch_bounds__(kRowsTile) k_filter_rows(const __grid_constant
     // 16-byte aligned tiles (every reference layout): cp.async straight into a DENSE shared tile -- no register
     // staging, no per-element address math.  Rows with an even float stride are scanned with a per-thread rotation
     // (below) instead of padding.  Odd shapes: scalar loads into a tile padded to an odd stride.
-    const bool dense = ((reinterpret_cast<uintptr_t>(src) & 15u) == 0) && ((nfl & 3) == 0);
+    const bool dense = ((reinterpret_cast<uintptr_t>(src) & 15u) == 0) && ((nfl & ((1 << kVecShift) - 1)) == 0);
     const int sstride = dense ? rw : (rw | 1);
     if (dense && !(flags & 1)) {
         const uint32_t dst = smem_u32(tile);
-        const int nv = nfl >> 2;
-        for (int i = threadIdx.x; i < nv; i += kRowsTile) cp_async16(dst + 16u * i, src + 4 * i);
+        const int nv = nfl >> kVecShift;
+        for (int i = threadIdx.x; i < nv; i += kRowsTile) cp_async16(dst + 16u * i, src + (1 << kVecShift) * i);
         cp_async_commit();
         cp_async_wait<0>();
     } else if (dense) {
@@ -608,15 +678,15 @@ __global__ void __launch_bounds__(kRowsTile) k_filter_rows(const __grid_constant
         if (threadIdx.x == 0) {
             mbar_init(b32, 1);
             asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-            mbar_expect_tx(b32, static_cast<uint32_t>(nfl) * 4u);
-            bulk_g2s(smem_u32(tile), src, static_cast<uint32_t>(nfl) * 4u, b32);
+            mbar_expect_tx(b32, static_cast<uint32_t>(nfl) * static_cast<uint32_t>(sizeof(T)));
+            bulk_g2s(smem_u32(tile), src, static_cast<uint32_t>(nfl) * static_cast<uint32_t>(sizeof(T)), b32);
         }
         __syncthreads();   // the barrier is initialised before anybody polls it
         mbar_wait(b32, 0u);
     } else {
         for (int e = threadIdx.x; e < nfl; e += kRowsTile) {
             const int row = e / rw, col = e - row * rw;
-            tile[row * sstride + col] = ldg_stream1(src + e);
+            tile[row * sstride + col] = ldg_stream1_raw(src + e);
         }
     }
     __syncthreads();
@@ -732,6 +802,7 @@ __global__ void __launch_bounds__(kRowsTile) k_filter_rows_ring(const __grid_con
 // eval_fcos.py:246-250).  False in every shipped yaml, so this kernel favours simplicity: one thread per candidate,
 // every class evaluated literally (sigmoid, multiply) twice -- once to count, once to write -- any input layout.
 // -------------------------------------------------------------------------------------------------------
+template <typename T>
 __global__ void __launch_bounds__(256) k_filter_multilabel(const __grid_constant__ Plan P, uint64_t *__restrict__ keys,
                                                            int64_t key_cap, int32_t *__restrict__ counts)
 {
@@ -739,7 +810,7 @@ __global__ void __launch_bounds__(256) k_filter_multilabel(const __grid_constant
     const int cand = blockIdx.y * blockDim.x + threadIdx.x;
     const bool active = cand < P.N;
     const bool decoded = P.input_kind == YSB_INPUT_DECODED_ROWS;
-    const float *cls = nullptr;
+    const T *cls = nullptr;
     size_t cstride = 1;
     float mult = 1.0f;
     if (active) {
@@ -749,21 +820,21 @@ __global__ void __launch_bounds__(256) k_filter_multilabel(const __grid_constant
         float objv = 0.0f;
         if (P.layout == LAYOUT_PLANES) {
             const int a = r / lv.hw, pos = r - a * lv.hw;
-            cls = lv.p0 + (static_cast<size_t>(img * P.A + a) * P.cls_nch + P.cls_ch) * lv.hw + pos;
+            cls = head_ptr<T>(lv.p0) + (static_cast<size_t>(img * P.A + a) * P.cls_nch + P.cls_ch) * lv.hw + pos;
             cstride = static_cast<size_t>(lv.hw);
             if (P.use_obj)
-                objv = __ldg((P.obj_src == 2 ? lv.p2 : lv.p0) + (static_cast<size_t>(img * P.A + a) * P.obj_nch + P.obj_ch) * lv.hw + pos);
+                objv = ldg_head(head_ptr<T>(P.obj_src == 2 ? lv.p2 : lv.p0) + (static_cast<size_t>(img * P.A + a) * P.obj_nch + P.obj_ch) * lv.hw + pos);
         } else {
-            const float *row = lv.p0 + (static_cast<size_t>(img) * lv.img_rows + r) * P.row_w_in;
+            const T *row = head_ptr<T>(lv.p0) + (static_cast<size_t>(img) * lv.img_rows + r) * P.row_w_in;
             cls = row + P.cls_col_in;
             if (P.use_obj)
-                objv = P.obj_src == 1 ? __ldg(P.lv[0].p1 + (static_cast<size_t>(img) * P.N + cand) * P.reg_row_w + 4)
-                                      : __ldg(row + P.obj_col_in);
+                objv = P.obj_src == 1 ? ldg_head(head_ptr<T>(P.lv[0].p1) + (static_cast<size_t>(img) * P.N + cand) * P.reg_row_w + 4)
+                                      : ldg_head(row + P.obj_col_in);
         }
         if (P.use_obj) mult = decoded ? objv : sigmoid_ref(objv);
     }
     auto score_of = [&](int k, float &sk) {
-        const float c = __ldg(cls + static_cast<size_t>(k) * cstride);
+        const float c = ldg_head(cls + static_cast<size_t>(k) * cstride);
         sk = decoded ? c : sigmoid_ref(c);
         return P.use_obj ? __fmul_rn(sk, mult) : sk;
     };
@@ -839,21 +910,18 @@ __global__ void __launch_bounds__(256) k_filter_multilabel(const __grid_constant
 #include "filter_variants_launch.inc"
 #endif
 
-// zero_counts = false: append to the key lists / counters a previous pass left (test-time-augmentation passes)
-cudaError_t launch_filter(const Plan &P, int vec, uint64_t *d_keys, int64_t key_cap, int32_t *d_counts,
-                          cudaStream_t stream, bool zero_counts)
+template <typename T>
+static cudaError_t launch_filter_t(const Plan &P, int vec, uint64_t *d_keys, int64_t key_cap, int32_t *d_counts,
+                                   cudaStream_t stream)
 {
     cudaError_t e = cudaSuccess;
-    if (zero_counts) e = cudaMemsetAsync(d_counts, 0, sizeof(int32_t) * 4 * static_cast<size_t>(P.batch), stream);
-    if (e != cudaSuccess) return e;
-    if (P.batch == 0 || P.N == 0) return cudaSuccess;
     if (P.multi_label) {
         const dim3 grid(P.batch, (P.N + 255) / 256);
-        k_filter_multilabel<<<grid, 256, 0, stream>>>(P, d_keys, key_cap, d_counts);
+        k_filter_multilabel<T><<<grid, 256, 0, stream>>>(P, d_keys, key_cap, d_counts);
         return cudaGetLastError();
     }
 #ifdef YSB_PROFILING_VARIANTS
-    {
+    if (sizeof(T) == 4) {   // the variants read float32 heads; 16-bit heads always run the product kernels
         bool handled = false;
         e = launch_filter_variant(P, vec, d_keys, key_cap, d_counts, stream, &handled);
         if (handled) return e;
@@ -866,33 +934,33 @@ cudaError_t launch_filter(const Plan &P, int vec, uint64_t *d_keys, int64_t key_
             // 80 classes + objectness = 9 batches of 9), 76 registers, 6 CTAs of 128 threads per SM
             const dim3 gv4(P.batch, (P.units_per_img + 127) / 128);
 #ifdef YSB_PROFILING_VARIANTS
-            {   // profiling build: YSB_K1_CARVEOUT=<percent of the SM's shared memory> as the kernel's preferred carve-out
+            if (sizeof(T) == 4) {   // profiling build: YSB_K1_CARVEOUT=<percent of the SM's shared memory> as the kernel's preferred carve-out
                 static int pct = -2;
                 if (pct == -2) { const char *ev = getenv("YSB_K1_CARVEOUT"); pct = ev ? atoi(ev) : -1; }
                 if (pct >= 0) {
-                    e = cudaFuncSetAttribute(k_filter_planes_v4<9, 128, 6>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
+                    e = cudaFuncSetAttribute(k_filter_planes_v4<T, 9, 128, 6>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
                     if (e != cudaSuccess) return e;
                 }
             }
 #endif
-            k_filter_planes_v4<9, 128, 6><<<gv4, 128, 0, stream>>>(P, d_keys, key_cap, d_counts);
+            k_filter_planes_v4<T, 9, 128, 6><<<gv4, 128, 0, stream>>>(P, d_keys, key_cap, d_counts);
         } else if (vec == 1) {
             const dim3 grid(P.batch, (P.units_per_img + 255) / 256);
-            k_filter_planes<1><<<grid, 256, 0, stream>>>(P, d_keys, key_cap, d_counts);
+            k_filter_planes<T, 1><<<grid, 256, 0, stream>>>(P, d_keys, key_cap, d_counts);
         } else {
             // levels that are not all 128-bit loadable (FCOS' 5x5 map): generic kernel, 128-thread CTAs, 12 loads of
             // 128 bits in flight per thread (96 registers, 5 CTAs/SM), 256-byte L2 prefetch
             const dim3 grid128(P.batch, (P.units_per_img + 127) / 128);
-            k_filter_planes<4, 12, 128, 5, 1><<<grid128, 128, 0, stream>>>(P, d_keys, key_cap, d_counts);
+            k_filter_planes<T, 4, 12, 128, 5, 1><<<grid128, 128, 0, stream>>>(P, d_keys, key_cap, d_counts);
         }
     } else {
-        const size_t smem = static_cast<size_t>(kRowsTile) * (P.row_w_in | 1) * sizeof(float);
+        const size_t smem = static_cast<size_t>(kRowsTile) * (P.row_w_in | 1) * sizeof(T);
 #ifdef YSB_PROFILING_VARIANTS
         // persistent ring kernel when two CTAs with kRingStages tiles each fit an SM and the tensors allow bulk copies
         // (16-byte aligned bases, image strides that keep every image's first row 16-byte aligned)
         static int ring_env = -1;
         if (ring_env < 0) { const char *ev = getenv("YSB_ROWS_RING"); ring_env = ev ? atoi(ev) : 0; }
-        bool ring_ok = ring_env != 0 && kRingStages * smem <= 110u * 1024u;
+        bool ring_ok = sizeof(T) == 4 && ring_env != 0 && kRingStages * smem <= 110u * 1024u;
         for (int l = 0; l < P.L && ring_ok; ++l)
             ring_ok = (reinterpret_cast<uintptr_t>(P.lv[l].p0) & 15u) == 0 &&
                       ((static_cast<long long>(P.lv[l].img_rows) * P.row_w_in) & 3) == 0;
@@ -920,16 +988,31 @@ cudaError_t launch_filter(const Plan &P, int vec, uint64_t *d_keys, int64_t key_
         {
             static int fenv = -2;
             if (fenv == -2) { const char *ev = getenv("YSB_ROWS_FLAGS"); fenv = ev ? atoi(ev) : -1; }
-            if (fenv >= 0) flags = fenv;
+            if (fenv >= 0 && sizeof(T) == 4) flags = fenv;
         }
 #endif
         if (smem > 48 * 1024) {
-            e = cudaFuncSetAttribute(k_filter_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
+            e = cudaFuncSetAttribute(k_filter_rows<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
             if (e != cudaSuccess) return e;
         }
-        k_filter_rows<<<grid, kRowsTile, smem, stream>>>(P, d_keys, key_cap, d_counts, flags);
+        k_filter_rows<T><<<grid, kRowsTile, smem, stream>>>(P, d_keys, key_cap, d_counts, flags);
     }
     return cudaGetLastError();
+}
+
+// zero_counts = false: append to the key lists / counters a previous pass left (test-time-augmentation passes)
+cudaError_t launch_filter(const Plan &P, int vec, uint64_t *d_keys, int64_t key_cap, int32_t *d_counts,
+                          cudaStream_t stream, bool zero_counts, int dtype)
+{
+    cudaError_t e = cudaSuccess;
+    if (zero_counts) e = cudaMemsetAsync(d_counts, 0, sizeof(int32_t) * 4 * static_cast<size_t>(P.batch), stream);
+    if (e != cudaSuccess) return e;
+    if (P.batch == 0 || P.N == 0) return cudaSuccess;
+    switch (dtype) {
+    case YSB_F16: return launch_filter_t<__half>(P, vec, d_keys, key_cap, d_counts, stream);
+    case YSB_BF16: return launch_filter_t<__nv_bfloat16>(P, vec, d_keys, key_cap, d_counts, stream);
+    default: return launch_filter_t<float>(P, vec, d_keys, key_cap, d_counts, stream);
+    }
 }
 
 }  // namespace ysb

@@ -51,7 +51,7 @@ void check_cuda(const at::Tensor &t, at::ScalarType dtype, const c10::Device &de
     TORCH_CHECK_VALUE(t.is_contiguous(), name, ": expected a contiguous tensor");
 }
 
-// heads -> array of device pointers; every head float32, contiguous, on one device
+// heads -> array of device pointers; every head of one dtype, contiguous, on one device
 std::vector<const void *> head_pointers(const at::TensorList &heads, c10::Device &dev)
 {
     TORCH_CHECK_VALUE(!heads.empty(), "heads: no tensors");
@@ -59,10 +59,24 @@ std::vector<const void *> head_pointers(const at::TensorList &heads, c10::Device
     std::vector<const void *> p;
     p.reserve(heads.size());
     for (const auto &h : heads) {
-        check_cuda(h, at::kFloat, dev, "heads");
+        check_cuda(h, heads[0].scalar_type(), dev, "heads");
         p.push_back(h.data_ptr());
     }
     return p;
+}
+
+// the heads' dtype is the one the params announce (ysb_params.head_dtype: float32, float16 or bfloat16)
+void check_head_dtype(const at::TensorList &heads, const ysb_params *p)
+{
+    at::ScalarType want = at::kFloat;
+    switch (p->head_dtype) {
+    case YSB_F32: break;
+    case YSB_F16: want = at::kHalf; break;
+    case YSB_BF16: want = at::kBFloat16; break;
+    default: TORCH_CHECK_VALUE(false, "params: unknown head_dtype ", p->head_dtype);
+    }
+    TORCH_CHECK_VALUE(heads[0].scalar_type() == want, "heads: expected ", want, " (params.head_dtype), got ",
+                      heads[0].scalar_type());
 }
 
 void *current_stream(const c10::Device &dev) { return at::cuda::getCurrentCUDAStream(dev.index()).stream(); }
@@ -74,6 +88,7 @@ void postprocess(at::TensorList heads, const at::Tensor &params, at::Tensor work
     c10::Device dev(c10::kCUDA, 0);
     const auto ptrs = head_pointers(heads, dev);
     const ysb_params *p = params_of(params);
+    check_head_dtype(heads, p);
     check_cuda(workspace, at::kByte, dev, "workspace");
     check_cuda(dets, at::kFloat, dev, "dets");
     check_cuda(det_idx, at::kInt, dev, "det_idx");
@@ -93,6 +108,7 @@ void filter_candidates(at::TensorList heads, const at::Tensor &params, at::Tenso
     c10::Device dev(c10::kCUDA, 0);
     const auto ptrs = head_pointers(heads, dev);
     const ysb_params *p = params_of(params);
+    check_head_dtype(heads, p);
     check_cuda(keys, at::kLong, dev, "keys");
     check_cuda(counts, at::kInt, dev, "counts");
     TORCH_CHECK_VALUE(keys.dim() == 2 && keys.size(0) == p->batch && counts.numel() >= 4 * static_cast<int64_t>(p->batch),
@@ -110,6 +126,7 @@ void select_nms(at::TensorList heads, const at::Tensor &params, const at::Tensor
     c10::Device dev(c10::kCUDA, 0);
     const auto ptrs = head_pointers(heads, dev);
     const ysb_params *p = params_of(params);
+    check_head_dtype(heads, p);
     check_cuda(keys, at::kLong, dev, "keys");
     check_cuda(counts, at::kInt, dev, "counts");
     check_cuda(dets, at::kFloat, dev, "dets");
@@ -133,6 +150,7 @@ at::Tensor decode(at::TensorList heads, const at::Tensor &params)
     c10::Device dev(c10::kCUDA, 0);
     const auto ptrs = head_pointers(heads, dev);
     const ysb_params *p = params_of(params);
+    check_head_dtype(heads, p);
     int64_t n = 0;
     int32_t row_w = 0;
     check_status(ysb_num_candidates(p, &n, &row_w), "ysb_num_candidates");
@@ -149,6 +167,7 @@ void decode_into(at::TensorList heads, const at::Tensor &params, at::Tensor merg
     c10::Device dev(c10::kCUDA, 0);
     const auto ptrs = head_pointers(heads, dev);
     const ysb_params *p = params_of(params);
+    check_head_dtype(heads, p);
     check_cuda(merged, at::kFloat, dev, "merged");
     TORCH_CHECK_VALUE(merged.dim() == 3 && merged.size(0) == p->batch, "merged must be (batch, rows_total, C')");
     c10::cuda::CUDAGuard guard(dev);

@@ -210,7 +210,8 @@ class ShardedPostProcessor:
     writes over NVLink, flow control by two tiny kernels); 'nccl': one all_gather_into_tensor per batch on the lane's
     stream (fallback when CUDA IPC is unavailable); world == 1: plain local buffers.  With ``graph`` (default: batch <=
     16) the per-lane launch sequence is captured once per set of head tensors and replayed.
-    A ticket's buffers are reused ``lanes`` submissions later.
+    A ticket's buffers are reused ``lanes`` submissions later.  The heads may be float32, float16 or bfloat16; the first
+    submission fixes the type, and a later batch of another type raises ValueError.
     """
 
     def __init__(self, family, hyp, batch, img_h, img_w, anchors=None, lanes=None, group=None, gather="auto", graph=None,
@@ -256,6 +257,7 @@ class ShardedPostProcessor:
         if self._ent is not None:
             return
         self._ent = self.pp._prepare(flat, self.batch, self.img_h, self.img_w, _lib.INPUT_RAW_HEADS)
+        self._head_dtype = flat[0].dtype
         n = self._ent["N"] * (int(self.pp.hyp["num_class"]) if self.pp.hyp["mutil_label"] else 1)
         self._key_cap = n
         b, d, dev = self.batch, self.max_det, self.device
@@ -327,6 +329,8 @@ class ShardedPostProcessor:
         if flat[0].shape[0] != self.batch:
             raise ValueError(f"expected {self.batch} images per rank, got {flat[0].shape[0]}")
         self._prepare(flat)
+        if any(t.dtype != self._head_dtype for t in flat):
+            raise ValueError(f"this processor was set up for {self._head_dtype} heads, got {sorted({str(t.dtype) for t in flat})}")
         lane = self._next % self.lanes
         self._next += 1
         st = self.streams[lane]

@@ -12,6 +12,9 @@ import torch
 from . import _lib, _ops
 from ._lib import YsbParams
 
+# element types the raw heads may have (ysb_dtype): 16-bit heads are read as they are and widened on the device
+HEAD_DTYPES = {torch.float32: _lib.DTYPE_F32, torch.float16: _lib.DTYPE_F16, torch.bfloat16: _lib.DTYPE_BF16}
+
 # strides fixed by the reference evaluators (self.ds_scales), trainer/eval_yolov5.py:21, eval_yolov7.py, eval_fcos.py:18
 _FIXED_STRIDES = {"yolov5": (8, 16, 32), "yolov7": (8, 16, 32), "fcos": (8, 16, 32, 64, 128)}
 
@@ -64,6 +67,24 @@ def normalise_heads(heads):
     return type(heads)(normalise_heads(v) for v in heads)
 
 
+def _leaves(heads):
+    if isinstance(heads, torch.Tensor):
+        return [heads]
+    if isinstance(heads, (dict, OrderedDict)):
+        heads = heads.values()
+    return [t for v in heads for t in _leaves(v)]
+
+
+def native_heads(heads):
+    """Model outputs as the engine takes them: unchanged when every tensor is contiguous and all share one of float32,
+    float16 or bfloat16 (16-bit heads are read natively, no conversion pass); anything else goes through
+    normalise_heads."""
+    leaves = _leaves(heads)
+    if leaves and leaves[0].dtype in HEAD_DTYPES and all(t.dtype == leaves[0].dtype and t.is_contiguous() for t in leaves):
+        return heads
+    return normalise_heads(heads)
+
+
 def _level_shapes(family, flat, num_class):
     if family in ("yolov5", "yolox", "yolov8"):
         return [(t.shape[-2], t.shape[-1]) for t in flat]
@@ -76,13 +97,16 @@ def _level_shapes(family, flat, num_class):
 
 
 def make_params(family, hyp, batch, img_h, img_w, level_shapes=None, anchors=None, input_kind=_lib.INPUT_RAW_HEADS,
-                compute_metric=False, num_anchors=None, decoded_rows=0, tta=None):
+                compute_metric=False, num_anchors=None, decoded_rows=0, tta=None, head_dtype=torch.float32):
     """Build ``ysb_params`` from the reference's flat ``hyp`` dict (SURVEY.md section 5 lists the keys).
 
     ``tta`` = (scale, flip_axis, org_h, org_w) describes one test-time-augmentation pass (trainer/eval_yolov5.py:152-179):
     the boxes decoded from this pass's heads are divided by ``scale`` and un-flipped (axis 2 or 3) against the size of
-    the un-augmented input."""
+    the un-augmented input.  ``head_dtype``: element type of the raw heads, torch.float32 / float16 / bfloat16."""
+    if head_dtype not in HEAD_DTYPES:
+        raise ValueError(f"head_dtype must be one of {sorted(map(str, HEAD_DTYPES))}, got {head_dtype}")
     p = YsbParams()
+    p.head_dtype = HEAD_DTYPES[head_dtype]
     p.family = _lib.FAMILY_IDS[family]
     p.input_kind = input_kind
     p.batch = int(batch)
@@ -216,13 +240,18 @@ def validate_heads(family, flat, num_class, anchors=None, dfl_bins=16, decoded_r
         bad("no tensors")
     b = flat[0].shape[0]
     for i, t in enumerate(flat):
-        if t.dtype != torch.float32 or not t.is_contiguous():
-            raise ValueError("head tensors must be contiguous float32")
+        if t.dtype not in HEAD_DTYPES or not t.is_contiguous():
+            raise ValueError(f"head tensors must be contiguous float32, float16 or bfloat16, got {t.dtype}")
+        if t.dtype != flat[0].dtype:
+            raise ValueError(f"head tensors must share one dtype (contiguous float32, float16 or bfloat16), got "
+                             f"{flat[0].dtype} and {t.dtype}")
         if t.dim() < 2 or t.shape[0] != b:
             bad(f"tensor {i} has batch {tuple(t.shape)[:1]}, expected {b}")
         if t.device != flat[0].device:
             bad("tensors live on different devices")
     if decoded_row_w is not None:
+        if flat[0].dtype != torch.float32:
+            raise ValueError(f"decoded tensor must be contiguous float32, got {flat[0].dtype}")
         if len(flat) != 1 or flat[0].dim() != 3 or flat[0].shape[2] != decoded_row_w:
             raise ValueError(f"decoded tensor must be (b, N, {decoded_row_w}), got {tuple(flat[0].shape)}")
         return
@@ -312,11 +341,11 @@ class PostProcessor:
             shapes = [(img_h // s, img_w // s) for s in strides]
         na = flat[0].shape[1] if (self.family == "yolox" and input_kind == _lib.INPUT_RAW_HEADS) else None
         rows = int(flat[0].shape[1]) if input_kind == _lib.INPUT_DECODED_ROWS else 0
-        key = (batch, img_h, img_w, input_kind, tuple(shapes or ()), dev.index, na, rows, tta)
+        key = (batch, img_h, img_w, input_kind, tuple(shapes or ()), dev.index, na, rows, tta, flat[0].dtype)
         ent = self._cache.get(key)
         if ent is None:
             params = make_params(self.family, self.hyp, batch, img_h, img_w, shapes, self.anchors, input_kind,
-                                 self.compute_metric, na, rows, tta)
+                                 self.compute_metric, na, rows, tta, flat[0].dtype)
             n = ctypes.c_int64()
             rw = ctypes.c_int32()
             _lib.check(self._lib.ysb_num_candidates(ctypes.byref(params), ctypes.byref(n), ctypes.byref(rw)),
@@ -341,7 +370,7 @@ class PostProcessor:
 
     # ---- public ops ----------------------------------------------------------------------------------------
     def decode(self, heads, img_h, img_w):
-        """do_inference: raw heads -> (b, N, C') float32 on the heads' device."""
+        """do_inference: raw heads (float32, float16 or bfloat16) -> (b, N, C') float32 on the heads' device."""
         flat = flatten_heads(self.family, heads)
         batch = flat[0].shape[0]
         ent = self._prepare(flat, batch, img_h, img_w, _lib.INPUT_RAW_HEADS)

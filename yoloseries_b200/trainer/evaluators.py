@@ -10,14 +10,15 @@
 
 ``__call__(inputs)`` returns ``list[Tensor(K,6) | None]`` -- CPU float32 rows [xmin, ymin, xmax, ymax, score, cls] in NMS
 keep order, ``None`` where the reference returns ``None`` (SURVEY.md 8a-4.3).  Without TTA the model's raw heads go
-straight into the fused CUDA path (no (b, N, C') tensor is ever written); ``do_inference`` / ``numba_nms`` remain
+straight into the fused CUDA path (no (b, N, C') tensor is ever written); contiguous float16 / bfloat16 heads (hyp['half'])
+are read as they are, with results bit-identical to their float32 widening.  ``do_inference`` / ``numba_nms`` remain
 available separately with the reference's signatures.  Everything heavy runs in libysb_postproc.so; there is no CPU path.
 """
 import numpy as np
 import torch
 import torch.nn.functional as F
 
-from ..engine import PostProcessor, normalise_heads
+from ..engine import PostProcessor, native_heads
 
 __all__ = ["YOLOV5Evaluator", "YOLOV7Evaluator", "YOLOXEvaluator", "YOLOV8Evaluator", "RetinaNetEvaluator",
            "RetinaNetEvaluatorExperiment", "FCOSEvaluator"]
@@ -53,14 +54,14 @@ class _Evaluator:
             # three model forwards, then ONE fused call: no decoded or merged tensor is written (ysb_postprocess_tta)
             out = self._pp.run_tta(self._tta_passes(inputs), (inputs.size(2), inputs.size(3)), info=info)
             return self._pp.to_list(out)
-        heads = normalise_heads(self._model(inputs))
+        heads = native_heads(self._model(inputs))
         out = self._pp.run(heads, inputs.size(2), inputs.size(3), info=info)
         return self._pp.to_list(out)
 
     @torch.no_grad()
     def do_inference(self, inputs):
         """model forward + decode -> (b, N, C') float32 on the heads' device (one CUDA kernel, ysb_decode)."""
-        heads = normalise_heads(self._model(inputs))
+        heads = native_heads(self._model(inputs))
         return self._pp.decode(heads, inputs.size(2), inputs.size(3))
 
     def numba_nms(self, preds_out):
@@ -135,7 +136,7 @@ class _Evaluator:
         for s, f in zip([1, 0.83, 0.67], [None, 2, 3]):
             img = inputs.flip(dims=(f,)) if f else inputs
             img = self.scale_img(img, s)
-            passes.append((normalise_heads(self._model(img)), img.size(2), img.size(3), s, f))
+            passes.append((native_heads(self._model(img)), img.size(2), img.size(3), s, f))
         return passes
 
     def test_time_augmentation(self, inputs):
