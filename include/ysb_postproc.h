@@ -200,6 +200,19 @@ int ysb_postprocess_tta_workspace_bytes(const ysb_params *passes, int num_passes
 int ysb_postprocess_tta(const ysb_params *passes, int num_passes, const void *const *d_heads, const int32_t *heads_per_pass,
                         void *d_workspace, size_t workspace_bytes, float *d_dets, int32_t *d_det_idx,
                         int32_t *d_det_cnt, void *stream);
+/* The two halves of ysb_postprocess_tta, for callers that own their key buffers (the pass list follows the same rules).
+ * d_keys (batch, key_capacity) uint64, d_counts (batch, 4) int32 as in ysb_filter_candidates; key_capacity >= the summed
+ * key slots of the passes (N_i each, N_i*C with multi_label), else YSB_ERR_WORKSPACE.  ysb_filter_candidates_tta runs
+ * the filter kernel of every pass, all appending to one key list per image; it zero-fills d_counts before the first
+ * pass.  ysb_select_nms_tta: outputs as ysb_postprocess_tta.  ysb_select_nms_tta_gather: the same, its rows and counts
+ * stored into every rank's slot like ysb_select_nms_gather (g->batch and g->max_det must match the passes; d_det_idx
+ * stays local, may be NULL).  Every refusal returns before any CUDA call. */
+int ysb_filter_candidates_tta(const ysb_params *passes, int num_passes, const void *const *d_heads,
+                              const int32_t *heads_per_pass, uint64_t *d_keys, int64_t key_capacity, int32_t *d_counts,
+                              void *stream);
+int ysb_select_nms_tta(const ysb_params *passes, int num_passes, const void *const *d_heads, const int32_t *heads_per_pass,
+                       const uint64_t *d_keys, int64_t key_capacity, const int32_t *d_counts, float *d_dets,
+                       int32_t *d_det_idx, int32_t *d_det_cnt, void *stream);
 
 /* Greedy NMS over one explicit box/score array (utils.numba_nms / utils.gpu_nms).
  *   d_boxes (m,4) float32, d_scores (m) float32 >= 0 (zero scores are never kept, utils/nms.py:16)
@@ -318,7 +331,8 @@ int ysb_undo_letterbox(float *d_dets, const int32_t *d_det_cnt, int batch, int m
  *   per step and slot, all on the caller's stream:
  *     ysb_gather_begin       zero the filter counters, tell every peer "I have consumed the previous use of this slot"
  *                            (a remote store per peer, no waiting)
- *     ysb_filter_candidates, ysb_select_nms_gather  (each image's CTA waits for the peers' acks of this slot -- sent a
+ *     ysb_filter_candidates, ysb_select_nms_gather  (or, for test-time augmentation, ysb_filter_candidates_tta and
+ *                            ysb_select_nms_tta_gather)  (each image's CTA waits for the peers' acks of this slot -- sent a
  *                            whole filter + NMS pass earlier -- then rows + counts -> every peer's slot, then arrival counts)
  *     ysb_gather_wait        wait until the rows of every rank have landed in MY slot
  *   Every rank must run the same sequence of (slot) steps.  Spins are bounded (~20 s); a timeout sets `err`, which
@@ -343,6 +357,10 @@ int ysb_gather_begin(const ysb_gather *g, int slot, int32_t *d_counts, int64_t n
 int ysb_select_nms_gather(const ysb_params *p, const void *const *d_heads, int num_heads, const uint64_t *d_keys,
                           int64_t key_capacity, const int32_t *d_counts, const ysb_gather *g, int slot,
                           int32_t *d_det_idx, void *stream);
+/* ysb_select_nms_tta whose rows/counts go to every rank's slot (declared here because it needs ysb_gather). */
+int ysb_select_nms_tta_gather(const ysb_params *passes, int num_passes, const void *const *d_heads,
+                              const int32_t *heads_per_pass, const uint64_t *d_keys, int64_t key_capacity,
+                              const int32_t *d_counts, const ysb_gather *g, int slot, int32_t *d_det_idx, void *stream);
 int ysb_gather_wait(const ysb_gather *g, int slot, void *stream);
 int ysb_gather_error(const ysb_gather *g, uint32_t *err_out);
 

@@ -119,6 +119,16 @@ _SIGNATURES = {
     "ysb_postprocess_tta": (ctypes.c_int, [ctypes.POINTER(YsbParams), ctypes.c_int, ctypes.POINTER(ctypes.c_void_p),
                                            ctypes.POINTER(ctypes.c_int32), ctypes.c_void_p, ctypes.c_size_t,
                                            ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
+    "ysb_filter_candidates_tta": (ctypes.c_int, [ctypes.POINTER(YsbParams), ctypes.c_int, ctypes.POINTER(ctypes.c_void_p),
+                                                 ctypes.POINTER(ctypes.c_int32), ctypes.c_void_p, ctypes.c_int64,
+                                                 ctypes.c_void_p, ctypes.c_void_p]),
+    "ysb_select_nms_tta": (ctypes.c_int, [ctypes.POINTER(YsbParams), ctypes.c_int, ctypes.POINTER(ctypes.c_void_p),
+                                          ctypes.POINTER(ctypes.c_int32), ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p,
+                                          ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
+    "ysb_select_nms_tta_gather": (ctypes.c_int, [ctypes.POINTER(YsbParams), ctypes.c_int, ctypes.POINTER(ctypes.c_void_p),
+                                                 ctypes.POINTER(ctypes.c_int32), ctypes.c_void_p, ctypes.c_int64,
+                                                 ctypes.c_void_p, ctypes.POINTER(YsbGather), ctypes.c_int, ctypes.c_void_p,
+                                                 ctypes.c_void_p]),
     "ysb_soft_nms": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_float, ctypes.c_int, ctypes.c_int,
                                     ctypes.c_float, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p, ctypes.c_void_p]),
     "ysb_undo_letterbox": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_void_p,

@@ -21,7 +21,7 @@ cudaError_t launch_gather_begin(const ysb_gather *g, int slot, int32_t *d_counts
 cudaError_t launch_gather_wait(const ysb_gather *g, int slot, cudaStream_t stream);
 cudaError_t launch_select_nms_tta(const Plan &P, const ExtraPasses &X, const uint64_t *d_keys, int64_t key_cap,
                                   const int32_t *d_counts, float *d_dets, int32_t *d_det_idx, int32_t *d_det_cnt,
-                                  cudaStream_t stream, int dtype);
+                                  cudaStream_t stream, const GatherSink *sink, int dtype);
 cudaError_t launch_decode(const Plan &P, float *d_out, int64_t rows_total, int64_t row_offset, cudaStream_t stream,
                           int dtype);
 cudaError_t launch_array_nms(const float *d_boxes, const float *d_scores, int64_t m, double iou_thr, int cmp, int iou_kind,
@@ -563,26 +563,9 @@ int ysb_postprocess_tta_workspace_bytes(const ysb_params *passes, int num_passes
     return YSB_OK;
 }
 
-int ysb_postprocess_tta(const ysb_params *passes, int num_passes, const void *const *d_heads, const int32_t *heads_per_pass,
-                        void *d_workspace, size_t workspace_bytes, float *d_dets, int32_t *d_det_idx,
-                        int32_t *d_det_cnt, void *stream)
+// Passes 1..n-1 as the selection/NMS kernel takes them (pass 0 is its own Plan).
+static ExtraPasses extra_passes(const BuiltPasses &bp, int num_passes)
 {
-    if (!d_heads || !heads_per_pass || !d_workspace || !d_dets || !d_det_cnt) return YSB_ERR_BAD_ARG;
-    BuiltPasses bp;
-    int st = build_passes(passes, num_passes, d_heads, heads_per_pass, &bp);
-    if (st != YSB_OK) return st;
-    const size_t batch = static_cast<size_t>(bp.b[0].plan.batch);
-    const size_t need = align256(sizeof(uint64_t) * static_cast<size_t>(bp.slots) * batch) + align256(sizeof(int32_t) * 4 * batch) + 256;
-    if (workspace_bytes < need) return YSB_ERR_WORKSPACE;
-    uintptr_t base = (reinterpret_cast<uintptr_t>(d_workspace) + 255) & ~static_cast<uintptr_t>(255);
-    uint64_t *d_keys = reinterpret_cast<uint64_t *>(base);
-    int32_t *d_counts = reinterpret_cast<int32_t *>(base + align256(sizeof(uint64_t) * static_cast<size_t>(bp.slots) * batch));
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
-    // every pass appends its survivors to the same per-image key list (the counters are zeroed by the first pass only)
-    for (int i = 0; i < num_passes; ++i) {
-        st = cuda_status(launch_filter(bp.b[i].plan, bp.b[i].vec, d_keys, bp.slots, d_counts, s, i == 0, bp.b[i].dtype));
-        if (st != YSB_OK) return st;
-    }
     ExtraPasses X;
     std::memset(&X, 0, sizeof(X));
     X.n = num_passes - 1;
@@ -590,8 +573,77 @@ int ysb_postprocess_tta(const ysb_params *passes, int num_passes, const void *co
         X.base[i - 1] = static_cast<int>(bp.base[i]);
         X.p[i - 1] = bp.b[i].plan;
     }
-    return cuda_status(launch_select_nms_tta(bp.b[0].plan, X, d_keys, bp.slots, d_counts, d_dets, d_det_idx, d_det_cnt, s,
-                                             bp.b[0].dtype));
+    return X;
+}
+
+int ysb_filter_candidates_tta(const ysb_params *passes, int num_passes, const void *const *d_heads,
+                              const int32_t *heads_per_pass, uint64_t *d_keys, int64_t key_capacity, int32_t *d_counts,
+                              void *stream)
+{
+    if (!d_heads || !heads_per_pass || !d_keys || !d_counts) return YSB_ERR_BAD_ARG;
+    BuiltPasses bp;
+    const int st = build_passes(passes, num_passes, d_heads, heads_per_pass, &bp);
+    if (st != YSB_OK) return st;
+    if (key_capacity < bp.slots) return YSB_ERR_WORKSPACE;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    // every pass appends its survivors to the same per-image key list (the counters are zeroed by the first pass only)
+    for (int i = 0; i < num_passes; ++i) {
+        const int e = cuda_status(launch_filter(bp.b[i].plan, bp.b[i].vec, d_keys, key_capacity, d_counts, s, i == 0,
+                                                bp.b[i].dtype));
+        if (e != YSB_OK) return e;
+    }
+    return YSB_OK;
+}
+
+int ysb_select_nms_tta(const ysb_params *passes, int num_passes, const void *const *d_heads, const int32_t *heads_per_pass,
+                       const uint64_t *d_keys, int64_t key_capacity, const int32_t *d_counts, float *d_dets,
+                       int32_t *d_det_idx, int32_t *d_det_cnt, void *stream)
+{
+    if (!d_heads || !heads_per_pass || !d_keys || !d_counts || !d_dets || !d_det_cnt) return YSB_ERR_BAD_ARG;
+    BuiltPasses bp;
+    const int st = build_passes(passes, num_passes, d_heads, heads_per_pass, &bp);
+    if (st != YSB_OK) return st;
+    if (key_capacity < bp.slots) return YSB_ERR_WORKSPACE;
+    const ExtraPasses X = extra_passes(bp, num_passes);
+    return cuda_status(launch_select_nms_tta(bp.b[0].plan, X, d_keys, key_capacity, d_counts, d_dets, d_det_idx, d_det_cnt,
+                                             static_cast<cudaStream_t>(stream), nullptr, bp.b[0].dtype));
+}
+
+int ysb_select_nms_tta_gather(const ysb_params *passes, int num_passes, const void *const *d_heads,
+                              const int32_t *heads_per_pass, const uint64_t *d_keys, int64_t key_capacity,
+                              const int32_t *d_counts, const ysb_gather *g, int slot, int32_t *d_det_idx, void *stream)
+{
+    if (!d_heads || !heads_per_pass || !d_keys || !d_counts) return YSB_ERR_BAD_ARG;
+    BuiltPasses bp;
+    const int st = build_passes(passes, num_passes, d_heads, heads_per_pass, &bp);
+    if (st != YSB_OK) return st;
+    if (key_capacity < bp.slots) return YSB_ERR_WORKSPACE;
+    GatherSink sink;
+    if (!make_gather_sink(g, slot, &sink)) return YSB_ERR_BAD_ARG;
+    if (g->batch != bp.b[0].plan.batch || g->max_det != bp.b[0].plan.max_det) return YSB_ERR_BAD_ARG;
+    const ExtraPasses X = extra_passes(bp, num_passes);
+    return cuda_status(launch_select_nms_tta(bp.b[0].plan, X, d_keys, key_capacity, d_counts, nullptr, d_det_idx, nullptr,
+                                             static_cast<cudaStream_t>(stream), &sink, bp.b[0].dtype));
+}
+
+int ysb_postprocess_tta(const ysb_params *passes, int num_passes, const void *const *d_heads, const int32_t *heads_per_pass,
+                        void *d_workspace, size_t workspace_bytes, float *d_dets, int32_t *d_det_idx,
+                        int32_t *d_det_cnt, void *stream)
+{
+    if (!d_heads || !heads_per_pass || !d_workspace || !d_dets || !d_det_cnt) return YSB_ERR_BAD_ARG;
+    BuiltPasses bp;
+    const int st = build_passes(passes, num_passes, d_heads, heads_per_pass, &bp);
+    if (st != YSB_OK) return st;
+    const size_t batch = static_cast<size_t>(bp.b[0].plan.batch);
+    const size_t need = align256(sizeof(uint64_t) * static_cast<size_t>(bp.slots) * batch) + align256(sizeof(int32_t) * 4 * batch) + 256;
+    if (workspace_bytes < need) return YSB_ERR_WORKSPACE;
+    uintptr_t base = (reinterpret_cast<uintptr_t>(d_workspace) + 255) & ~static_cast<uintptr_t>(255);
+    uint64_t *d_keys = reinterpret_cast<uint64_t *>(base);
+    int32_t *d_counts = reinterpret_cast<int32_t *>(base + align256(sizeof(uint64_t) * static_cast<size_t>(bp.slots) * batch));
+    const int e = ysb_filter_candidates_tta(passes, num_passes, d_heads, heads_per_pass, d_keys, bp.slots, d_counts, stream);
+    if (e != YSB_OK) return e;
+    return ysb_select_nms_tta(passes, num_passes, d_heads, heads_per_pass, d_keys, bp.slots, d_counts, d_dets, d_det_idx,
+                              d_det_cnt, stream);
 }
 
 int ysb_nms_workspace_bytes(int64_t m, size_t *bytes_out)

@@ -1165,12 +1165,13 @@ cudaError_t launch_select_nms(const Plan &P, const uint64_t *d_keys, int64_t key
     return launch_any_dt(P, NoExtraPasses{}, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink, dtype);
 }
 
-// test-time augmentation: one selection/NMS over the key lists the passes appended to; X describes passes 1..n
+// test-time augmentation: one selection/NMS over the key lists the passes appended to; X describes passes 1..n.  sink:
+// as launch_select_nms (nullptr = the caller's dets / det_cnt; a detection gather = every rank's slot)
 cudaError_t launch_select_nms_tta(const Plan &P, const ExtraPasses &X, const uint64_t *d_keys, int64_t key_cap,
                                   const int32_t *d_counts, float *d_dets, int32_t *d_det_idx, int32_t *d_det_cnt,
-                                  cudaStream_t stream, int dtype)
+                                  cudaStream_t stream, const GatherSink *sink, int dtype)
 {
-    return launch_any_dt(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, nullptr, dtype);
+    return launch_any_dt(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink, dtype);
 }
 
 // ---- array flavour: utils.numba_nms / utils.gpu_nms over one explicit (m,4)/(m) pair ---------------------------

@@ -212,6 +212,18 @@ class ShardedPostProcessor:
     16) the per-lane launch sequence is captured once per set of head tensors and replayed.
     A ticket's buffers are reused ``lanes`` submissions later.  The heads may be float32, float16 or bfloat16; the first
     submission fixes the type, and a later batch of another type raises ValueError.
+
+    Test-time augmentation (hyp['use_tta'], trainer/eval_yolov5.py:152-179) goes through ``submit_tta`` with the passes
+    of ``PostProcessor.run_tta``; ``img_h, img_w`` are then the un-augmented input size the boxes are mapped back to:
+
+        passes = [(heads0, 640, 640, 1, None), (heads1, 640, 640, 0.83, 2), (heads2, 640, 640, 0.67, 3)]
+        t = spp.submit_tta(passes)             # every pass's filter -> one merged NMS (+ peer stores) -> arrival wait
+        rows, cnt = spp.gathered(t)            # as above; rows in un-augmented network-input pixels
+
+    Lanes, graphs and the gather work as for ``submit``.  The first submission fixes the kind (plain or TTA): a processor
+    takes only ``submit`` or only ``submit_tta`` calls.  For TTA it also fixes the number of passes, each pass's
+    (img_h, img_w, scale, flip_axis) and the head shapes, and sizes the key buffers to the passes' summed key slots; a
+    later submission that differs raises ValueError.
     """
 
     def __init__(self, family, hyp, batch, img_h, img_w, anchors=None, lanes=None, group=None, gather="auto", graph=None,
@@ -247,6 +259,8 @@ class ShardedPostProcessor:
                 self.mode = "nccl"
         self.streams = [torch.cuda.Stream(device=self.device) for _ in range(self.lanes)]
         self._ent = None
+        self._kind = None      # "plain" (submit) or "tta" (submit_tta), fixed by the first submission
+        self._tta = None       # TTA set-up: pass geometry, cache entries, ctypes params / heads-per-pass arrays
         self._slots = None
         self._graphs = {}
         self._warmed = False
@@ -258,7 +272,24 @@ class ShardedPostProcessor:
             return
         self._ent = self.pp._prepare(flat, self.batch, self.img_h, self.img_w, _lib.INPUT_RAW_HEADS)
         self._head_dtype = flat[0].dtype
-        n = self._ent["N"] * (int(self.pp.hyp["num_class"]) if self.pp.hyp["mutil_label"] else 1)
+        self._alloc_lanes(self._ent["N"] * self._slots_per_candidate())
+
+    def _slots_per_candidate(self):
+        return int(self.pp.hyp["num_class"]) if self.pp.hyp["mutil_label"] else 1
+
+    def _prepare_tta(self, ents, geom):
+        """TTA set-up of the first submit_tta: params of every pass, key buffers sized to the summed key slots."""
+        n = len(ents)
+        params = (_lib.YsbParams * n)(*[e["params"] for _, e in ents])
+        for i in range(n):
+            params[i].d_letterbox = None   # rows stay in network-input pixels, as with submit
+        self._tta = dict(geom=geom, ents=[e for _, e in ents], params=params,
+                         per_pass=(ctypes.c_int32 * n)(*[len(flat) for flat, _ in ents]))
+        self._head_dtype = ents[0][0][0].dtype
+        self._alloc_lanes(sum(e["N"] for _, e in ents) * self._slots_per_candidate())
+
+    def _alloc_lanes(self, n):
+        """Key / count / output buffers of every lane; ``n`` key slots per image."""
         self._key_cap = n
         b, d, dev = self.batch, self.max_det, self.device
         self._slots = []
@@ -289,8 +320,17 @@ class ShardedPostProcessor:
 
     def _enqueue(self, ptrs, nheads, lane, st, events=None):
         """The launch sequence of one batch on stream ``st`` (plain C-ABI calls: capturable into a CUDA graph)."""
-        lib, sl, params = self.lib, self._slots[lane], self._ent["params"]
+        lib, sl = self.lib, self._slots[lane]
         sp = ctypes.c_void_p(st.cuda_stream)
+        # the plain and the TTA entry points take the same arguments after the heads
+        if self._kind == "tta":
+            tta, sfx = self._tta, "_tta"
+            head = (tta["params"], len(tta["params"]), ptrs, tta["per_pass"])
+        else:
+            sfx = ""
+            head = (ctypes.byref(self._ent["params"]), ptrs, nheads)
+        filt, nms = getattr(lib, "ysb_filter_candidates" + sfx), getattr(lib, "ysb_select_nms" + sfx)
+        nms_gather = getattr(lib, "ysb_select_nms" + sfx + "_gather")
         if self.mode == "p2p":
             # first thing of the step: tell the peers this slot's previous contents have been consumed (they check it
             # right before storing into it, a filter + NMS pass from now)
@@ -298,14 +338,13 @@ class ShardedPostProcessor:
             _lib.check(lib.ysb_gather_begin(g, lane, None, 0, sp), "ysb_gather_begin")
         if events:
             events[0].record(st)
-        _lib.check(lib.ysb_filter_candidates(ctypes.byref(params), ptrs, nheads, sl["keys"].data_ptr(), self._key_cap,
-                                             sl["counts"].data_ptr(), sp), "ysb_filter_candidates")
+        _lib.check(filt(*head, sl["keys"].data_ptr(), self._key_cap, sl["counts"].data_ptr(), sp),
+                   "ysb_filter_candidates" + sfx)
         if events:
             events[1].record(st)
         if self.mode == "p2p":
-            _lib.check(lib.ysb_select_nms_gather(ctypes.byref(params), ptrs, nheads, sl["keys"].data_ptr(), self._key_cap,
-                                                 sl["counts"].data_ptr(), g, lane, sl["idx"].data_ptr(), sp),
-                       "ysb_select_nms_gather")
+            _lib.check(nms_gather(*head, sl["keys"].data_ptr(), self._key_cap, sl["counts"].data_ptr(), g, lane,
+                                  sl["idx"].data_ptr(), sp), "ysb_select_nms" + sfx + "_gather")
             if events:
                 events[2].record(st)
             _lib.check(lib.ysb_gather_wait(g, lane, sp), "ysb_gather_wait")
@@ -314,9 +353,8 @@ class ShardedPostProcessor:
                 rows_ptr, cnt_ptr = sl["send"].data_ptr(), sl["send"].data_ptr() + self.batch * self.max_det * 24
             else:
                 rows_ptr, cnt_ptr = sl["rows"].data_ptr(), sl["cnt"].data_ptr()
-            _lib.check(lib.ysb_select_nms(ctypes.byref(params), ptrs, nheads, sl["keys"].data_ptr(), self._key_cap,
-                                          sl["counts"].data_ptr(), rows_ptr, sl["idx"].data_ptr(), cnt_ptr, sp),
-                       "ysb_select_nms")
+            _lib.check(nms(*head, sl["keys"].data_ptr(), self._key_cap, sl["counts"].data_ptr(), rows_ptr,
+                           sl["idx"].data_ptr(), cnt_ptr, sp), "ysb_select_nms" + sfx)
             if events:
                 events[2].record(st)
 
@@ -325,12 +363,53 @@ class ShardedPostProcessor:
         """Enqueue one batch.  ``events``: optional 3 timing events (start, filter done, NMS done) recorded on the lane's
         stream.  ``sync_input=False`` skips the wait on the caller's current stream (heads known to be ready)."""
         from .engine import flatten_heads
+        if self._kind == "tta":
+            raise ValueError("this processor was set up for test-time-augmented batches: use submit_tta")
         flat = flatten_heads(self.family, heads)
         if flat[0].shape[0] != self.batch:
             raise ValueError(f"expected {self.batch} images per rank, got {flat[0].shape[0]}")
         self._prepare(flat)
+        self._kind = "plain"
         if any(t.dtype != self._head_dtype for t in flat):
             raise ValueError(f"this processor was set up for {self._head_dtype} heads, got {sorted({str(t.dtype) for t in flat})}")
+        return self._submit(flat, events, sync_input)
+
+    def submit_tta(self, passes, events=None, sync_input=True):
+        """Enqueue one test-time-augmented batch: ``passes`` = [(heads, img_h, img_w, scale, flip_axis), ...] as for
+        PostProcessor.run_tta, undone against the constructor's (img_h, img_w).  The passes' filter kernels append to one
+        key list per image and one NMS kernel selects over all of them; rows are in un-augmented network-input pixels and
+        the local det_idx counts through the passes in order.  ``events`` / ``sync_input`` as for ``submit``."""
+        from .engine import flatten_heads
+        if self._kind == "plain":
+            raise ValueError("this processor was set up for plain batches: use submit")
+        passes = list(passes)
+        if not 1 <= len(passes) <= _lib.YSB_MAX_PASSES:
+            raise ValueError(f"1..{_lib.YSB_MAX_PASSES} passes, got {len(passes)}")
+        flats = [flatten_heads(self.family, p[0]) for p in passes]
+        for k, flat in enumerate(flats):
+            if flat[0].shape[0] != self.batch:
+                raise ValueError(f"expected {self.batch} images per rank, got {flat[0].shape[0]} in pass {k}")
+        geom = tuple((int(h), int(w), float(s), int(f or 0)) for _, h, w, s, f in passes)
+        dtypes = {t.dtype for flat in flats for t in flat}
+        if len(dtypes) != 1:
+            raise ValueError(f"every pass must have heads of one dtype, got {sorted(map(str, dtypes))}")
+        if self._tta is not None:
+            if geom != self._tta["geom"]:
+                raise ValueError(f"this processor was set up for the passes (img_h, img_w, scale, flip) "
+                                 f"{list(self._tta['geom'])}, got {list(geom)}")
+            if dtypes != {self._head_dtype}:
+                raise ValueError(f"this processor was set up for {self._head_dtype} heads, got {sorted(map(str, dtypes))}")
+        ents = self.pp._tta_entries(passes, (self.img_h, self.img_w))
+        if self._tta is None:
+            self._prepare_tta(ents, geom)
+            self._kind = "tta"
+        elif any(e is not k for (_, e), k in zip(ents, self._tta["ents"])):
+            raise ValueError("the head shapes differ from those of the first submit_tta")
+        return self._submit([t for flat in flats for t in flat], events, sync_input)
+
+    def _submit(self, flat, events, sync_input):
+        """Lane choice, plain launches / graph capture / replay and the NCCL all-gather of one batch whose heads (all
+        passes' for TTA) are ``flat``."""
         lane = self._next % self.lanes
         self._next += 1
         st = self.streams[lane]
@@ -369,7 +448,7 @@ class ShardedPostProcessor:
         g = torch.cuda.CUDAGraph()
         with torch.cuda.graph(g, stream=st, capture_error_mode="thread_local"):
             self._enqueue(ptrs, len(flat), lane, st)
-        g._ysb_keep = (ptrs, flat)
+        g._ysb_keep = (ptrs, flat, self._tta)   # pointer arrays, heads and (TTA) the params / heads-per-pass arrays
         return g
 
     def gathered(self, ticket):
@@ -413,4 +492,4 @@ class ShardedPostProcessor:
         if self.dg is not None:
             self.dg.close()
             self.dg = None
-        self._slots, self._ent = None, None
+        self._slots, self._ent, self._tta = None, None, None
