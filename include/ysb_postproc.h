@@ -82,9 +82,19 @@ typedef enum ysb_dtype {
     YSB_BF16 = 2   /* bfloat16 (torch.bfloat16) */
 } ysb_dtype;
 
+/* What d_heads point to.  RAW_HEADS_NHWC (added in ABI version 6 without a layout change of ysb_params; an older library
+ * refuses it with YSB_ERR_BAD_ARG) is raw heads in channels-last memory, as a model run with
+ * torch.channels_last emits them.  The logical shapes are those of enum ysb_family, the memory is:
+ *   YOLOv5 level (b, H, W, A*(5+C));  YOLOX level (b, H, W, A, 5+C) (the (b, A, 5+C, H, W) view of a channels-last conv);
+ *   YOLOv8 level (b, H, W, 4*bins + C);  FCOS cls (b, H, W, C), reg (b, H, W, 4), ctr (b, H, W, 1).
+ * Results (rows, det_idx, counts, decoded rows) are bit-identical to RAW_HEADS on the same values.  YOLOv7 and RetinaNet
+ * heads already are rows: kind 2 returns YSB_ERR_BAD_ARG for them.  A candidate's channels form one row that the filter
+ * kernel stages in shared memory: rows wider than that tile allows (5+C, 4*bins+C or C above ~450) return YSB_ERR_LIMIT.
+ * Every entry point that takes raw heads accepts it, with every head_dtype; the passes of one TTA call share one kind. */
 typedef enum ysb_input_kind {
-    YSB_INPUT_RAW_HEADS = 0,   /* raw model outputs; decode is fused into the filter/NMS kernels */
-    YSB_INPUT_DECODED_ROWS = 1 /* the (b, N, C') tensor do_inference returns; heads[0] points at it */
+    YSB_INPUT_RAW_HEADS = 0,      /* raw model outputs (contiguous NCHW); decode is fused into the filter/NMS kernels */
+    YSB_INPUT_DECODED_ROWS = 1,   /* the (b, N, C') tensor do_inference returns; heads[0] points at it */
+    YSB_INPUT_RAW_HEADS_NHWC = 2  /* raw model outputs in channels-last memory (above) */
 } ysb_input_kind;
 
 /* IoU flavours.  NUMBA_F64MIX is the live path (utils/bbox_tools.py:12-35: float32 sides/areas,

@@ -20,6 +20,7 @@ YOLOV5, YOLOV7, YOLOX, YOLOV8, RETINANET, RETINANET_EXP, FCOS = range(7)
 FAMILY_IDS = {"yolov5": YOLOV5, "yolov7": YOLOV7, "yolox": YOLOX, "yolov8": YOLOV8, "retinanet": RETINANET,
               "retinanet_exp": RETINANET_EXP, "fcos": FCOS}
 INPUT_RAW_HEADS, INPUT_DECODED_ROWS = 0, 1
+INPUT_RAW_HEADS_NHWC = 2   # raw heads in channels-last memory (YOLOv5, YOLOX, YOLOv8, FCOS)
 # enum ysb_dtype (element type of the raw heads)
 DTYPE_F32, DTYPE_F16, DTYPE_BF16 = 0, 1, 2
 IOU_NUMBA_F64MIX, IOU_F32, GIOU, DIOU, CIOU = range(5)

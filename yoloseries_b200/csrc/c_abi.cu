@@ -93,7 +93,13 @@ static int build_plan(const ysb_params *p, const void *const *d_heads, int num_h
 {
     if (!p || !out) return YSB_ERR_BAD_ARG;
     if (p->family < YSB_YOLOV5 || p->family > YSB_FCOS) return YSB_ERR_BAD_ARG;
-    if (p->input_kind != YSB_INPUT_RAW_HEADS && p->input_kind != YSB_INPUT_DECODED_ROWS) return YSB_ERR_BAD_ARG;
+    if (p->input_kind != YSB_INPUT_RAW_HEADS && p->input_kind != YSB_INPUT_DECODED_ROWS &&
+        p->input_kind != YSB_INPUT_RAW_HEADS_NHWC)
+        return YSB_ERR_BAD_ARG;
+    // channels-last memory is a layout of the planes families only (YOLOv7 / RetinaNet heads already are rows)
+    const bool nhwc = p->input_kind == YSB_INPUT_RAW_HEADS_NHWC;
+    if (nhwc && p->family != YSB_YOLOV5 && p->family != YSB_YOLOX && p->family != YSB_YOLOV8 && p->family != YSB_FCOS)
+        return YSB_ERR_BAD_ARG;
     if (p->head_dtype != YSB_F32 && p->head_dtype != YSB_F16 && p->head_dtype != YSB_BF16) return YSB_ERR_BAD_ARG;
     if (p->head_dtype != YSB_F32 && p->input_kind == YSB_INPUT_DECODED_ROWS) return YSB_ERR_BAD_ARG;  // decoded rows: float32
     if (p->batch < 0 || p->num_classes <= 0 || p->num_levels <= 0 || p->num_levels > YSB_MAX_LEVELS) return YSB_ERR_BAD_ARG;
@@ -108,7 +114,7 @@ static int build_plan(const ysb_params *p, const void *const *d_heads, int num_h
     Plan &P = out->plan;
     std::memset(&P, 0, sizeof(P));
     P.family = p->family;
-    P.input_kind = p->input_kind;
+    P.input_kind = nhwc ? YSB_INPUT_RAW_HEADS : p->input_kind;   // NHWC heads take every raw-head branch (layout below)
     P.batch = p->batch;
     P.C = C;
     P.A = A;
@@ -135,7 +141,7 @@ static int build_plan(const ysb_params *p, const void *const *d_heads, int num_h
     if (p->tta_flip != 0 && p->tta_flip != 2 && p->tta_flip != 3) return YSB_ERR_BAD_ARG;
     if (p->tta_scale < 0.0f || p->tta_scale != p->tta_scale) return YSB_ERR_BAD_ARG;
     P.tta_on = (p->tta_scale != 0.0f && p->tta_scale != 1.0f) || p->tta_flip != 0;
-    if (P.tta_on && p->input_kind != YSB_INPUT_RAW_HEADS) return YSB_ERR_BAD_ARG;
+    if (P.tta_on && P.input_kind != YSB_INPUT_RAW_HEADS) return YSB_ERR_BAD_ARG;
     P.tta_div = p->tta_scale == 0.0f ? 1.0f : p->tta_scale;
     P.tta_flip = p->tta_flip;
     P.tta_h = static_cast<float>(p->tta_img_h);
@@ -205,6 +211,14 @@ static int build_plan(const ysb_params *p, const void *const *d_heads, int num_h
         break;
     default: return YSB_ERR_BAD_ARG;
     }
+    if (nhwc) {
+        // channels-last planes-family heads: a level is one (H*W*A, K) row matrix per image, K = the channels of one
+        // anchor; the filter kernel scans it like YOLOv7's rows (cls_nch / obj_nch stay: head_elem addresses the rest)
+        P.layout = LAYOUT_ROWS_NHWC;
+        P.row_w_in = P.cls_nch;
+        P.cls_col_in = P.cls_ch;
+        P.obj_col_in = (p->family == YSB_YOLOV5 || p->family == YSB_YOLOX) ? P.obj_ch : -1;   // FCOS: ctr tensor (obj_src 2)
+    }
     if (p->input_kind == YSB_INPUT_DECODED_ROWS) {
         // the (b, N, C') tensor: one rows segment, objectness (if any) inside the row
         P.layout = LAYOUT_ROWS;
@@ -215,7 +229,7 @@ static int build_plan(const ysb_params *p, const void *const *d_heads, int num_h
 
     // rows layout: the filter kernel stages a tile of 128 rows in shared memory (filter_kernels.cu, k_filter_rows);
     // rows wider than ~450 floats would not fit the 227 KB a CTA can opt into
-    if (P.layout == LAYOUT_ROWS && static_cast<size_t>(128) * (P.row_w_in | 1) * sizeof(float) > 227u * 1024u) return YSB_ERR_LIMIT;
+    if (P.layout != LAYOUT_PLANES && static_cast<size_t>(128) * (P.row_w_in | 1) * sizeof(float) > 227u * 1024u) return YSB_ERR_LIMIT;
 
     out->heads_expected = expected_heads(p);
     out->dtype = p->head_dtype;
@@ -248,7 +262,7 @@ static int build_plan(const ysb_params *p, const void *const *d_heads, int num_h
         for (int l = 0; l < L; ++l) {
             const int rows_l = A * P.lv[l].hw;
             P.lv[l].unit_off = tiles;
-            P.lv[l].img_rows = (p->family == YSB_YOLOV7) ? rows_l : P.N;
+            P.lv[l].img_rows = (p->family == YSB_YOLOV7 || nhwc) ? rows_l : P.N;
             tiles += (rows_l + 127) / 128;
         }
         P.units_per_img = tiles;
@@ -322,7 +336,7 @@ int ysb_num_candidates(const ysb_params *p, int64_t *n_out, int32_t *row_width_o
 int ysb_decode(const ysb_params *p, const void *const *d_heads, int num_heads, float *d_decoded, void *stream)
 {
     if (!d_heads || !d_decoded) return YSB_ERR_BAD_ARG;
-    if (p && p->input_kind != YSB_INPUT_RAW_HEADS) return YSB_ERR_BAD_ARG;
+    if (p && p->input_kind != YSB_INPUT_RAW_HEADS && p->input_kind != YSB_INPUT_RAW_HEADS_NHWC) return YSB_ERR_BAD_ARG;
     Built b;
     const int st = build_plan(p, d_heads, num_heads, &b);
     if (st != YSB_OK) return st;
@@ -333,7 +347,7 @@ int ysb_decode_into(const ysb_params *p, const void *const *d_heads, int num_hea
                     int64_t row_offset, void *stream)
 {
     if (!d_heads || !d_decoded) return YSB_ERR_BAD_ARG;
-    if (p && p->input_kind != YSB_INPUT_RAW_HEADS) return YSB_ERR_BAD_ARG;
+    if (p && p->input_kind != YSB_INPUT_RAW_HEADS && p->input_kind != YSB_INPUT_RAW_HEADS_NHWC) return YSB_ERR_BAD_ARG;
     Built b;
     const int st = build_plan(p, d_heads, num_heads, &b);
     if (st != YSB_OK) return st;
@@ -527,15 +541,15 @@ static int build_passes(const ysb_params *passes, int num_passes, const void *co
     int head0 = 0;
     for (int i = 0; i < num_passes; ++i) {
         const ysb_params *p = passes + i;
-        if (p->input_kind != YSB_INPUT_RAW_HEADS) return YSB_ERR_BAD_ARG;
-        // one evaluator, one hyp: everything but the geometry and the undo must agree with pass 0
+        if (p->input_kind != YSB_INPUT_RAW_HEADS && p->input_kind != YSB_INPUT_RAW_HEADS_NHWC) return YSB_ERR_BAD_ARG;
+        // one evaluator, one hyp: everything but the geometry and the undo must agree with pass 0 (one head layout too)
         const ysb_params *q = passes;
         if (p->family != q->family || p->batch != q->batch || p->num_classes != q->num_classes ||
             p->conf_thr != q->conf_thr || p->cls_thr != q->cls_thr || p->pre_nms_thr != q->pre_nms_thr ||
             p->iou_thr != q->iou_thr || p->max_det != q->max_det || p->class_aware != q->class_aware ||
             p->multi_label != q->multi_label || p->postprocess_bbox != q->postprocess_bbox ||
             p->min_box_wh != q->min_box_wh || p->pre_nms_topk != q->pre_nms_topk ||
-            p->thresh_with_ctr != q->thresh_with_ctr || p->head_dtype != q->head_dtype)
+            p->thresh_with_ctr != q->thresh_with_ctr || p->head_dtype != q->head_dtype || p->input_kind != q->input_kind)
             return YSB_ERR_BAD_ARG;
         const int nh = d_heads ? heads_per_pass[i] : 0;
         const int st = build_plan(p, d_heads ? d_heads + head0 : nullptr, nh, &out->b[i]);

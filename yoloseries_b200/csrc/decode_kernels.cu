@@ -31,7 +31,7 @@ struct CandAddr {
     const T *obj;  // objectness / centerness / conf logit, nullptr when the family has none
 };
 
-template <typename T>
+template <typename T, bool NHWC>
 __device__ __forceinline__ CandAddr<T> cand_addr(const Plan &P, int img, int cand)
 {
     CandAddr<T> c;
@@ -39,12 +39,13 @@ __device__ __forceinline__ CandAddr<T> cand_addr(const Plan &P, int img, int can
     const LevelDesc &lv = P.lv[l];
     const int r = cand - lv.cand_off;
     c.obj = nullptr;
-    if (P.layout == LAYOUT_PLANES) {
+    bool planes = P.layout == LAYOUT_PLANES;
+    if constexpr (NHWC) planes = true;
+    if (planes) {   // planes-family raw heads, NCHW or NHWC
         const int a = r / lv.hw, pos = r - a * lv.hw;
-        c.cls = head_ptr<T>(lv.p0) + (static_cast<size_t>(img * P.A + a) * P.cls_nch + P.cls_ch) * lv.hw + pos;
-        c.cstride = static_cast<size_t>(lv.hw);
-        if (P.obj_col >= 0)
-            c.obj = head_ptr<T>(P.obj_src == 2 ? lv.p2 : lv.p0) + (static_cast<size_t>(img * P.A + a) * P.obj_nch + P.obj_ch) * lv.hw + pos;
+        c.cls = head_elem<T, NHWC>(lv, lv.p0, P.A, P.cls_nch, img, a, pos, P.cls_ch);
+        c.cstride = static_cast<size_t>(head_step<NHWC>(lv));
+        if (P.obj_col >= 0) c.obj = head_elem<T, NHWC>(lv, P.obj_src == 2 ? lv.p2 : lv.p0, P.A, P.obj_nch, img, a, pos, P.obj_ch);
     } else {
         const T *row = head_ptr<T>(lv.p0) + (static_cast<size_t>(img) * lv.img_rows + r) * P.row_w_in;
         c.cls = row + P.cls_col_in;
@@ -55,9 +56,10 @@ __device__ __forceinline__ CandAddr<T> cand_addr(const Plan &P, int img, int can
     return c;
 }
 
-// ROWS = candidates per CTA: 32 for channels-last heads (their rows are contiguous anyway), 128 for NCHW planes so that
+// ROWS = candidates per CTA: 32 for channels-last heads (their rows are contiguous anyway; NHWC planes-family heads take
+// the rows branch: cand_addr gives class step 1 and decode_box_cols reads their boxes), 128 for NCHW planes so that
 // every plane access of a CTA covers 512 contiguous bytes.
-template <int ROWS, typename T>
+template <int ROWS, typename T, bool NHWC>
 __global__ void __launch_bounds__(kDecThreads) k_decode_rows(const __grid_constant__ Plan P, float *__restrict__ out,
                                                               int64_t rows_total, int64_t row_offset)
 {
@@ -67,12 +69,12 @@ __global__ void __launch_bounds__(kDecThreads) k_decode_rows(const __grid_consta
     const int nrows = min(ROWS, P.N - c0);
     const int rw = P.row_w;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (P.layout == LAYOUT_PLANES) {
+    if (P.layout == LAYOUT_PLANES) {   // (NHWC plans: LAYOUT_ROWS_NHWC, the rows branch)
         // thread = (candidate, class phase): consecutive threads take consecutive positions of one plane
         constexpr int kPhases = kDecThreads / ROWS;  // 2 for ROWS = 128
         const int rr = threadIdx.x % ROWS, ph = threadIdx.x / ROWS;
         if (rr < nrows) {
-            const CandAddr<T> ca = cand_addr<T>(P, img, c0 + rr);
+            const CandAddr<T> ca = cand_addr<T, NHWC>(P, img, c0 + rr);
             float *tc = tile + rr * rw + P.cls_col;
             const size_t step = static_cast<size_t>(kPhases) * ca.cstride;
             // kDecInFlight independent loads per thread before the first sigmoid: the kernel is bound by memory-level
@@ -108,7 +110,7 @@ __global__ void __launch_bounds__(kDecThreads) k_decode_rows(const __grid_consta
             for (int base = 0; base < nrows; base += kDecThreads / 4) {
                 const int r4 = base + (threadIdx.x >> 2), side = threadIdx.x & 3;
                 float sv = 0.0f;
-                if (r4 < nrows) sv = v8_side_value<T>(P, img, c0 + r4, side);
+                if (r4 < nrows) sv = v8_side_value<T, NHWC>(P, img, c0 + r4, side);
                 const unsigned qb = lane & ~3u;
                 const float s0 = __shfl_sync(0xffffffffu, sv, qb), s1 = __shfl_sync(0xffffffffu, sv, qb + 1);
                 const float s2 = __shfl_sync(0xffffffffu, sv, qb + 2), s3 = __shfl_sync(0xffffffffu, sv, qb + 3);
@@ -120,7 +122,7 @@ __global__ void __launch_bounds__(kDecThreads) k_decode_rows(const __grid_consta
             }
         } else if (threadIdx.x >= kDecThreads - ROWS && threadIdx.x - (kDecThreads - ROWS) < nrows) {
             const int rb = threadIdx.x - (kDecThreads - ROWS);
-            const float4 b = tta_undo(P, decode_box_cols<T>(P, img, c0 + rb));
+            const float4 b = tta_undo(P, decode_box_cols<T, NHWC>(P, img, c0 + rb));
             float *t = tile + rb * rw + P.box_col;
             t[0] = b.x; t[1] = b.y; t[2] = b.z; t[3] = b.w;
         }
@@ -129,7 +131,7 @@ __global__ void __launch_bounds__(kDecThreads) k_decode_rows(const __grid_consta
         // fetched sector fully used; kDecInFlightRows loads in flight per thread.  Lane-per-candidate box / objectness decode.
         const int r = threadIdx.x >> 3, q = threadIdx.x & 7;
         if (r < nrows) {
-            const CandAddr<T> ca = cand_addr<T>(P, img, c0 + r);
+            const CandAddr<T> ca = cand_addr<T, NHWC>(P, img, c0 + r);
             float *tc = tile + r * rw + P.cls_col;
             int k = q;
             for (; k + 8 * (kDecInFlightRows - 1) < P.C; k += 8 * kDecInFlightRows) {
@@ -155,11 +157,11 @@ __global__ void __launch_bounds__(kDecThreads) k_decode_rows(const __grid_consta
         }
         if (warp == 0 && lane < nrows) {
             const int cand = c0 + lane;
-            const float4 b = tta_undo(P, decode_box_cols<T>(P, img, cand));
+            const float4 b = tta_undo(P, decode_box_cols<T, NHWC>(P, img, cand));
             float *t = tile + lane * rw + P.box_col;
             t[0] = b.x; t[1] = b.y; t[2] = b.z; t[3] = b.w;
             if (P.obj_col >= 0) {
-                const CandAddr<T> ca = cand_addr<T>(P, img, cand);
+                const CandAddr<T> ca = cand_addr<T, NHWC>(P, img, cand);
                 t[P.obj_col - P.box_col] = sigmoid_ref(ldg_head(ca.obj));
             }
         }
@@ -177,23 +179,24 @@ __global__ void __launch_bounds__(kDecThreads) k_decode_rows(const __grid_consta
     }
 }
 
-template <int ROWS, typename T>
+template <int ROWS, typename T, bool NHWC = false>
 static cudaError_t launch_decode_t(const Plan &P, float *d_out, int64_t rows_total, int64_t row_offset, cudaStream_t stream)
 {
     const size_t smem = static_cast<size_t>(ROWS) * P.row_w * sizeof(float);
     if (smem > 200 * 1024) return cudaErrorInvalidValue;
     if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(k_decode_rows<ROWS, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
+        cudaError_t e = cudaFuncSetAttribute(k_decode_rows<ROWS, T, NHWC>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
         if (e != cudaSuccess) return e;
     }
     const dim3 grid((P.N + ROWS - 1) / ROWS, P.batch);
-    k_decode_rows<ROWS, T><<<grid, kDecThreads, smem, stream>>>(P, d_out, rows_total, row_offset);
+    k_decode_rows<ROWS, T, NHWC><<<grid, kDecThreads, smem, stream>>>(P, d_out, rows_total, row_offset);
     return cudaGetLastError();
 }
 
 template <typename T>
 static cudaError_t launch_decode_dt(const Plan &P, float *d_out, int64_t rows_total, int64_t row_offset, cudaStream_t stream)
 {
+    if (P.layout == LAYOUT_ROWS_NHWC) return launch_decode_t<32, T, true>(P, d_out, rows_total, row_offset, stream);   // rows branch, 32 rows / CTA
     if (P.layout == LAYOUT_PLANES && static_cast<size_t>(128) * P.row_w * sizeof(float) <= 100 * 1024)
         return launch_decode_t<128, T>(P, d_out, rows_total, row_offset, stream);
     return launch_decode_t<32, T>(P, d_out, rows_total, row_offset, stream);

@@ -21,7 +21,8 @@
 // Kernels in this file (dispatch: launch_filter at the bottom):
 //   k_filter_planes_v4     NCHW heads whose levels are all 128-bit loadable (YOLOv5 / YOLOX / YOLOv8)   -- product path
 //   k_filter_planes        NCHW heads with levels that are not (FCOS' 5x5 map); generic                   -- product path
-//   k_filter_rows          channels-last heads and the decoded (b, N, C') tensor (YOLOv7, RetinaNet)      -- product path
+//   k_filter_rows          channels-last heads and the decoded (b, N, C') tensor (YOLOv7, RetinaNet; NHWC  -- product path
+//                          YOLOv5 / YOLOX / YOLOv8 / FCOS heads through its NHWC instantiation)
 //   k_filter_multilabel    hyp['mutil_label']: one key per (candidate, class)                              -- product path
 // The cp.async ring, 1-D bulk-copy TMA ring and 2-D tensor-map TMA ring variants that were measured against these (same
 // survivor sets, slower on this access pattern; profiles/README.md) live in filter_variants.cuh and are compiled only with
@@ -518,7 +519,8 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst_smem, const void *src_gmem
 #endif
 
 // -------------------------------------------------------------------------------------------------------
-// rows layout (channels-last heads: YOLOv7, RetinaNet cls; and the decoded (b, N, C') tensor of any family).
+// rows layout (channels-last heads: YOLOv7, RetinaNet cls, NHWC YOLOv5 / YOLOX / YOLOv8 / FCOS cls; and the decoded
+// (b, N, C') tensor of any family).
 // A CTA stages a tile of 128 whole rows in shared memory with one bulk copy (rows are 340 B / 320 B and only 4-byte
 // aligned individually, but the tile is contiguous and 16-byte aligned), then one thread scans one row: 128-bit shared
 // loads when the class run of every row is 16-byte aligned, else scalar loads; rows with an even stride are walked with
@@ -533,7 +535,9 @@ constexpr int kRowsTile = 128;
 
 // One thread scans one staged row (thread t of the tile -> row r0 + t of level lv), decides it and the warp appends the
 // survivors.  Every thread of the warp must call (rows beyond nrows contribute nothing).
-template <typename T>
+// NHWC: the tile holds rows of channels-last planes-family heads (YOLOv5, YOLOX, YOLOv8, FCOS cls): memory row m of a level
+// is candidate a*hw + p with p = m / A, a = m % A, and FCOS' centerness is read from its own (b, H, W, 1) tensor.
+template <typename T, bool NHWC = false>
 __device__ __forceinline__ void rows_scan_emit(const Plan &P, const LevelDesc &lv, int img, const T *tile, int sstride,
                                                int nrows, int r0, int t, uint64_t *__restrict__ keys, int64_t key_cap,
                                                int32_t *__restrict__ counts, bool vec4 = false, const uint2 *ext_seen = nullptr)
@@ -609,10 +613,17 @@ __device__ __forceinline__ void rows_scan_emit(const Plan &P, const LevelDesc &l
                 }
             }
         }
-        const int cand = lv.cand_off + r0 + t;
+        int cand = lv.cand_off + r0 + t, pos = 0;
+        if (NHWC) {
+            const int m = r0 + t, a = m % P.A;
+            pos = m / P.A;
+            cand = lv.cand_off + a * lv.hw + pos;
+        }
         float objv = 0.0f;
         if (P.use_obj) {
-            if (P.obj_src == 1)  // RetinaNet-exp: conf logit is the last column of the reg tensor
+            if (NHWC && P.obj_src == 2)  // FCOS centerness (A == 1)
+                objv = ldg_head(head_elem<T, true>(lv, lv.p2, 1, P.obj_nch, img, 0, pos, P.obj_ch));
+            else if (P.obj_src == 1)  // RetinaNet-exp: conf logit is the last column of the reg tensor
                 objv = ldg_head(head_ptr<T>(P.lv[0].p1) + (static_cast<size_t>(img) * P.N + cand) * P.reg_row_w + 4);
             else
                 objv = widen(row[P.obj_col_in]);
@@ -636,7 +647,7 @@ __device__ __forceinline__ void rows_scan_emit(const Plan &P, const LevelDesc &l
                  counts + img * 4, P.pre_kind == PRE_ANY_GT, ext_seen);
 }
 
-template <typename T>
+template <typename T, bool NHWC>
 __global__ void __launch_bounds__(kRowsTile) k_filter_rows(const __grid_constant__ Plan P, uint64_t *__restrict__ keys,
                                                            int64_t key_cap, int32_t *__restrict__ counts, int flags)
 {
@@ -691,8 +702,8 @@ __global__ void __launch_bounds__(kRowsTile) k_filter_rows(const __grid_constant
     }
     __syncthreads();
 
-    rows_scan_emit(P, lv, img, tile, sstride, nrows, r0, static_cast<int>(threadIdx.x), keys, key_cap, counts, (flags & 2) != 0,
-                   &ext_seen);
+    rows_scan_emit<T, NHWC>(P, lv, img, tile, sstride, nrows, r0, static_cast<int>(threadIdx.x), keys, key_cap, counts,
+                            (flags & 2) != 0, &ext_seen);
 }
 
 #ifdef YSB_PROFILING_VARIANTS
@@ -802,7 +813,7 @@ __global__ void __launch_bounds__(kRowsTile) k_filter_rows_ring(const __grid_con
 // eval_fcos.py:246-250).  False in every shipped yaml, so this kernel favours simplicity: one thread per candidate,
 // every class evaluated literally (sigmoid, multiply) twice -- once to count, once to write -- any input layout.
 // -------------------------------------------------------------------------------------------------------
-template <typename T>
+template <typename T, bool NHWC>
 __global__ void __launch_bounds__(256) k_filter_multilabel(const __grid_constant__ Plan P, uint64_t *__restrict__ keys,
                                                            int64_t key_cap, int32_t *__restrict__ counts)
 {
@@ -818,12 +829,11 @@ __global__ void __launch_bounds__(256) k_filter_multilabel(const __grid_constant
         const LevelDesc &lv = P.lv[l];
         const int r = cand - lv.cand_off;
         float objv = 0.0f;
-        if (P.layout == LAYOUT_PLANES) {
+        if (NHWC || P.layout == LAYOUT_PLANES) {   // planes-family raw heads, NCHW or NHWC
             const int a = r / lv.hw, pos = r - a * lv.hw;
-            cls = head_ptr<T>(lv.p0) + (static_cast<size_t>(img * P.A + a) * P.cls_nch + P.cls_ch) * lv.hw + pos;
-            cstride = static_cast<size_t>(lv.hw);
-            if (P.use_obj)
-                objv = ldg_head(head_ptr<T>(P.obj_src == 2 ? lv.p2 : lv.p0) + (static_cast<size_t>(img * P.A + a) * P.obj_nch + P.obj_ch) * lv.hw + pos);
+            cls = head_elem<T, NHWC>(lv, lv.p0, P.A, P.cls_nch, img, a, pos, P.cls_ch);
+            cstride = static_cast<size_t>(head_step<NHWC>(lv));
+            if (P.use_obj) objv = ldg_head(head_elem<T, NHWC>(lv, P.obj_src == 2 ? lv.p2 : lv.p0, P.A, P.obj_nch, img, a, pos, P.obj_ch));
         } else {
             const T *row = head_ptr<T>(lv.p0) + (static_cast<size_t>(img) * lv.img_rows + r) * P.row_w_in;
             cls = row + P.cls_col_in;
@@ -917,11 +927,12 @@ static cudaError_t launch_filter_t(const Plan &P, int vec, uint64_t *d_keys, int
     cudaError_t e = cudaSuccess;
     if (P.multi_label) {
         const dim3 grid(P.batch, (P.N + 255) / 256);
-        k_filter_multilabel<T><<<grid, 256, 0, stream>>>(P, d_keys, key_cap, d_counts);
+        if (P.layout == LAYOUT_ROWS_NHWC) k_filter_multilabel<T, true><<<grid, 256, 0, stream>>>(P, d_keys, key_cap, d_counts);
+        else k_filter_multilabel<T, false><<<grid, 256, 0, stream>>>(P, d_keys, key_cap, d_counts);
         return cudaGetLastError();
     }
 #ifdef YSB_PROFILING_VARIANTS
-    if (sizeof(T) == 4) {   // the variants read float32 heads; 16-bit heads always run the product kernels
+    if (sizeof(T) == 4 && P.layout != LAYOUT_ROWS_NHWC) {   // the variants read float32 NCHW heads; 16-bit and NHWC heads run the product kernels
         bool handled = false;
         e = launch_filter_variant(P, vec, d_keys, key_cap, d_counts, stream, &handled);
         if (handled) return e;
@@ -960,7 +971,7 @@ static cudaError_t launch_filter_t(const Plan &P, int vec, uint64_t *d_keys, int
         // (16-byte aligned bases, image strides that keep every image's first row 16-byte aligned)
         static int ring_env = -1;
         if (ring_env < 0) { const char *ev = getenv("YSB_ROWS_RING"); ring_env = ev ? atoi(ev) : 0; }
-        bool ring_ok = sizeof(T) == 4 && ring_env != 0 && kRingStages * smem <= 110u * 1024u;
+        bool ring_ok = sizeof(T) == 4 && P.layout != LAYOUT_ROWS_NHWC && ring_env != 0 && kRingStages * smem <= 110u * 1024u;
         for (int l = 0; l < P.L && ring_ok; ++l)
             ring_ok = (reinterpret_cast<uintptr_t>(P.lv[l].p0) & 15u) == 0 &&
                       ((static_cast<long long>(P.lv[l].img_rows) * P.row_w_in) & 3) == 0;
@@ -991,11 +1002,13 @@ static cudaError_t launch_filter_t(const Plan &P, int vec, uint64_t *d_keys, int
             if (fenv >= 0 && sizeof(T) == 4) flags = fenv;
         }
 #endif
+        // NHWC planes-family heads: the same kernel over each level's (H*W*A, K) row matrix, rows mapped to candidates
+        auto kern = P.layout == LAYOUT_ROWS_NHWC ? k_filter_rows<T, true> : k_filter_rows<T, false>;
         if (smem > 48 * 1024) {
-            e = cudaFuncSetAttribute(k_filter_rows<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
+            e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
             if (e != cudaSuccess) return e;
         }
-        k_filter_rows<T><<<grid, kRowsTile, smem, stream>>>(P, d_keys, key_cap, d_counts, flags);
+        kern<<<grid, kRowsTile, smem, stream>>>(P, d_keys, key_cap, d_counts, flags);
     }
     return cudaGetLastError();
 }

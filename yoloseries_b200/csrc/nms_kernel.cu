@@ -398,7 +398,7 @@ __device__ __forceinline__ const Plan &pass_of(const Plan &P, const ExtraPasses 
 // scattered loads; one thread per (candidate, side) keeps its 16 bin loads in flight together and runs the softmax
 // expectation in registers (the decode kernel's bin order), the four sides of a candidate meet by shuffle -- THREADS/4
 // boxes per DRAM round trip.  Every other layout: one thread per box.
-template <bool ARRAY, typename EXTRA, int THREADS, int KEEP, typename T>
+template <bool ARRAY, typename EXTRA, int THREADS, int KEEP, typename T, bool NHWC>
 __device__ __forceinline__ void decode_boxes(NmsSmem<KEEP> &S, const Plan &P, const EXTRA &X, const ArrayArgs &aa, int img,
                                              int from, int upto, int &lo_x, int &hi_x, bool &bad)
 {
@@ -416,7 +416,7 @@ __device__ __forceinline__ void decode_boxes(NmsSmem<KEEP> &S, const Plan &P, co
             if (ok) {
                 int cand = static_cast<int>(key_cand(S.keys[i]));
                 const Plan &Q = pass_of(P, X, cand);
-                sv = v8_side_value<T>(Q, img, cand, side);
+                sv = v8_side_value<T, NHWC>(Q, img, cand, side);
             }
             const unsigned qb = (tid & 31) & ~3u;
             const float s0 = __shfl_sync(0xffffffffu, sv, qb), s1 = __shfl_sync(0xffffffffu, sv, qb + 1);
@@ -436,7 +436,7 @@ __device__ __forceinline__ void decode_boxes(NmsSmem<KEEP> &S, const Plan &P, co
                 S.raw[i] = __ldg(aa.boxes + cand);
             } else {
                 const Plan &Q = pass_of(P, X, cand);
-                const float4 b = candidate_xyxy<T>(Q, img, cand);
+                const float4 b = candidate_xyxy<T, NHWC>(Q, img, cand);
                 S.raw[i] = b;
                 span(b);
             }
@@ -446,7 +446,7 @@ __device__ __forceinline__ void decode_boxes(NmsSmem<KEEP> &S, const Plan &P, co
 
 // EXTRA = NoExtraPasses (one set of heads) or ExtraPasses (TTA: boxes are decoded from the pass a candidate came from;
 // thresholds / NMS settings are those of P, identical in every pass).
-template <bool ARRAY, typename EXTRA, int THREADS, int KEEP, typename T = float>
+template <bool ARRAY, typename EXTRA, int THREADS, int KEEP, typename T = float, bool NHWC = false>
 __global__ void __launch_bounds__(THREADS, 1024 / THREADS)
 k_select_nms(const __grid_constant__ Plan P, const __grid_constant__ EXTRA X, const uint64_t *__restrict__ keys_all,
              int64_t key_cap, const int32_t *__restrict__ counts, float *__restrict__ dets,
@@ -547,7 +547,7 @@ k_select_nms(const __grid_constant__ Plan P, const __grid_constant__ EXTRA X, co
                 const int upto = min(n_use, decoded_upto + (dfl ? max(THREADS / 4, kChunk) : THREADS));
                 int d_lo = 0x7fffffff, d_hi = static_cast<int>(0x80000000u);
                 bool d_bad = false;
-                decode_boxes<ARRAY, EXTRA, THREADS, KEEP, T>(S, P, X, aa, img, decoded_upto, upto, d_lo, d_hi, d_bad);
+                decode_boxes<ARRAY, EXTRA, THREADS, KEEP, T, NHWC>(S, P, X, aa, img, decoded_upto, upto, d_lo, d_hi, d_bad);
                 decoded_upto = upto;
                 if (!ARRAY) {
                     d_lo = __reduce_min_sync(0xffffffffu, d_lo);
@@ -807,9 +807,9 @@ k_select_nms(const __grid_constant__ Plan P, const __grid_constant__ EXTRA X, co
             if (!resident) {
                 for (int i = tid; i < mm; i += THREADS) S.keys[i] = __ldg(keys + b0 + i);
                 __syncthreads();
-                decode_boxes<false, EXTRA, THREADS, KEEP, T>(S, P, X, aa, img, 0, mm, pf_lo, pf_hi, pf_bad);
+                decode_boxes<false, EXTRA, THREADS, KEEP, T, NHWC>(S, P, X, aa, img, 0, mm, pf_lo, pf_hi, pf_bad);
             } else if (decoded_upto < mm) {
-                decode_boxes<false, EXTRA, THREADS, KEEP, T>(S, P, X, aa, img, decoded_upto, mm, pf_lo, pf_hi, pf_bad);
+                decode_boxes<false, EXTRA, THREADS, KEEP, T, NHWC>(S, P, X, aa, img, decoded_upto, mm, pf_lo, pf_hi, pf_bad);
             }
             __syncthreads();
             if (!P.merge_boxes) {
@@ -1092,13 +1092,13 @@ static int device_sm_count()
     return n;
 }
 
-template <typename EXTRA, int THREADS, int KEEP, typename T>
+template <typename EXTRA, int THREADS, int KEEP, typename T, bool NHWC>
 static cudaError_t launch_flavour(const Plan &P, const EXTRA &X, const uint64_t *d_keys, int64_t key_cap, const int32_t *d_counts,
                                   float *d_dets, int32_t *d_det_idx, int32_t *d_det_cnt, cudaStream_t stream, const GatherSink &G)
 {
     // per-device attribute; set on every launch (host-side, sub-microsecond) so that a process driving several
     // devices never launches with the default 48 KB limit
-    auto kern = k_select_nms<false, EXTRA, THREADS, KEEP, T>;
+    auto kern = k_select_nms<false, EXTRA, THREADS, KEEP, T, NHWC>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(sizeof(NmsSmem<KEEP>)));
     if (e != cudaSuccess) return e;
     ArrayArgs aa{};
@@ -1118,7 +1118,7 @@ static cudaError_t launch_flavour(const Plan &P, const EXTRA &X, const uint64_t 
     return cudaGetLastError();
 }
 
-template <typename EXTRA, typename T>
+template <typename EXTRA, typename T, bool NHWC>
 static cudaError_t launch_any(const Plan &P, const EXTRA &X, const uint64_t *d_keys, int64_t key_cap, const int32_t *d_counts,
                               float *d_dets, int32_t *d_det_idx, int32_t *d_det_cnt, cudaStream_t stream, const GatherSink *sink)
 {
@@ -1140,29 +1140,39 @@ static cudaError_t launch_any(const Plan &P, const EXTRA &X, const uint64_t *d_k
 #endif
     if (g_force_threads == 512 && small_keep) threads = 512;
     if (g_force_threads == 1024) threads = 1024;
-    if (!small_keep) return launch_flavour<EXTRA, 1024, 1024, T>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, G);
-    if (threads == 512) return launch_flavour<EXTRA, 512, 320, T>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, G);
-    return launch_flavour<EXTRA, 1024, 320, T>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, G);
+    if (!small_keep) return launch_flavour<EXTRA, 1024, 1024, T, NHWC>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, G);
+    if (threads == 512) return launch_flavour<EXTRA, 512, 320, T, NHWC>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, G);
+    return launch_flavour<EXTRA, 1024, 320, T, NHWC>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, G);
 }
 
-template <typename EXTRA>
+template <typename EXTRA, bool NHWC>
 static cudaError_t launch_any_dt(const Plan &P, const EXTRA &X, const uint64_t *d_keys, int64_t key_cap, const int32_t *d_counts,
                                  float *d_dets, int32_t *d_det_idx, int32_t *d_det_cnt, cudaStream_t stream,
                                  const GatherSink *sink, int dtype)
 {
     switch (dtype) {
-    case YSB_F16: return launch_any<EXTRA, __half>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink);
+    case YSB_F16: return launch_any<EXTRA, __half, NHWC>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink);
     case YSB_BF16:
-        return launch_any<EXTRA, __nv_bfloat16>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink);
-    default: return launch_any<EXTRA, float>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink);
+        return launch_any<EXTRA, __nv_bfloat16, NHWC>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink);
+    default: return launch_any<EXTRA, float, NHWC>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink);
     }
+}
+
+// NHWC heads (LAYOUT_ROWS_NHWC, YSB_INPUT_RAW_HEADS_NHWC): the kernel's box decode addresses channels-last memory
+template <typename EXTRA>
+static cudaError_t launch_any_layout(const Plan &P, const EXTRA &X, const uint64_t *d_keys, int64_t key_cap,
+                                     const int32_t *d_counts, float *d_dets, int32_t *d_det_idx, int32_t *d_det_cnt,
+                                     cudaStream_t stream, const GatherSink *sink, int dtype)
+{
+    if (P.layout == LAYOUT_ROWS_NHWC) return launch_any_dt<EXTRA, true>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink, dtype);
+    return launch_any_dt<EXTRA, false>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink, dtype);
 }
 
 cudaError_t launch_select_nms(const Plan &P, const uint64_t *d_keys, int64_t key_cap, const int32_t *d_counts,
                               float *d_dets, int32_t *d_det_idx, int32_t *d_det_cnt, cudaStream_t stream,
                               const GatherSink *sink, int dtype)
 {
-    return launch_any_dt(P, NoExtraPasses{}, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink, dtype);
+    return launch_any_layout(P, NoExtraPasses{}, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink, dtype);
 }
 
 // test-time augmentation: one selection/NMS over the key lists the passes appended to; X describes passes 1..n.  sink:
@@ -1171,7 +1181,7 @@ cudaError_t launch_select_nms_tta(const Plan &P, const ExtraPasses &X, const uin
                                   const int32_t *d_counts, float *d_dets, int32_t *d_det_idx, int32_t *d_det_cnt,
                                   cudaStream_t stream, const GatherSink *sink, int dtype)
 {
-    return launch_any_dt(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink, dtype);
+    return launch_any_layout(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink, dtype);
 }
 
 // ---- array flavour: utils.numba_nms / utils.gpu_nms over one explicit (m,4)/(m) pair ---------------------------

@@ -43,15 +43,16 @@ const ysb_params *params_of(const at::Tensor &blob)
     return reinterpret_cast<const ysb_params *>(blob.data_ptr());
 }
 
-void check_cuda(const at::Tensor &t, at::ScalarType dtype, const c10::Device &dev, const char *name)
+void check_cuda(const at::Tensor &t, at::ScalarType dtype, const c10::Device &dev, const char *name, bool contiguous = true)
 {
     TORCH_CHECK_VALUE(t.is_cuda(), name, ": expected a CUDA tensor (yoloseries_b200 has no CPU fallback)");
     TORCH_CHECK_VALUE(t.device() == dev, name, ": on ", t.device(), ", the other tensors are on ", dev);
     TORCH_CHECK_VALUE(t.scalar_type() == dtype, name, ": expected ", dtype, ", got ", t.scalar_type());
-    TORCH_CHECK_VALUE(t.is_contiguous(), name, ": expected a contiguous tensor");
+    if (contiguous) TORCH_CHECK_VALUE(t.is_contiguous(), name, ": expected a contiguous tensor");
 }
 
-// heads -> array of device pointers; every head of one dtype, contiguous, on one device
+// heads -> array of device pointers; every head of one dtype, on one device (their strides: check_head_layout, once the
+// params say which layout the heads have)
 std::vector<const void *> head_pointers(const at::TensorList &heads, c10::Device &dev)
 {
     TORCH_CHECK_VALUE(!heads.empty(), "heads: no tensors");
@@ -59,10 +60,41 @@ std::vector<const void *> head_pointers(const at::TensorList &heads, c10::Device
     std::vector<const void *> p;
     p.reserve(heads.size());
     for (const auto &h : heads) {
-        check_cuda(h, heads[0].scalar_type(), dev, "heads");
+        check_cuda(h, heads[0].scalar_type(), dev, "heads", false);
         p.push_back(h.data_ptr());
     }
     return p;
+}
+
+// A channels-last head of the family (include/ysb_postproc.h, YSB_INPUT_RAW_HEADS_NHWC): (b, K, H, W) stored as
+// (b, H, W, K), or YOLOX' (b, A, K, H, W) view of a channels-last (b, A*K, H, W).  Strides of size-1 dims do not matter.
+bool is_channels_last_head(const at::Tensor &t, int family)
+{
+    std::vector<int64_t> want;
+    const auto s = t.sizes();
+    if ((family == YSB_YOLOV5 || family == YSB_YOLOV8 || family == YSB_FCOS) && t.dim() == 4)
+        want = {s[2] * s[3] * s[1], 1, s[3] * s[1], s[1]};
+    else if (family == YSB_YOLOX && t.dim() == 5)
+        want = {s[3] * s[4] * s[1] * s[2], s[2], 1, s[4] * s[1] * s[2], s[1] * s[2]};
+    else
+        return false;
+    for (int64_t d = 0; d < t.dim(); ++d)
+        if (s[d] != 1 && t.stride(d) != want[d]) return false;
+    return true;
+}
+
+// the heads' memory is the layout the params announce: channels-last for YSB_INPUT_RAW_HEADS_NHWC, contiguous otherwise
+void check_head_layout(const at::TensorList &heads, const ysb_params *p)
+{
+    for (const auto &h : heads) {
+        if (p->input_kind == YSB_INPUT_RAW_HEADS_NHWC) {
+            // (a message of string literals only: an exception message that streams tensor sizes crashed the process here)
+            TORCH_CHECK_VALUE(is_channels_last_head(h, p->family),
+                              "heads: expected channels-last heads of the params' family (params.input_kind)");
+        } else {
+            TORCH_CHECK_VALUE(h.is_contiguous(), "heads: expected a contiguous tensor");
+        }
+    }
 }
 
 // the heads' dtype is the one the params announce (ysb_params.head_dtype: float32, float16 or bfloat16)
@@ -89,6 +121,7 @@ void postprocess(at::TensorList heads, const at::Tensor &params, at::Tensor work
     const auto ptrs = head_pointers(heads, dev);
     const ysb_params *p = params_of(params);
     check_head_dtype(heads, p);
+    check_head_layout(heads, p);
     check_cuda(workspace, at::kByte, dev, "workspace");
     check_cuda(dets, at::kFloat, dev, "dets");
     check_cuda(det_idx, at::kInt, dev, "det_idx");
@@ -109,6 +142,7 @@ void filter_candidates(at::TensorList heads, const at::Tensor &params, at::Tenso
     const auto ptrs = head_pointers(heads, dev);
     const ysb_params *p = params_of(params);
     check_head_dtype(heads, p);
+    check_head_layout(heads, p);
     check_cuda(keys, at::kLong, dev, "keys");
     check_cuda(counts, at::kInt, dev, "counts");
     TORCH_CHECK_VALUE(keys.dim() == 2 && keys.size(0) == p->batch && counts.numel() >= 4 * static_cast<int64_t>(p->batch),
@@ -127,6 +161,7 @@ void select_nms(at::TensorList heads, const at::Tensor &params, const at::Tensor
     const auto ptrs = head_pointers(heads, dev);
     const ysb_params *p = params_of(params);
     check_head_dtype(heads, p);
+    check_head_layout(heads, p);
     check_cuda(keys, at::kLong, dev, "keys");
     check_cuda(counts, at::kInt, dev, "counts");
     check_cuda(dets, at::kFloat, dev, "dets");
@@ -151,6 +186,7 @@ at::Tensor decode(at::TensorList heads, const at::Tensor &params)
     const auto ptrs = head_pointers(heads, dev);
     const ysb_params *p = params_of(params);
     check_head_dtype(heads, p);
+    check_head_layout(heads, p);
     int64_t n = 0;
     int32_t row_w = 0;
     check_status(ysb_num_candidates(p, &n, &row_w), "ysb_num_candidates");
@@ -168,6 +204,7 @@ void decode_into(at::TensorList heads, const at::Tensor &params, at::Tensor merg
     const auto ptrs = head_pointers(heads, dev);
     const ysb_params *p = params_of(params);
     check_head_dtype(heads, p);
+    check_head_layout(heads, p);
     check_cuda(merged, at::kFloat, dev, "merged");
     TORCH_CHECK_VALUE(merged.dim() == 3 && merged.size(0) == p->batch, "merged must be (batch, rows_total, C')");
     c10::cuda::CUDAGuard guard(dev);

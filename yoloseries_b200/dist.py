@@ -65,6 +65,8 @@ import os
 
 from . import _lib
 
+_LAYOUT_NAMES = {_lib.INPUT_RAW_HEADS: "contiguous", _lib.INPUT_RAW_HEADS_NHWC: "channels-last"}
+
 
 def exchange_bytes(payload: bytes, group=None):
     """All-gather one small bytes object per rank (IPC handles) through torch.distributed; works on gloo and NCCL."""
@@ -220,6 +222,9 @@ class ShardedPostProcessor:
         t = spp.submit_tta(passes)             # every pass's filter -> one merged NMS (+ peer stores) -> arrival wait
         rows, cnt = spp.gathered(t)            # as above; rows in un-augmented network-input pixels
 
+    Contiguous (NCHW) and channels-last heads (YOLOv5, YOLOX, YOLOv8, FCOS; include/ysb_postproc.h) are both read as they
+    are; like the dtype, the first submission fixes the layout and a later batch in the other one raises ValueError.
+
     Lanes, graphs and the gather work as for ``submit``.  The first submission fixes the kind (plain or TTA): a processor
     takes only ``submit`` or only ``submit_tta`` calls.  For TTA it also fixes the number of passes, each pass's
     (img_h, img_w, scale, flip_axis) and the head shapes, and sizes the key buffers to the passes' summed key slots; a
@@ -272,6 +277,7 @@ class ShardedPostProcessor:
             return
         self._ent = self.pp._prepare(flat, self.batch, self.img_h, self.img_w, _lib.INPUT_RAW_HEADS)
         self._head_dtype = flat[0].dtype
+        self._layout = self._ent["params"].input_kind
         self._alloc_lanes(self._ent["N"] * self._slots_per_candidate())
 
     def _slots_per_candidate(self):
@@ -286,6 +292,7 @@ class ShardedPostProcessor:
         self._tta = dict(geom=geom, ents=[e for _, e in ents], params=params,
                          per_pass=(ctypes.c_int32 * n)(*[len(flat) for flat, _ in ents]))
         self._head_dtype = ents[0][0][0].dtype
+        self._layout = ents[0][1]["params"].input_kind
         self._alloc_lanes(sum(e["N"] for _, e in ents) * self._slots_per_candidate())
 
     def _alloc_lanes(self, n):
@@ -362,7 +369,7 @@ class ShardedPostProcessor:
     def submit(self, heads, events=None, sync_input=True):
         """Enqueue one batch.  ``events``: optional 3 timing events (start, filter done, NMS done) recorded on the lane's
         stream.  ``sync_input=False`` skips the wait on the caller's current stream (heads known to be ready)."""
-        from .engine import flatten_heads
+        from .engine import flatten_heads, head_layout
         if self._kind == "tta":
             raise ValueError("this processor was set up for test-time-augmented batches: use submit_tta")
         flat = flatten_heads(self.family, heads)
@@ -372,7 +379,13 @@ class ShardedPostProcessor:
         self._kind = "plain"
         if any(t.dtype != self._head_dtype for t in flat):
             raise ValueError(f"this processor was set up for {self._head_dtype} heads, got {sorted({str(t.dtype) for t in flat})}")
+        self._check_layout(head_layout(self.family, flat))
         return self._submit(flat, events, sync_input)
+
+    def _check_layout(self, kind):
+        if kind != self._layout:
+            raise ValueError(f"this processor was set up for {_LAYOUT_NAMES[self._layout]} heads, got "
+                             f"{_LAYOUT_NAMES[kind]} ones")
 
     def submit_tta(self, passes, events=None, sync_input=True):
         """Enqueue one test-time-augmented batch: ``passes`` = [(heads, img_h, img_w, scale, flip_axis), ...] as for
@@ -403,7 +416,8 @@ class ShardedPostProcessor:
         if self._tta is None:
             self._prepare_tta(ents, geom)
             self._kind = "tta"
-        elif any(e is not k for (_, e), k in zip(ents, self._tta["ents"])):
+        self._check_layout(ents[0][1]["params"].input_kind)
+        if any(e is not k for (_, e), k in zip(ents, self._tta["ents"])):
             raise ValueError("the head shapes differ from those of the first submit_tta")
         return self._submit([t for flat in flats for t in flat], events, sync_input)
 

@@ -15,6 +15,12 @@ from ._lib import YsbParams
 # element types the raw heads may have (ysb_dtype): 16-bit heads are read as they are and widened on the device
 HEAD_DTYPES = {torch.float32: _lib.DTYPE_F32, torch.float16: _lib.DTYPE_F16, torch.bfloat16: _lib.DTYPE_BF16}
 
+# families whose raw heads the engine also reads in channels-last memory (include/ysb_postproc.h, YSB_INPUT_RAW_HEADS_NHWC)
+NHWC_FAMILIES = ("yolov5", "yolox", "yolov8", "fcos")
+# A channels-last head is read as rows of one anchor's channels (5+C, 4*reg+C or C values); the filter kernel stages 128 of
+# them in shared memory, at most 227 KB: 128 * (width | 1) * 4 bytes (csrc/c_abi.cu), i.e. rows of up to 453 values.
+NHWC_MAX_ROW_WIDTH = 453
+
 # strides fixed by the reference evaluators (self.ds_scales), trainer/eval_yolov5.py:21, eval_yolov7.py, eval_fcos.py:18
 _FIXED_STRIDES = {"yolov5": (8, 16, 32), "yolov7": (8, 16, 32), "fcos": (8, 16, 32, 64, 128)}
 
@@ -75,13 +81,58 @@ def _leaves(heads):
     return [t for v in heads for t in _leaves(v)]
 
 
-def native_heads(heads):
+def nhwc_row_width(family, num_class, dfl_bins=16):
+    """Values per row of a channels-last head of ``family``: the channels of one anchor (FCOS: of the cls tensor)."""
+    C = int(num_class)
+    return {"yolov5": 5 + C, "yolox": 5 + C, "yolov8": 4 * int(dfl_bins) + C, "fcos": C}[family]
+
+
+def _channels_last_strides(family, t):
+    """The strides ``t`` has when it is a channels-last head of ``family`` (None: no such pattern for its rank)."""
+    if family in ("yolov5", "yolov8", "fcos") and t.dim() == 4:   # (b, K, H, W) stored as (b, H, W, K)
+        _, K, H, W = t.shape
+        return (H * W * K, 1, W * K, K)
+    if family == "yolox" and t.dim() == 5:                         # (b, A, K, H, W) view of a channels-last (b, A*K, H, W)
+        _, A, K, H, W = t.shape
+        return (H * W * A * K, K, 1, W * A * K, A * K)
+    return None
+
+
+def is_channels_last_head(family, t):
+    """True when ``t`` has the channels-last memory of a ``family`` head; the strides of size-1 dims do not matter (a
+    1-channel ctr or a 1x1 level qualifies)."""
+    want = _channels_last_strides(family, t)
+    return want is not None and all(n == 1 or s == w for n, s, w in zip(t.shape, t.stride(), want))
+
+
+def head_layout(family, flat):
+    """Input kind of a flat head list: INPUT_RAW_HEADS when every tensor is contiguous (checked first, so a list that
+    fits both patterns is NCHW), INPUT_RAW_HEADS_NHWC when every tensor is a channels-last head of ``family`` (YOLOv5,
+    YOLOX, YOLOv8, FCOS).  Anything else -- views of other strides, or levels of different layouts -- raises ValueError."""
+    if all(t.is_contiguous() for t in flat):
+        return _lib.INPUT_RAW_HEADS
+    if family in NHWC_FAMILIES and all(is_channels_last_head(family, t) for t in flat):
+        return _lib.INPUT_RAW_HEADS_NHWC
+    cl = f"; or all channels-last ({', '.join(NHWC_FAMILIES)})" if family in NHWC_FAMILIES else ""
+    raise ValueError(f"head tensors must be contiguous float32, float16 or bfloat16{cl}, got strides "
+                     f"{[tuple(t.stride()) for t in flat]} for shapes {[tuple(t.shape) for t in flat]}")
+
+
+def native_heads(heads, family=None, num_class=None, dfl_bins=16):
     """Model outputs as the engine takes them: unchanged when every tensor is contiguous and all share one of float32,
     float16 or bfloat16 (16-bit heads are read natively, no conversion pass); anything else goes through
-    normalise_heads."""
+    normalise_heads.  With ``family`` (and ``num_class``, ``dfl_bins`` for YOLOv8), heads that are all channels-last
+    (a model run with torch.channels_last) are passed through unchanged too, unless their rows are wider than
+    NHWC_MAX_ROW_WIDTH."""
     leaves = _leaves(heads)
-    if leaves and leaves[0].dtype in HEAD_DTYPES and all(t.dtype == leaves[0].dtype and t.is_contiguous() for t in leaves):
-        return heads
+    if leaves and leaves[0].dtype in HEAD_DTYPES and all(t.dtype == leaves[0].dtype for t in leaves):
+        if all(t.is_contiguous() for t in leaves):
+            return heads
+        if family in NHWC_FAMILIES and all(is_channels_last_head(family, t) for t in leaves):
+            if num_class is None:
+                raise ValueError("native_heads: num_class is required with a family")
+            if nhwc_row_width(family, num_class, dfl_bins) <= NHWC_MAX_ROW_WIDTH:
+                return heads
     return normalise_heads(heads)
 
 
@@ -240,7 +291,7 @@ def validate_heads(family, flat, num_class, anchors=None, dfl_bins=16, decoded_r
         bad("no tensors")
     b = flat[0].shape[0]
     for i, t in enumerate(flat):
-        if t.dtype not in HEAD_DTYPES or not t.is_contiguous():
+        if t.dtype not in HEAD_DTYPES or (decoded_row_w is not None and not t.is_contiguous()):
             raise ValueError(f"head tensors must be contiguous float32, float16 or bfloat16, got {t.dtype}")
         if t.dtype != flat[0].dtype:
             raise ValueError(f"head tensors must share one dtype (contiguous float32, float16 or bfloat16), got "
@@ -254,7 +305,8 @@ def validate_heads(family, flat, num_class, anchors=None, dfl_bins=16, decoded_r
             raise ValueError(f"decoded tensor must be contiguous float32, got {flat[0].dtype}")
         if len(flat) != 1 or flat[0].dim() != 3 or flat[0].shape[2] != decoded_row_w:
             raise ValueError(f"decoded tensor must be (b, N, {decoded_row_w}), got {tuple(flat[0].shape)}")
-        return
+        return _lib.INPUT_DECODED_ROWS
+    kind = head_layout(family, flat)   # contiguous (NCHW) or, for the planes families, channels-last
     if family in ("yolov5", "yolov7"):
         if anchors is None:
             bad("anchors (L, A, 2) are required")
@@ -296,6 +348,7 @@ def validate_heads(family, flat, num_class, anchors=None, dfl_bins=16, decoded_r
                     f"{tuple(c.shape)}, {tuple(r.shape)}, {tuple(q.shape)}")
     else:
         raise ValueError(f"unknown family {family!r}")
+    return kind
 
 
 class DetectionBuffers:
@@ -327,19 +380,26 @@ class PostProcessor:
         dev = flat[0].device
         if dev.type != "cuda":
             raise RuntimeError("yoloseries_b200 runs on CUDA devices only (no CPU fallback); got " + str(dev))
-        if input_kind == _lib.INPUT_RAW_HEADS:
-            validate_heads(self.family, flat, self.hyp["num_class"], self.anchors, self.hyp.get("reg", 16))
+        raw = input_kind != _lib.INPUT_DECODED_ROWS
+        if raw:
+            # the layout picks the input kind: contiguous NCHW heads or channels-last ones
+            input_kind = validate_heads(self.family, flat, self.hyp["num_class"], self.anchors, self.hyp.get("reg", 16))
+            if input_kind == _lib.INPUT_RAW_HEADS_NHWC:
+                k = nhwc_row_width(self.family, self.hyp["num_class"], self.hyp.get("reg", 16))
+                if k > NHWC_MAX_ROW_WIDTH:
+                    raise ValueError(f"{self.family} channels-last heads: rows of {k} values exceed the limit of "
+                                     f"{NHWC_MAX_ROW_WIDTH} (NHWC_MAX_ROW_WIDTH); pass contiguous heads")
         else:
             for t in flat:
                 if t.dtype != torch.float32 or not t.is_contiguous():
                     raise ValueError("head tensors must be contiguous float32")
         shapes = None
-        if input_kind == _lib.INPUT_RAW_HEADS and self.family not in ("retinanet", "retinanet_exp"):
+        if raw and self.family not in ("retinanet", "retinanet_exp"):
             shapes = _level_shapes(self.family, flat, self.hyp["num_class"])
         elif self.family not in ("retinanet", "retinanet_exp"):
             strides = _FIXED_STRIDES.get(self.family) or ((4, 8, 16, 32) if self.family == "yolov8" else (8, 16, 32))
             shapes = [(img_h // s, img_w // s) for s in strides]
-        na = flat[0].shape[1] if (self.family == "yolox" and input_kind == _lib.INPUT_RAW_HEADS) else None
+        na = flat[0].shape[1] if (self.family == "yolox" and raw) else None
         rows = int(flat[0].shape[1]) if input_kind == _lib.INPUT_DECODED_ROWS else 0
         key = (batch, img_h, img_w, input_kind, tuple(shapes or ()), dev.index, na, rows, tta, flat[0].dtype)
         ent = self._cache.get(key)
@@ -357,7 +417,7 @@ class PostProcessor:
                        workspace=torch.empty(max(ws.value, 1), dtype=torch.uint8, device=dev),
                        out=DetectionBuffers(batch, params.max_det, dev))
             self._cache[key] = ent
-        if input_kind == _lib.INPUT_RAW_HEADS and self.family in ("retinanet", "retinanet_exp") and flat[0].shape[1] != ent["N"]:
+        if raw and self.family in ("retinanet", "retinanet_exp") and flat[0].shape[1] != ent["N"]:
             raise ValueError(f"{self.family} heads: {flat[0].shape[1]} anchors per image, but a {img_h}x{img_w} input has {ent['N']}")
         if input_kind == _lib.INPUT_DECODED_ROWS:
             validate_heads(self.family, flat, self.hyp["num_class"], decoded_row_w=ent["row_w"])
@@ -420,6 +480,8 @@ class PostProcessor:
             ents.append((flat, self._prepare(flat, flat[0].shape[0], int(img_h), int(img_w), _lib.INPUT_RAW_HEADS, tta)))
         if len({e["params"].batch for _, e in ents}) != 1:
             raise ValueError("every pass must hold the same images")
+        if len({e["params"].input_kind for _, e in ents}) != 1:
+            raise ValueError("every pass must have heads of one layout (all contiguous or all channels-last)")
         return ents
 
     def decode_tta(self, passes, org_hw):
@@ -558,9 +620,17 @@ class PipelinedPostProcessor:
         self._pps = [PostProcessor(family, hyp, anchors, compute_metric) for _ in range(lanes)]
         self._streams = None
         self._next = 0
+        self._layout = None   # contiguous or channels-last raw heads: fixed by the first submission
 
     def submit(self, heads, img_h, img_w, decoded=False):
         flat = [heads] if decoded else flatten_heads(self._pps[0].family, heads)
+        if not decoded:
+            kind = head_layout(self._pps[0].family, flat)
+            if self._layout is None:
+                self._layout = kind
+            elif kind != self._layout:
+                names = {_lib.INPUT_RAW_HEADS: "contiguous", _lib.INPUT_RAW_HEADS_NHWC: "channels-last"}
+                raise ValueError(f"this processor was set up for {names[self._layout]} heads, got {names[kind]} ones")
         dev = flat[0].device
         if self._streams is None:
             self._streams = [torch.cuda.Stream(device=dev) for _ in self._pps]

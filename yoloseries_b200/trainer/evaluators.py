@@ -41,6 +41,12 @@ class _Evaluator:
             self.conf_threshold = hyp[pre + "conf_threshold"]
         self._pp = PostProcessor(self.family, hyp, anchors=anchors, compute_metric=compute_metric)
 
+    def _native(self, heads):
+        """The model's outputs as the engine reads them: contiguous or channels-last heads of one 16/32-bit float type are
+        passed through unchanged; anything else (and channels-last rows wider than the filter kernel's tile) is converted
+        by normalise_heads."""
+        return native_heads(heads, self.family, self.num_class, self.hyp.get("reg", 16))
+
     # ---- reference API -------------------------------------------------------------------------------------------
     @torch.no_grad()
     def __call__(self, inputs, info=None):
@@ -54,14 +60,14 @@ class _Evaluator:
             # three model forwards, then ONE fused call: no decoded or merged tensor is written (ysb_postprocess_tta)
             out = self._pp.run_tta(self._tta_passes(inputs), (inputs.size(2), inputs.size(3)), info=info)
             return self._pp.to_list(out)
-        heads = native_heads(self._model(inputs))
+        heads = self._native(self._model(inputs))
         out = self._pp.run(heads, inputs.size(2), inputs.size(3), info=info)
         return self._pp.to_list(out)
 
     @torch.no_grad()
     def do_inference(self, inputs):
         """model forward + decode -> (b, N, C') float32 on the heads' device (one CUDA kernel, ysb_decode)."""
-        heads = native_heads(self._model(inputs))
+        heads = self._native(self._model(inputs))
         return self._pp.decode(heads, inputs.size(2), inputs.size(3))
 
     def numba_nms(self, preds_out):
@@ -136,7 +142,7 @@ class _Evaluator:
         for s, f in zip([1, 0.83, 0.67], [None, 2, 3]):
             img = inputs.flip(dims=(f,)) if f else inputs
             img = self.scale_img(img, s)
-            passes.append((native_heads(self._model(img)), img.size(2), img.size(3), s, f))
+            passes.append((self._native(self._model(img)), img.size(2), img.size(3), s, f))
         return passes
 
     def test_time_augmentation(self, inputs):
