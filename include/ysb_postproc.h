@@ -49,8 +49,13 @@ extern "C" {
 #define YSB_MAX_ANCHORS 9
 #define YSB_MAX_PASSES 4             /* test-time-augmentation passes merged by ysb_postprocess_tta */
 #define YSB_MAX_DET_LIMIT 1024      /* max_det upper bound (kept list lives in shared memory) */
-#define YSB_MAX_CANDIDATES 4194303  /* candidate index must fit 22 bits of the sort key */
-#define YSB_MAX_CLASSES 1024        /* class id must fit 10 bits of the sort key */
+/* Sort-key layouts (ysb_filter_candidates): up to 1024 classes the key has 22 candidate bits and 10 class bits; from
+ * 1025 to YSB_MAX_CLASSES classes it has 21 candidate bits and 11 class bits, so those calls accept at most
+ * YSB_MAX_CANDIDATES_WIDE candidates per image (summed over the passes of a TTA call).  Libraries before 2048-class
+ * support refuse num_classes > 1024 with YSB_ERR_LIMIT. */
+#define YSB_MAX_CANDIDATES 4194303       /* candidate index must fit 22 bits of the sort key (num_classes <= 1024) */
+#define YSB_MAX_CANDIDATES_WIDE 2097151  /* 21 bits: the limit when num_classes > 1024 */
+#define YSB_MAX_CLASSES 2048             /* class id must fit 11 bits of the wide sort key */
 #define YSB_MAX_PEERS 16            /* ranks (GPUs of one NVLink domain) in a detection gather */
 #define YSB_IPC_HANDLE_BYTES 64     /* sizeof(cudaIpcMemHandle_t) */
 
@@ -179,7 +184,8 @@ int ysb_decode_into(const ysb_params *p, const void *const *d_heads, int num_hea
                     int64_t row_offset, void *stream);
 
 /* Filter + class pick + compaction.  d_keys: (batch, key_capacity) uint64 sort keys
- *   key = score_bits << 32 | (YSB_MAX_CANDIDATES - cand) << 10 | (1023 - cls)
+ *   key = score_bits << 32 | (YSB_MAX_CANDIDATES - cand) << 10 | (1023 - cls)         num_classes <= 1024
+ *   key = score_bits << 32 | (YSB_MAX_CANDIDATES_WIDE - cand) << 11 | (2047 - cls)   num_classes 1025..2048
  * so that "descending key" == (score desc, candidate asc, class asc), the order numba_nms visits boxes.
  * d_counts: (batch, 4) int32 = {survivors M, pre-mask passes (FCOS top-k), max score bits, ~min score bits};
  * zero-filled by this call before the kernels run.  key_capacity >= N (N*C with multi_label). */

@@ -14,6 +14,8 @@ YSB_MAX_LEVELS = 8
 YSB_MAX_ANCHORS = 9
 YSB_MAX_DET_LIMIT = 1024
 YSB_MAX_CANDIDATES = 4194303
+YSB_MAX_CANDIDATES_WIDE = 2097151   # candidate limit when num_classes > 1024 (11-bit class field of the sort key)
+YSB_MAX_CLASSES = 2048
 
 # enum ysb_family
 YOLOV5, YOLOV7, YOLOX, YOLOV8, RETINANET, RETINANET_EXP, FCOS = range(7)
@@ -212,6 +214,20 @@ def check(status, what="ysb call"):
     if status == YSB_ERR_UNSUPPORTED:
         raise NotImplementedError(f"{what}: {msg}")
     raise YsbError(status, f"{what}: {msg}")
+
+
+def unpack_keys(keys_u64, num_classes):
+    """Sort keys written by ysb_filter_candidates -> (score float32, cand int64, cls int64).  The key layout depends on the
+    call's class count (include/ysb_postproc.h): 10 class bits up to 1024 classes, 11 above."""
+    import numpy as np
+    cls_bits = 11 if num_classes > 1024 else 10
+    cand_mask = (1 << (32 - cls_bits)) - 1
+    cls_mask = (1 << cls_bits) - 1
+    k = np.asarray(keys_u64).astype(np.uint64)
+    score = (k >> np.uint64(32)).astype(np.uint32).view(np.float32)
+    cand = cand_mask - ((k >> np.uint64(cls_bits)) & np.uint64(cand_mask)).astype(np.int64)
+    cls = cls_mask - (k & np.uint64(cls_mask)).astype(np.int64)
+    return score, cand, cls
 
 
 def head_pointer_array(tensors):

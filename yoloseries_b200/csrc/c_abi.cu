@@ -77,6 +77,12 @@ struct Built {
 
 static size_t dtype_bytes(int dtype) { return dtype == YSB_F32 ? 4 : 2; }
 
+// candidates per image (summed over TTA passes) the sort key of a call with this many classes can index
+static int64_t max_candidates(int num_classes)
+{
+    return wide_keys(num_classes) ? YSB_MAX_CANDIDATES_WIDE : YSB_MAX_CANDIDATES;
+}
+
 static int expected_heads(const ysb_params *p)
 {
     if (p->input_kind == YSB_INPUT_DECODED_ROWS) return 1;
@@ -158,10 +164,10 @@ static int build_plan(const ysb_params *p, const void *const *d_heads, int num_h
         lv.stride = p->level_stride[l];
         lv.cand_off = static_cast<int>(n);
         n += static_cast<int64_t>(A) * lv.hw;
-        if (n > YSB_MAX_CANDIDATES) return YSB_ERR_LIMIT;
+        if (n > max_candidates(C)) return YSB_ERR_LIMIT;
     }
     if (p->input_kind == YSB_INPUT_DECODED_ROWS && p->decoded_rows > 0) n = p->decoded_rows;
-    if (p->decoded_rows < 0 || n > YSB_MAX_CANDIDATES) return YSB_ERR_LIMIT;
+    if (p->decoded_rows < 0 || n > max_candidates(C)) return YSB_ERR_LIMIT;
     P.N = static_cast<int>(n);
 
     // ---- per-family operators and layouts (SURVEY.md 8a-1, 8a-2) ---------------------------------------------
@@ -227,9 +233,10 @@ static int build_plan(const ysb_params *p, const void *const *d_heads, int num_h
         if (p->family == YSB_FCOS) P.obj_src = 0;
     }
 
-    // rows layout: the filter kernel stages a tile of 128 rows in shared memory (filter_kernels.cu, k_filter_rows);
-    // rows wider than ~450 floats would not fit the 227 KB a CTA can opt into
-    if (P.layout != LAYOUT_PLANES && static_cast<size_t>(128) * (P.row_w_in | 1) * sizeof(float) > 227u * 1024u) return YSB_ERR_LIMIT;
+    // channels-last heads: the filter kernel stages a tile of 128 rows in shared memory (filter_kernels.cu, k_filter_rows);
+    // rows wider than ~450 floats would not fit the 227 KB a CTA can opt into.  Other rows inputs that wide (YOLOv7,
+    // RetinaNet, decoded rows) run k_filter_rows_wide, which reads its rows straight from global memory.
+    if (nhwc && !rows_fit_tile(P.row_w_in)) return YSB_ERR_LIMIT;
 
     out->heads_expected = expected_heads(p);
     out->dtype = p->head_dtype;
@@ -559,7 +566,7 @@ static int build_passes(const ysb_params *passes, int num_passes, const void *co
         out->b[i].plan.cand_base = static_cast<int>(base);
         base += out->b[i].plan.N;
         slots += key_slots(out->b[i].plan);
-        if (base > YSB_MAX_CANDIDATES) return YSB_ERR_LIMIT;
+        if (base > max_candidates(p->num_classes)) return YSB_ERR_LIMIT;
     }
     out->base[num_passes] = base;
     out->slots = slots;

@@ -58,7 +58,8 @@ __device__ __forceinline__ CandAddr<T> cand_addr(const Plan &P, int img, int can
 
 // ROWS = candidates per CTA: 32 for channels-last heads (their rows are contiguous anyway; NHWC planes-family heads take
 // the rows branch: cand_addr gives class step 1 and decode_box_cols reads their boxes), 128 for NCHW planes so that
-// every plane access of a CTA covers 512 contiguous bytes.
+// every plane access of a CTA covers 512 contiguous bytes; 16 for rows whose [32][row_w] tile exceeds the launcher's
+// 200 KB (more than ~1596 classes), with 16 threads per row in the rows branch.
 template <int ROWS, typename T, bool NHWC>
 __global__ void __launch_bounds__(kDecThreads) k_decode_rows(const __grid_constant__ Plan P, float *__restrict__ out,
                                                               int64_t rows_total, int64_t row_offset)
@@ -129,30 +130,31 @@ __global__ void __launch_bounds__(kDecThreads) k_decode_rows(const __grid_consta
     } else {
         // eight threads per candidate row (32 rows x 8): a warp reads 4 rows x 32 contiguous bytes per step, every
         // fetched sector fully used; kDecInFlightRows loads in flight per thread.  Lane-per-candidate box / objectness decode.
-        const int r = threadIdx.x >> 3, q = threadIdx.x & 7;
+        constexpr int TPR = ROWS >= 32 ? 8 : kDecThreads / ROWS;   // threads per row
+        const int r = threadIdx.x / TPR, q = threadIdx.x % TPR;
         if (r < nrows) {
             const CandAddr<T> ca = cand_addr<T, NHWC>(P, img, c0 + r);
             float *tc = tile + r * rw + P.cls_col;
             int k = q;
-            for (; k + 8 * (kDecInFlightRows - 1) < P.C; k += 8 * kDecInFlightRows) {
+            for (; k + TPR * (kDecInFlightRows - 1) < P.C; k += TPR * kDecInFlightRows) {
                 float v[kDecInFlightRows];
 #pragma unroll
-                for (int u = 0; u < kDecInFlightRows; ++u) v[u] = ldg_head(ca.cls + k + 8 * u);
+                for (int u = 0; u < kDecInFlightRows; ++u) v[u] = ldg_head(ca.cls + k + TPR * u);
                 bool redo = false;
 #pragma unroll
-                for (int u = 0; u < kDecInFlightRows; ++u) tc[k + 8 * u] = sigmoid_fast(v[u], redo);
+                for (int u = 0; u < kDecInFlightRows; ++u) tc[k + TPR * u] = sigmoid_fast(v[u], redo);
                 if (__builtin_expect(redo, 0)) {
 #pragma unroll
-                    for (int u = 0; u < kDecInFlightRows; ++u) tc[k + 8 * u] = sigmoid_ref(v[u]);
+                    for (int u = 0; u < kDecInFlightRows; ++u) tc[k + TPR * u] = sigmoid_ref(v[u]);
                 }
             }
             if (k < P.C) {
                 float v[kDecInFlightRows];
 #pragma unroll
-                for (int u = 0; u < kDecInFlightRows; ++u) v[u] = (k + 8 * u < P.C) ? ldg_head(ca.cls + k + 8 * u) : 0.0f;
+                for (int u = 0; u < kDecInFlightRows; ++u) v[u] = (k + TPR * u < P.C) ? ldg_head(ca.cls + k + TPR * u) : 0.0f;
 #pragma unroll
                 for (int u = 0; u < kDecInFlightRows; ++u)
-                    if (k + 8 * u < P.C) tc[k + 8 * u] = sigmoid_ref(v[u]);
+                    if (k + TPR * u < P.C) tc[k + TPR * u] = sigmoid_ref(v[u]);
             }
         }
         if (warp == 0 && lane < nrows) {
@@ -199,7 +201,8 @@ static cudaError_t launch_decode_dt(const Plan &P, float *d_out, int64_t rows_to
     if (P.layout == LAYOUT_ROWS_NHWC) return launch_decode_t<32, T, true>(P, d_out, rows_total, row_offset, stream);   // rows branch, 32 rows / CTA
     if (P.layout == LAYOUT_PLANES && static_cast<size_t>(128) * P.row_w * sizeof(float) <= 100 * 1024)
         return launch_decode_t<128, T>(P, d_out, rows_total, row_offset, stream);
-    return launch_decode_t<32, T>(P, d_out, rows_total, row_offset, stream);
+    if (static_cast<size_t>(32) * P.row_w * sizeof(float) <= 200 * 1024) return launch_decode_t<32, T>(P, d_out, rows_total, row_offset, stream);
+    return launch_decode_t<16, T>(P, d_out, rows_total, row_offset, stream);   // rows of more than 1600 values
 }
 
 // rows_total / row_offset: the pass fills rows [row_offset, row_offset + N) of a (batch, rows_total, C') tensor

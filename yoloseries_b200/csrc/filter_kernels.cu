@@ -241,7 +241,7 @@ __device__ __forceinline__ void emit_keys(const uint64_t (&k)[VEC], unsigned okm
 // planes layout (NCHW heads: YOLOv5, YOLOX, YOLOv8, FCOS).  One thread = VEC consecutive positions of one
 // (image, anchor); per class plane a warp reads 32*VEC*4 contiguous bytes (512 B with 128-bit loads).
 // -------------------------------------------------------------------------------------------------------
-template <typename T, int VEC, int U = 8, int THREADS = 256, int MINB = 1, int HINT = 0, int PROBE = 0>
+template <typename T, int VEC, int U = 8, int THREADS = 256, int MINB = 1, int HINT = 0, int PROBE = 0, bool WIDE = false>
 __global__ void __launch_bounds__(THREADS, MINB) k_filter_planes(const __grid_constant__ Plan P, uint64_t *__restrict__ keys,
                                                                  int64_t key_cap, int32_t *__restrict__ counts)
 {
@@ -339,7 +339,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_filter_planes(const __grid_co
                 score, c, pre);
             npre += pre ? 1 : 0;
             if (ok) {
-                out[j] = pack_key(score, static_cast<uint32_t>(P.cand_base + cand0 + j), static_cast<uint32_t>(c));
+                out[j] = pack_key<WIDE>(score, static_cast<uint32_t>(P.cand_base + cand0 + j), static_cast<uint32_t>(c));
                 okm |= 1u << j;
                 const uint32_t sb = __float_as_uint(score);
                 smax_bits = max(smax_bits, sb);
@@ -362,7 +362,7 @@ __device__ __forceinline__ void prefetch_l2(const void *p) { asm volatile("prefe
 
 // PF > 0: while the loads of batch b are in flight, the lines of batch b + PF are requested into L2 with prefetch
 // instructions (no registers held): the demand loads of later batches then hit L2 instead of waiting a DRAM round trip.
-template <typename T, int U, int THREADS, int MINB, int PF = 0>
+template <typename T, int U, int THREADS, int MINB, int PF = 0, bool WIDE = false>
 __global__ void __launch_bounds__(THREADS, MINB) k_filter_planes_v4(const __grid_constant__ Plan P, uint64_t *__restrict__ keys,
                                                                     int64_t key_cap, int32_t *__restrict__ counts)
 {
@@ -455,7 +455,7 @@ __global__ void __launch_bounds__(THREADS, MINB) k_filter_planes_v4(const __grid
                 P, m1[j], m2[j], k0[j], objv[j], [&](int kk) { return ldg_head(cj + static_cast<size_t>(kk) * hw); }, score, c, pre);
             npre += pre ? 1 : 0;
             if (ok) {
-                out[j] = pack_key(score, static_cast<uint32_t>(P.cand_base + cand0 + j), static_cast<uint32_t>(c));
+                out[j] = pack_key<WIDE>(score, static_cast<uint32_t>(P.cand_base + cand0 + j), static_cast<uint32_t>(c));
                 okm |= 1u << j;
                 const uint32_t sb = __float_as_uint(score);
                 smax_bits = max(smax_bits, sb);
@@ -706,6 +706,138 @@ __global__ void __launch_bounds__(kRowsTile) k_filter_rows(const __grid_constant
                             (flags & 2) != 0, &ext_seen);
 }
 
+// -------------------------------------------------------------------------------------------------------
+// rows layout, rows wider than the 128-row shared tile (!rows_fit_tile: YOLOv7 rows of 5 + C from C = 449, RetinaNet /
+// RetinaNet-exp class rows from C = 454, decoded rows; up to 2048 classes, narrow or wide keys).
+// Same grid as k_filter_rows (one CTA per image and 128-row tile), no shared memory: warp w scans rows 32w .. 32w + 31 of
+// the tile one at a time, the whole warp on one row, straight from global memory in 16-byte loads (4 float32 / 8 16-bit
+// values; a row start that is not 16-byte aligned -- YOLOv7's 5 + C values -- is peeled into scalar head and tail loads).
+// Each lane keeps its own (max, runner-up, first index of max) over the columns it visits in ascending order; the lanes
+// merge by butterfly shuffle (merge_top2), and lane j keeps row 32w + j.  Then every lane decides its row with the tail
+// of rows_scan_emit (decide_candidate, whose literal path re-reads the row from global memory) and the warp appends.
+// -------------------------------------------------------------------------------------------------------
+constexpr int kWideRowsInFlight = 4;   // 16-byte loads in flight per lane
+
+__device__ __forceinline__ void ldg16(const float *p, float (&v)[4])
+{
+    const float4 t = ldg_stream4(p);
+    v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
+}
+template <typename T>
+__device__ __forceinline__ void ldg16(const T *p, float (&v)[8])
+{
+    uint4 r;
+    asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
+    const float4 a = widen4(make_uint2(r.x, r.y), p), b = widen4(make_uint2(r.z, r.w), p);
+    v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
+}
+
+// Merge another lane's (b1, b2, bk) into (m1, m2, k0), with the semantics of top2_update_t<T>: float32 -- equal maxima
+// leave runner-up == maximum (the literal path); 16-bit -- m2 is the largest value strictly below m1 and k0 the lowest
+// index of m1.  Symmetric, so every lane of a butterfly ends with the same triple.
+template <typename T>
+__device__ __forceinline__ void merge_top2(float &m1, float &m2, int &k0, float b1, float b2, int bk)
+{
+    if (sizeof(T) == 4) m2 = fmaxf(fmaxf(m2, b2), fminf(m1, b1));
+    else m2 = (b1 > m1) ? fmaxf(m1, b2) : ((b1 < m1) ? fmaxf(m2, b1) : fmaxf(m2, b2));
+    k0 = (b1 > m1 || (b1 == m1 && bk < k0)) ? bk : k0;
+    m1 = fmaxf(m1, b1);
+}
+
+template <typename T, bool WIDE>
+__global__ void __launch_bounds__(kRowsTile) k_filter_rows_wide(const __grid_constant__ Plan P, uint64_t *__restrict__ keys,
+                                                                int64_t key_cap, int32_t *__restrict__ counts)
+{
+    constexpr int E = 16 / static_cast<int>(sizeof(T));   // values per 16-byte load
+    const int img = blockIdx.x;
+    const int t = blockIdx.y;
+    int l = 0;
+#pragma unroll
+    for (int i = 1; i < YSB_MAX_LEVELS; ++i)
+        if (i < P.L && t >= P.lv[i].unit_off) l = i;
+    const LevelDesc &lv = P.lv[l];
+    const int rows_l = (l + 1 < P.L ? P.lv[l + 1].cand_off : P.N) - lv.cand_off;
+    const int r0 = (t - lv.unit_off) * kRowsTile;
+    const int nrows = min(kRowsTile, rows_l - r0);
+    const int rw = P.row_w_in, C = P.C;
+    const T *tile = head_ptr<T>(lv.p0) + (static_cast<size_t>(img) * lv.img_rows + r0) * rw;
+    const volatile unsigned int *ext_p = reinterpret_cast<const volatile unsigned int *>(counts + img * 4 + 2);
+    const uint2 ext_seen = make_uint2(ext_p[0], ext_p[1]);
+    const int lane = threadIdx.x & 31;
+    const int wr0 = (threadIdx.x >> 5) * 32;
+
+    float my1 = -INFINITY, my2 = -INFINITY;
+    int myk = 0;
+    for (int i = 0; i < 32 && wr0 + i < nrows; ++i) {   // warp-uniform
+        const T *cls = tile + static_cast<size_t>(wr0 + i) * rw + P.cls_col_in;
+        const int head = min(C, static_cast<int>(((16u - (reinterpret_cast<uintptr_t>(cls) & 15u)) & 15u) / sizeof(T)));
+        const int nv = (C - head) / E;
+        const int tail0 = head + nv * E;
+        float m1 = -INFINITY, m2 = -INFINITY;
+        int k0 = 0;
+        if (lane < head) top2_update_t<T>(ldg_stream1(cls + lane), lane, m1, m2, k0);
+        const T *body = cls + head;
+        for (int v0 = 0; v0 < nv; v0 += 32 * kWideRowsInFlight) {
+            float x[kWideRowsInFlight][E];
+#pragma unroll
+            for (int q = 0; q < kWideRowsInFlight; ++q) {
+                const int v = v0 + 32 * q + lane;
+                if (v < nv) {
+                    ldg16(body + static_cast<size_t>(v) * E, x[q]);
+                } else {
+#pragma unroll
+                    for (int j = 0; j < E; ++j) x[q][j] = -INFINITY;
+                }
+            }
+#pragma unroll
+            for (int q = 0; q < kWideRowsInFlight; ++q) {
+                const int k = head + (v0 + 32 * q + lane) * E;
+#pragma unroll
+                for (int j = 0; j < E; ++j) top2_update_t<T>(x[q][j], k + j, m1, m2, k0);
+            }
+        }
+        if (tail0 + lane < C) top2_update_t<T>(ldg_stream1(cls + tail0 + lane), tail0 + lane, m1, m2, k0);
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) {
+            const float b1 = __shfl_xor_sync(0xffffffffu, m1, d), b2 = __shfl_xor_sync(0xffffffffu, m2, d);
+            const int bk = __shfl_xor_sync(0xffffffffu, k0, d);
+            merge_top2<T>(m1, m2, k0, b1, b2, bk);
+        }
+        if (lane == i) { my1 = m1; my2 = m2; myk = k0; }
+    }
+
+    uint64_t out[1] = {0ull};
+    unsigned okm = 0u;
+    int npre = 0;
+    uint32_t smax_bits = 0u, smin_inv = 0u;
+    const int rj = wr0 + lane;
+    if (rj < nrows) {
+        const T *row = tile + static_cast<size_t>(rj) * rw;
+        const T *cls = row + P.cls_col_in;
+        const int cand = lv.cand_off + r0 + rj;
+        float objv = 0.0f;
+        if (P.use_obj)
+            objv = P.obj_src == 1 ? ldg_head(head_ptr<T>(P.lv[0].p1) + (static_cast<size_t>(img) * P.N + cand) * P.reg_row_w + 4)
+                                  : ldg_head(row + P.obj_col_in);
+        float score;
+        int c;
+        bool pre, ok;
+        if (P.input_kind == YSB_INPUT_DECODED_ROWS)
+            ok = decide_candidate<true>(P, my1, my2, myk, objv, [&](int kk) { return ldg_head(cls + kk); }, score, c, pre);
+        else
+            ok = decide_candidate<false>(P, my1, my2, myk, objv, [&](int kk) { return ldg_head(cls + kk); }, score, c, pre);
+        npre = pre ? 1 : 0;
+        if (ok) {
+            out[0] = pack_key<WIDE>(score, static_cast<uint32_t>(P.cand_base + cand), static_cast<uint32_t>(c));
+            okm = 1u;
+            smax_bits = __float_as_uint(score);
+            smin_inv = ~smax_bits;
+        }
+    }
+    emit_keys<1>(out, okm, npre, smax_bits, smin_inv, keys + static_cast<int64_t>(img) * key_cap, key_cap, counts + img * 4,
+                 P.pre_kind == PRE_ANY_GT, &ext_seen);
+}
+
 #ifdef YSB_PROFILING_VARIANTS
 // -------------------------------------------------------------------------------------------------------
 // rows layout, persistent ring version (profiling build, YSB_ROWS_RING=1; measured SLOWER than k_filter_rows: 8 scanning
@@ -813,7 +945,7 @@ __global__ void __launch_bounds__(kRowsTile) k_filter_rows_ring(const __grid_con
 // eval_fcos.py:246-250).  False in every shipped yaml, so this kernel favours simplicity: one thread per candidate,
 // every class evaluated literally (sigmoid, multiply) twice -- once to count, once to write -- any input layout.
 // -------------------------------------------------------------------------------------------------------
-template <typename T, bool NHWC>
+template <typename T, bool NHWC, bool WIDE = false>
 __global__ void __launch_bounds__(256) k_filter_multilabel(const __grid_constant__ Plan P, uint64_t *__restrict__ keys,
                                                            int64_t key_cap, int32_t *__restrict__ counts)
 {
@@ -906,7 +1038,7 @@ __global__ void __launch_bounds__(256) k_filter_multilabel(const __grid_constant
             float sk;
             const float p = score_of(k, sk);
             if (passes(p)) {
-                if (at < key_cap) dst[at] = pack_key(p, static_cast<uint32_t>(P.cand_base + cand), static_cast<uint32_t>(k));
+                if (at < key_cap) dst[at] = pack_key<WIDE>(p, static_cast<uint32_t>(P.cand_base + cand), static_cast<uint32_t>(k));
                 ++at;
             }
         }
@@ -920,16 +1052,63 @@ __global__ void __launch_bounds__(256) k_filter_multilabel(const __grid_constant
 #include "filter_variants_launch.inc"
 #endif
 
+// planes layout (NCHW heads).  WIDE: the sort-key layout of plans with more than 1024 classes
+template <typename T, bool WIDE>
+static cudaError_t launch_planes(const Plan &P, int vec, uint64_t *d_keys, int64_t key_cap, int32_t *d_counts,
+                                 cudaStream_t stream)
+{
+    cudaError_t e = cudaSuccess;
+    // image-fastest grids: CTAs that run at the same time append to different images' counters
+    if (vec == 4) {
+        // every level 128-bit loadable (the common case): 9 loads of 128 bits in flight per thread (YOLOv5 / YOLOX:
+        // 80 classes + objectness = 9 batches of 9), 76 registers, 6 CTAs of 128 threads per SM
+        const dim3 gv4(P.batch, (P.units_per_img + 127) / 128);
+#ifdef YSB_PROFILING_VARIANTS
+        if (sizeof(T) == 4) {   // profiling build: YSB_K1_CARVEOUT=<percent of the SM's shared memory> as the kernel's preferred carve-out
+            static int pct = -2;
+            if (pct == -2) { const char *ev = getenv("YSB_K1_CARVEOUT"); pct = ev ? atoi(ev) : -1; }
+            if (pct >= 0) {
+                e = cudaFuncSetAttribute(k_filter_planes_v4<T, 9, 128, 6, 0, WIDE>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
+                if (e != cudaSuccess) return e;
+            }
+        }
+#endif
+        k_filter_planes_v4<T, 9, 128, 6, 0, WIDE><<<gv4, 128, 0, stream>>>(P, d_keys, key_cap, d_counts);
+    } else if (vec == 1) {
+        const dim3 grid(P.batch, (P.units_per_img + 255) / 256);
+        k_filter_planes<T, 1, 8, 256, 1, 0, 0, WIDE><<<grid, 256, 0, stream>>>(P, d_keys, key_cap, d_counts);
+    } else {
+        // levels that are not all 128-bit loadable (FCOS' 5x5 map): generic kernel, 128-thread CTAs, 12 loads of
+        // 128 bits in flight per thread (96 registers, 5 CTAs/SM), 256-byte L2 prefetch
+        const dim3 grid128(P.batch, (P.units_per_img + 127) / 128);
+        k_filter_planes<T, 4, 12, 128, 5, 1, 0, WIDE><<<grid128, 128, 0, stream>>>(P, d_keys, key_cap, d_counts);
+    }
+    return e;
+}
+
 template <typename T>
 static cudaError_t launch_filter_t(const Plan &P, int vec, uint64_t *d_keys, int64_t key_cap, int32_t *d_counts,
                                    cudaStream_t stream)
 {
     cudaError_t e = cudaSuccess;
+    const bool wide = wide_keys(P.C);
     if (P.multi_label) {
         const dim3 grid(P.batch, (P.N + 255) / 256);
         if (P.layout == LAYOUT_ROWS_NHWC) k_filter_multilabel<T, true><<<grid, 256, 0, stream>>>(P, d_keys, key_cap, d_counts);
+        else if (wide) k_filter_multilabel<T, false, true><<<grid, 256, 0, stream>>>(P, d_keys, key_cap, d_counts);
         else k_filter_multilabel<T, false><<<grid, 256, 0, stream>>>(P, d_keys, key_cap, d_counts);
         return cudaGetLastError();
+    }
+    if (P.layout != LAYOUT_PLANES && !rows_fit_tile(P.row_w_in)) {
+        // rows wider than the shared tile (never channels-last: the ABI refuses those)
+        const dim3 grid(P.batch, P.units_per_img);
+        if (wide) k_filter_rows_wide<T, true><<<grid, kRowsTile, 0, stream>>>(P, d_keys, key_cap, d_counts);
+        else k_filter_rows_wide<T, false><<<grid, kRowsTile, 0, stream>>>(P, d_keys, key_cap, d_counts);
+        return cudaGetLastError();
+    }
+    if (P.layout == LAYOUT_PLANES && wide) {   // (the profiling variants pack narrow keys)
+        e = launch_planes<T, true>(P, vec, d_keys, key_cap, d_counts, stream);
+        return e != cudaSuccess ? e : cudaGetLastError();
     }
 #ifdef YSB_PROFILING_VARIANTS
     if (sizeof(T) == 4 && P.layout != LAYOUT_ROWS_NHWC) {   // the variants read float32 NCHW heads; 16-bit and NHWC heads run the product kernels
@@ -939,31 +1118,8 @@ static cudaError_t launch_filter_t(const Plan &P, int vec, uint64_t *d_keys, int
     }
 #endif
     if (P.layout == LAYOUT_PLANES) {
-        // image-fastest grids: CTAs that run at the same time append to different images' counters
-        if (vec == 4) {
-            // every level 128-bit loadable (the common case): 9 loads of 128 bits in flight per thread (YOLOv5 / YOLOX:
-            // 80 classes + objectness = 9 batches of 9), 76 registers, 6 CTAs of 128 threads per SM
-            const dim3 gv4(P.batch, (P.units_per_img + 127) / 128);
-#ifdef YSB_PROFILING_VARIANTS
-            if (sizeof(T) == 4) {   // profiling build: YSB_K1_CARVEOUT=<percent of the SM's shared memory> as the kernel's preferred carve-out
-                static int pct = -2;
-                if (pct == -2) { const char *ev = getenv("YSB_K1_CARVEOUT"); pct = ev ? atoi(ev) : -1; }
-                if (pct >= 0) {
-                    e = cudaFuncSetAttribute(k_filter_planes_v4<T, 9, 128, 6>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-                    if (e != cudaSuccess) return e;
-                }
-            }
-#endif
-            k_filter_planes_v4<T, 9, 128, 6><<<gv4, 128, 0, stream>>>(P, d_keys, key_cap, d_counts);
-        } else if (vec == 1) {
-            const dim3 grid(P.batch, (P.units_per_img + 255) / 256);
-            k_filter_planes<T, 1><<<grid, 256, 0, stream>>>(P, d_keys, key_cap, d_counts);
-        } else {
-            // levels that are not all 128-bit loadable (FCOS' 5x5 map): generic kernel, 128-thread CTAs, 12 loads of
-            // 128 bits in flight per thread (96 registers, 5 CTAs/SM), 256-byte L2 prefetch
-            const dim3 grid128(P.batch, (P.units_per_img + 127) / 128);
-            k_filter_planes<T, 4, 12, 128, 5, 1><<<grid128, 128, 0, stream>>>(P, d_keys, key_cap, d_counts);
-        }
+        e = launch_planes<T, false>(P, vec, d_keys, key_cap, d_counts, stream);
+        if (e != cudaSuccess) return e;
     } else {
         const size_t smem = static_cast<size_t>(kRowsTile) * (P.row_w_in | 1) * sizeof(T);
 #ifdef YSB_PROFILING_VARIANTS

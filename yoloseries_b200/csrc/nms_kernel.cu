@@ -398,7 +398,7 @@ __device__ __forceinline__ const Plan &pass_of(const Plan &P, const ExtraPasses 
 // scattered loads; one thread per (candidate, side) keeps its 16 bin loads in flight together and runs the softmax
 // expectation in registers (the decode kernel's bin order), the four sides of a candidate meet by shuffle -- THREADS/4
 // boxes per DRAM round trip.  Every other layout: one thread per box.
-template <bool ARRAY, typename EXTRA, int THREADS, int KEEP, typename T, bool NHWC>
+template <bool ARRAY, typename EXTRA, int THREADS, int KEEP, typename T, bool NHWC, bool WIDE>
 __device__ __forceinline__ void decode_boxes(NmsSmem<KEEP> &S, const Plan &P, const EXTRA &X, const ArrayArgs &aa, int img,
                                              int from, int upto, int &lo_x, int &hi_x, bool &bad)
 {
@@ -414,7 +414,7 @@ __device__ __forceinline__ void decode_boxes(NmsSmem<KEEP> &S, const Plan &P, co
             float sv = 0.0f;
             const bool ok = i < upto;
             if (ok) {
-                int cand = static_cast<int>(key_cand(S.keys[i]));
+                int cand = static_cast<int>(key_cand<WIDE>(S.keys[i]));
                 const Plan &Q = pass_of(P, X, cand);
                 sv = v8_side_value<T, NHWC>(Q, img, cand, side);
             }
@@ -422,7 +422,7 @@ __device__ __forceinline__ void decode_boxes(NmsSmem<KEEP> &S, const Plan &P, co
             const float s0 = __shfl_sync(0xffffffffu, sv, qb), s1 = __shfl_sync(0xffffffffu, sv, qb + 1);
             const float s2 = __shfl_sync(0xffffffffu, sv, qb + 2), s3 = __shfl_sync(0xffffffffu, sv, qb + 3);
             if (ok && side == 0) {
-                int c2 = static_cast<int>(key_cand(S.keys[i]));
+                int c2 = static_cast<int>(key_cand<WIDE>(S.keys[i]));
                 const Plan &Q = pass_of(P, X, c2);
                 const float4 b = tta_undo(Q, v8_box_from_sides(Q, c2, s0, s1, s2, s3));
                 S.raw[i] = b;
@@ -431,7 +431,7 @@ __device__ __forceinline__ void decode_boxes(NmsSmem<KEEP> &S, const Plan &P, co
         }
     } else {
         for (int i = from + tid; i < upto; i += THREADS) {
-            int cand = static_cast<int>(key_cand(S.keys[i]));
+            int cand = static_cast<int>(key_cand<WIDE>(S.keys[i]));
             if (ARRAY) {
                 S.raw[i] = __ldg(aa.boxes + cand);
             } else {
@@ -446,7 +446,8 @@ __device__ __forceinline__ void decode_boxes(NmsSmem<KEEP> &S, const Plan &P, co
 
 // EXTRA = NoExtraPasses (one set of heads) or ExtraPasses (TTA: boxes are decoded from the pass a candidate came from;
 // thresholds / NMS settings are those of P, identical in every pass).
-template <bool ARRAY, typename EXTRA, int THREADS, int KEEP, typename T = float, bool NHWC = false>
+// WIDE: the sort-key layout of plans with more than 1024 classes (ysb_internal.cuh, KeyLayout)
+template <bool ARRAY, typename EXTRA, int THREADS, int KEEP, typename T = float, bool NHWC = false, bool WIDE = false>
 __global__ void __launch_bounds__(THREADS, 1024 / THREADS)
 k_select_nms(const __grid_constant__ Plan P, const __grid_constant__ EXTRA X, const uint64_t *__restrict__ keys_all,
              int64_t key_cap, const int32_t *__restrict__ counts, float *__restrict__ dets,
@@ -547,7 +548,7 @@ k_select_nms(const __grid_constant__ Plan P, const __grid_constant__ EXTRA X, co
                 const int upto = min(n_use, decoded_upto + (dfl ? max(THREADS / 4, kChunk) : THREADS));
                 int d_lo = 0x7fffffff, d_hi = static_cast<int>(0x80000000u);
                 bool d_bad = false;
-                decode_boxes<ARRAY, EXTRA, THREADS, KEEP, T, NHWC>(S, P, X, aa, img, decoded_upto, upto, d_lo, d_hi, d_bad);
+                decode_boxes<ARRAY, EXTRA, THREADS, KEEP, T, NHWC, WIDE>(S, P, X, aa, img, decoded_upto, upto, d_lo, d_hi, d_bad);
                 decoded_upto = upto;
                 if (!ARRAY) {
                     d_lo = __reduce_min_sync(0xffffffffu, d_lo);
@@ -580,10 +581,10 @@ k_select_nms(const __grid_constant__ Plan P, const __grid_constant__ EXTRA X, co
                 if (valid) {
                     const uint64_t key = S.keys[c0 + j];
                     score = key_score(key);
-                    const float off = P.class_aware ? __fmul_rn(static_cast<float>(key_cls(key)), 4096.0f) : 0.0f;
+                    const float off = P.class_aware ? __fmul_rn(static_cast<float>(key_cls<WIDE>(key)), 4096.0f) : 0.0f;
                     ob = make_offbox(S.raw[c0 + j], off);
                     if (cls_fast) {
-                        const uint32_t *km = S.kept_mask[key_cls(key) & (kMaskBuckets<KEEP> - 1)];
+                        const uint32_t *km = S.kept_mask[key_cls<WIDE>(key) & (kMaskBuckets<KEEP> - 1)];
                         const int nw = (kept + 31) >> 5;
                         for (int wd = sub; wd < nw; wd += TPC) {
                             uint32_t m = km[wd];
@@ -593,7 +594,7 @@ k_select_nms(const __grid_constant__ Plan P, const __grid_constant__ EXTRA X, co
                                 sup |= pair_hit<ARRAY>(kept_box, i, ob, thr, aa);
                             }
                         }
-                        if (sub == 0) atomicOr(&S.chunk_mask[key_cls(key) & (kMaskBuckets<KEEP> - 1)][j >> 5], 1u << (j & 31));
+                        if (sub == 0) atomicOr(&S.chunk_mask[key_cls<WIDE>(key) & (kMaskBuckets<KEEP> - 1)][j >> 5], 1u << (j & 31));
                     } else {
                         sup = any_hit_strided<ARRAY>(kept_box, sub, TPC, kept, ob, thr, aa);
                     }
@@ -616,7 +617,7 @@ k_select_nms(const __grid_constant__ Plan P, const __grid_constant__ EXTRA X, co
                 if (cls_fast) {
                     if (j < cn && S.chunk_alive[j]) {
                         const OffBox bj = soa_load(chunk_box, j);
-                        const uint32_t *cm = S.chunk_mask[key_cls(S.keys[c0 + j]) & (kMaskBuckets<KEEP> - 1)];
+                        const uint32_t *cm = S.chunk_mask[key_cls<WIDE>(S.keys[c0 + j]) & (kMaskBuckets<KEEP> - 1)];
                         for (int wd = sub; wd <= (j >> 5); wd += TPC) {
                             uint32_t m = cm[wd];
                             if (wd == (j >> 5)) m &= (1u << (j & 31)) - 1u;   // earlier candidates only
@@ -745,16 +746,16 @@ k_select_nms(const __grid_constant__ Plan P, const __grid_constant__ EXTRA X, co
                     if (((mine >> (tid & 31)) & 1u) && at < max_det) {
                         soa_store(kept_box, at, soa_load(chunk_box, tid));
                         if (ARRAY) {
-                            aa.keep[at] = static_cast<int32_t>(key_cand(S.keys[c0 + tid]));
+                            aa.keep[at] = static_cast<int32_t>(key_cand<WIDE>(S.keys[c0 + tid]));
                         } else {
                             S.kept_key[at] = S.keys[c0 + tid];
                             S.kept_raw[at] = S.raw[c0 + tid];
                             // (maintained even while the walk tests all pairs: cheap, and the span can only grow)
-                            atomicOr(&S.kept_mask[key_cls(S.keys[c0 + tid]) & (kMaskBuckets<KEEP> - 1)][at >> 5], 1u << (at & 31));
+                            atomicOr(&S.kept_mask[key_cls<WIDE>(S.keys[c0 + tid]) & (kMaskBuckets<KEEP> - 1)][at >> 5], 1u << (at & 31));
                         }
                     }
                     // the chunk's class-bucket mask is all zero again for the next chunk
-                    if (!ARRAY && cls_fast && tid < cn) S.chunk_mask[key_cls(S.keys[c0 + tid]) & (kMaskBuckets<KEEP> - 1)][tid >> 5] = 0u;
+                    if (!ARRAY && cls_fast && tid < cn) S.chunk_mask[key_cls<WIDE>(S.keys[c0 + tid]) & (kMaskBuckets<KEEP> - 1)][tid >> 5] = 0u;
                 }
             }
             kept += added;
@@ -807,23 +808,26 @@ k_select_nms(const __grid_constant__ Plan P, const __grid_constant__ EXTRA X, co
             if (!resident) {
                 for (int i = tid; i < mm; i += THREADS) S.keys[i] = __ldg(keys + b0 + i);
                 __syncthreads();
-                decode_boxes<false, EXTRA, THREADS, KEEP, T, NHWC>(S, P, X, aa, img, 0, mm, pf_lo, pf_hi, pf_bad);
+                decode_boxes<false, EXTRA, THREADS, KEEP, T, NHWC, WIDE>(S, P, X, aa, img, 0, mm, pf_lo, pf_hi, pf_bad);
             } else if (decoded_upto < mm) {
-                decode_boxes<false, EXTRA, THREADS, KEEP, T, NHWC>(S, P, X, aa, img, decoded_upto, mm, pf_lo, pf_hi, pf_bad);
+                decode_boxes<false, EXTRA, THREADS, KEEP, T, NHWC, WIDE>(S, P, X, aa, img, decoded_upto, mm, pf_lo, pf_hi, pf_bad);
             }
             __syncthreads();
             if (!P.merge_boxes) {
                 // offset boxes + areas once per survivor (in place).  The 4096-px class offset keeps boxes of different
-                // classes disjoint in x as long as the raw boxes span at most 4095 px: for classes a < b,
-                // fl(x2 + 4096 a) - fl(x1' + 4096 b) <= (max x2 - min x1) - 4096 + 0.5 < 0 (offset values stay below 2^23,
-                // so each rounding moves them by at most 0.25).  Then a kept box only needs the survivors of its own
-                // class: bucket the block by class (counting sort of indices in shared memory) and walk one bucket per
-                // kept box.  Otherwise (huge boxes -- the reference then lets classes interact) every pair is tested.
+                // classes disjoint in x as long as the raw boxes span at most 4095 px: for classes a < b the exact values
+                // satisfy x2 + 4096 a < x1' + 4096 b (x2 - x1' <= span < 4096; 4096 cls is exact for every class id), and
+                // rounding is monotone, so fl(x2 + 4096 a) <= fl(x1' + 4096 b): the x overlap is <= 0 and the pair cannot
+                // reach a positive threshold.  This needs no bound on the offset values, so it holds where they pass 2^23
+                // (class 2047 plus a box coordinate) and the float32 spacing grows to 1.  Then a kept box only needs the
+                // survivors of its own class: bucket the block by class (counting sort of indices in shared memory, up to
+                // kBins / 2 = 1024 classes; wider plans test every pair) and walk one bucket per kept box.  Otherwise
+                // (huge boxes -- the reference then lets classes interact) every pair is tested.
                 int lo_x = k_lo, hi_x = k_hi;
                 bool finite = k_fin;
                 for (int jj = tid; jj < mm; jj += THREADS) {
                     const uint64_t key = S.keys[jj];
-                    const float off = P.class_aware ? __fmul_rn(static_cast<float>(key_cls(key)), 4096.0f) : 0.0f;
+                    const float off = P.class_aware ? __fmul_rn(static_cast<float>(key_cls<WIDE>(key)), 4096.0f) : 0.0f;
                     const float4 rb = S.raw[jj];
                     finite = finite && (fabsf(rb.x) <= 3.0e38f) && (fabsf(rb.z) <= 3.0e38f);  // false for NaN / inf
                     lo_x = min(lo_x, float_ordered(rb.x));
@@ -845,7 +849,7 @@ k_select_nms(const __grid_constant__ Plan P, const __grid_constant__ EXTRA X, co
                     uint32_t *cursor = S.hist + kBins / 2;
                     for (int c = tid; c < kBins / 2; c += THREADS) cnt_cls[c] = 0;
                     __syncthreads();
-                    for (int jj = tid; jj < mm; jj += THREADS) atomicAdd(&cnt_cls[key_cls(S.keys[jj])], 1u);
+                    for (int jj = tid; jj < mm; jj += THREADS) atomicAdd(&cnt_cls[key_cls<WIDE>(S.keys[jj])], 1u);
                     __syncthreads();
                     // exclusive scan over the classes: PERC consecutive classes per thread
                     constexpr int PERC = (kBins / 2) / THREADS;
@@ -880,13 +884,13 @@ k_select_nms(const __grid_constant__ Plan P, const __grid_constant__ EXTRA X, co
                     }
                     __syncthreads();
                     for (int jj = tid; jj < mm; jj += THREADS) {
-                        const uint32_t at = atomicAdd(&cursor[key_cls(S.keys[jj])], 1u);
+                        const uint32_t at = atomicAdd(&cursor[key_cls<WIDE>(S.keys[jj])], 1u);
                         S.order[at] = static_cast<uint16_t>(jj);
                     }
                     __syncthreads();
                     for (int r = warp; r < kept; r += THREADS / 32) {
                         const OffBox br = soa_load(kept_box, r);
-                        const uint32_t cls_r = key_cls(S.kept_key[r]);
+                        const uint32_t cls_r = key_cls<WIDE>(S.kept_key[r]);
                         const int lo = static_cast<int>(cnt_cls[cls_r]), hi = static_cast<int>(cursor[cls_r]);
                         int c = 0;
                         for (int q = lo + lane; q < hi; q += 32) {
@@ -922,7 +926,7 @@ k_select_nms(const __grid_constant__ Plan P, const __grid_constant__ EXTRA X, co
                     float ax = 0.f, ay = 0.f, az = 0.f, aw = 0.f, ws = 0.f;
                     for (int jj = lane; jj < mm; jj += 32) {
                         const uint64_t key = S.keys[jj];
-                        const float off = P.class_aware ? __fmul_rn(static_cast<float>(key_cls(key)), 4096.0f) : 0.0f;
+                        const float off = P.class_aware ? __fmul_rn(static_cast<float>(key_cls<WIDE>(key)), 4096.0f) : 0.0f;
                         const float4 rj = S.raw[jj];
                         if (iou_reaches<true>(br, make_offbox(rj, off), thr)) {
                             ++c;
@@ -1013,7 +1017,7 @@ k_select_nms(const __grid_constant__ Plan P, const __grid_constant__ EXTRA X, co
             const int at = before + __popc(bal & ((1u << (tid & 31)) - 1u));
             const float sc = key_score(key);
             const float s_out = P.topk_sqrt ? sqrtf(sc) : sc;  // FCOS: x[:, 4] = sqrt(x[:, 4]) (trainer/eval_fcos.py:281)
-            const float c_out = static_cast<float>(key_cls(key));
+            const float c_out = static_cast<float>(key_cls<WIDE>(key));
             if (lb) {
                 box.x = fminf(fmaxf(__fdiv_rn(__fsub_rn(box.x, lb_left), lb_scale), 1.0f), lb_hi_x);
                 box.z = fminf(fmaxf(__fdiv_rn(__fsub_rn(box.z, lb_left), lb_scale), 1.0f), lb_hi_x);
@@ -1024,7 +1028,7 @@ k_select_nms(const __grid_constant__ Plan P, const __grid_constant__ EXTRA X, co
             row[0] = box.x; row[1] = box.y; row[2] = box.z; row[3] = box.w;
             row[4] = s_out;
             row[5] = c_out;
-            if (det_idx) det_idx[static_cast<size_t>(img) * max_det + at] = static_cast<int32_t>(key_cand(key));
+            if (det_idx) det_idx[static_cast<size_t>(img) * max_det + at] = static_cast<int32_t>(key_cand<WIDE>(key));
         }
         written = total;
     }
@@ -1092,13 +1096,13 @@ static int device_sm_count()
     return n;
 }
 
-template <typename EXTRA, int THREADS, int KEEP, typename T, bool NHWC>
+template <typename EXTRA, int THREADS, int KEEP, typename T, bool NHWC, bool WIDE>
 static cudaError_t launch_flavour(const Plan &P, const EXTRA &X, const uint64_t *d_keys, int64_t key_cap, const int32_t *d_counts,
                                   float *d_dets, int32_t *d_det_idx, int32_t *d_det_cnt, cudaStream_t stream, const GatherSink &G)
 {
     // per-device attribute; set on every launch (host-side, sub-microsecond) so that a process driving several
     // devices never launches with the default 48 KB limit
-    auto kern = k_select_nms<false, EXTRA, THREADS, KEEP, T, NHWC>;
+    auto kern = k_select_nms<false, EXTRA, THREADS, KEEP, T, NHWC, WIDE>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(sizeof(NmsSmem<KEEP>)));
     if (e != cudaSuccess) return e;
     ArrayArgs aa{};
@@ -1118,7 +1122,7 @@ static cudaError_t launch_flavour(const Plan &P, const EXTRA &X, const uint64_t 
     return cudaGetLastError();
 }
 
-template <typename EXTRA, typename T, bool NHWC>
+template <typename EXTRA, typename T, bool NHWC, bool WIDE>
 static cudaError_t launch_any(const Plan &P, const EXTRA &X, const uint64_t *d_keys, int64_t key_cap, const int32_t *d_counts,
                               float *d_dets, int32_t *d_det_idx, int32_t *d_det_cnt, cudaStream_t stream, const GatherSink *sink)
 {
@@ -1140,32 +1144,34 @@ static cudaError_t launch_any(const Plan &P, const EXTRA &X, const uint64_t *d_k
 #endif
     if (g_force_threads == 512 && small_keep) threads = 512;
     if (g_force_threads == 1024) threads = 1024;
-    if (!small_keep) return launch_flavour<EXTRA, 1024, 1024, T, NHWC>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, G);
-    if (threads == 512) return launch_flavour<EXTRA, 512, 320, T, NHWC>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, G);
-    return launch_flavour<EXTRA, 1024, 320, T, NHWC>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, G);
+    if (!small_keep) return launch_flavour<EXTRA, 1024, 1024, T, NHWC, WIDE>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, G);
+    if (threads == 512) return launch_flavour<EXTRA, 512, 320, T, NHWC, WIDE>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, G);
+    return launch_flavour<EXTRA, 1024, 320, T, NHWC, WIDE>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, G);
 }
 
-template <typename EXTRA, bool NHWC>
+template <typename EXTRA, bool NHWC, bool WIDE>
 static cudaError_t launch_any_dt(const Plan &P, const EXTRA &X, const uint64_t *d_keys, int64_t key_cap, const int32_t *d_counts,
                                  float *d_dets, int32_t *d_det_idx, int32_t *d_det_cnt, cudaStream_t stream,
                                  const GatherSink *sink, int dtype)
 {
     switch (dtype) {
-    case YSB_F16: return launch_any<EXTRA, __half, NHWC>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink);
+    case YSB_F16: return launch_any<EXTRA, __half, NHWC, WIDE>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink);
     case YSB_BF16:
-        return launch_any<EXTRA, __nv_bfloat16, NHWC>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink);
-    default: return launch_any<EXTRA, float, NHWC>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink);
+        return launch_any<EXTRA, __nv_bfloat16, NHWC, WIDE>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink);
+    default: return launch_any<EXTRA, float, NHWC, WIDE>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink);
     }
 }
 
-// NHWC heads (LAYOUT_ROWS_NHWC, YSB_INPUT_RAW_HEADS_NHWC): the kernel's box decode addresses channels-last memory
+// NHWC heads (LAYOUT_ROWS_NHWC, YSB_INPUT_RAW_HEADS_NHWC): the kernel's box decode addresses channels-last memory.
+// More than 1024 classes: wide sort keys (never with NHWC heads, whose rows that wide the ABI refuses).
 template <typename EXTRA>
 static cudaError_t launch_any_layout(const Plan &P, const EXTRA &X, const uint64_t *d_keys, int64_t key_cap,
                                      const int32_t *d_counts, float *d_dets, int32_t *d_det_idx, int32_t *d_det_cnt,
                                      cudaStream_t stream, const GatherSink *sink, int dtype)
 {
-    if (P.layout == LAYOUT_ROWS_NHWC) return launch_any_dt<EXTRA, true>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink, dtype);
-    return launch_any_dt<EXTRA, false>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink, dtype);
+    if (P.layout == LAYOUT_ROWS_NHWC) return launch_any_dt<EXTRA, true, false>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink, dtype);
+    if (wide_keys(P.C)) return launch_any_dt<EXTRA, false, true>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink, dtype);
+    return launch_any_dt<EXTRA, false, false>(P, X, d_keys, key_cap, d_counts, d_dets, d_det_idx, d_det_cnt, stream, sink, dtype);
 }
 
 cudaError_t launch_select_nms(const Plan &P, const uint64_t *d_keys, int64_t key_cap, const int32_t *d_counts,

@@ -289,6 +289,8 @@ def validate_heads(family, flat, num_class, anchors=None, dfl_bins=16, decoded_r
         raise ValueError(f"{family} heads: {msg}")
     if not flat:
         bad("no tensors")
+    if not 1 <= C <= _lib.YSB_MAX_CLASSES:
+        bad(f"num_class {C} is outside 1..{_lib.YSB_MAX_CLASSES} (YSB_MAX_CLASSES)")
     b = flat[0].shape[0]
     for i, t in enumerate(flat):
         if t.dtype not in HEAD_DTYPES or (decoded_row_w is not None and not t.is_contiguous()):
