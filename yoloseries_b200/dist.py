@@ -225,6 +225,16 @@ class ShardedPostProcessor:
     Contiguous (NCHW) and channels-last heads (YOLOv5, YOLOX, YOLOv8, FCOS; include/ysb_postproc.h) are both read as they
     are; like the dtype, the first submission fixes the layout and a later batch in the other one raises ValueError.
 
+    Rows in original-picture pixels (the box half of preds_postprocess, val_yolov5.py:166-172): every rank passes the
+    letterbox dicts of its own images, as for PostProcessor.run(info=...).  The NMS kernel maps the rows before it stores
+    them into every rank's slot, so each rank receives mapped rows of all world*batch images without exchanging the dicts:
+
+        t = spp.submit(heads, info=info)       # info: this rank's batch dicts (scale, pad_top, pad_left, org_shape)
+        rows, cnt = spp.gathered(t)            # every rank's rows in its own original-picture pixels
+        t = spp.submit_tta(passes, info=info)  # TTA undo first, then the letterbox undo, as in run_tta(info=...)
+
+    ``info`` is decided per submission (None: network-input pixels); one dict per image, otherwise ValueError.
+
     Lanes, graphs and the gather work as for ``submit``.  The first submission fixes the kind (plain or TTA): a processor
     takes only ``submit`` or only ``submit_tta`` calls.  For TTA it also fixes the number of passes, each pass's
     (img_h, img_w, scale, flip_axis) and the head shapes, and sizes the key buffers to the passes' summed key slots; a
@@ -287,8 +297,6 @@ class ShardedPostProcessor:
         """TTA set-up of the first submit_tta: params of every pass, key buffers sized to the summed key slots."""
         n = len(ents)
         params = (_lib.YsbParams * n)(*[e["params"] for _, e in ents])
-        for i in range(n):
-            params[i].d_letterbox = None   # rows stay in network-input pixels, as with submit
         self._tta = dict(geom=geom, ents=[e for _, e in ents], params=params,
                          per_pass=(ctypes.c_int32 * n)(*[len(flat) for flat, _ in ents]))
         self._head_dtype = ents[0][0][0].dtype
@@ -297,6 +305,7 @@ class ShardedPostProcessor:
 
     def _alloc_lanes(self, n):
         """Key / count / output buffers of every lane; ``n`` key slots per image."""
+        from .engine import LetterboxStaging
         self._key_cap = n
         b, d, dev = self.batch, self.max_det, self.device
         self._slots = []
@@ -312,6 +321,7 @@ class ShardedPostProcessor:
                 sl = {"keys": torch.empty((b, n), dtype=torch.int64, device=dev),
                       "counts": torch.zeros((b, 4), dtype=torch.int32, device=dev),
                       "idx": torch.empty((b, d), dtype=torch.int32, device=dev),
+                      "lb": LetterboxStaging(b, dev),
                       "done": torch.cuda.Event()}
                 if self.mode == "p2p":
                     sl["rows"], sl["cnt"] = self.dg.views(s)
@@ -325,16 +335,22 @@ class ShardedPostProcessor:
                     sl["cnt"] = torch.zeros((1, b), dtype=torch.int32, device=dev)
             self._slots.append(sl)
 
-    def _enqueue(self, ptrs, nheads, lane, st, events=None):
-        """The launch sequence of one batch on stream ``st`` (plain C-ABI calls: capturable into a CUDA graph)."""
+    def _enqueue(self, ptrs, nheads, lane, st, events=None, lb=None):
+        """The launch sequence of one batch on stream ``st`` (plain C-ABI calls and a copy: capturable into a CUDA
+        graph).  ``lb``: address of the lane's letterbox table, whose staged rows the sequence copies in first, or None
+        for rows in network-input pixels."""
         lib, sl = self.lib, self._slots[lane]
         sp = ctypes.c_void_p(st.cuda_stream)
-        # the plain and the TTA entry points take the same arguments after the heads
+        # the plain and the TTA entry points take the same arguments after the heads; the params are shared by the lanes,
+        # and every call copies them, so the lane's table pointer is set right before the calls
         if self._kind == "tta":
             tta, sfx = self._tta, "_tta"
+            for p in tta["params"]:
+                p.d_letterbox = lb
             head = (tta["params"], len(tta["params"]), ptrs, tta["per_pass"])
         else:
             sfx = ""
+            self._ent["params"].d_letterbox = lb
             head = (ctypes.byref(self._ent["params"]), ptrs, nheads)
         filt, nms = getattr(lib, "ysb_filter_candidates" + sfx), getattr(lib, "ysb_select_nms" + sfx)
         nms_gather = getattr(lib, "ysb_select_nms" + sfx + "_gather")
@@ -343,6 +359,9 @@ class ShardedPostProcessor:
             # right before storing into it, a filter + NMS pass from now)
             g = ctypes.byref(self.dg.g)
             _lib.check(lib.ysb_gather_begin(g, lane, None, 0, sp), "ysb_gather_begin")
+        if lb is not None:
+            with torch.cuda.stream(st):
+                sl["lb"].enqueue_copy()
         if events:
             events[0].record(st)
         _lib.check(filt(*head, sl["keys"].data_ptr(), self._key_cap, sl["counts"].data_ptr(), sp),
@@ -366,33 +385,38 @@ class ShardedPostProcessor:
                 events[2].record(st)
 
     # ---- public ----------------------------------------------------------------------------------------------------
-    def submit(self, heads, events=None, sync_input=True):
+    def submit(self, heads, events=None, sync_input=True, info=None):
         """Enqueue one batch.  ``events``: optional 3 timing events (start, filter done, NMS done) recorded on the lane's
-        stream.  ``sync_input=False`` skips the wait on the caller's current stream (heads known to be ready)."""
-        from .engine import flatten_heads, head_layout
+        stream.  ``sync_input=False`` skips the wait on the caller's current stream (heads known to be ready).  ``info``:
+        this rank's letterbox dicts (scale, pad_top, pad_left, org_shape), one per image as for PostProcessor.run: its
+        rows are then stored in original-picture pixels, into every rank's slot; None keeps network-input pixels."""
+        from .engine import flatten_heads, head_layout, letterbox_rows
         if self._kind == "tta":
             raise ValueError("this processor was set up for test-time-augmented batches: use submit_tta")
         flat = flatten_heads(self.family, heads)
         if flat[0].shape[0] != self.batch:
             raise ValueError(f"expected {self.batch} images per rank, got {flat[0].shape[0]}")
+        rows = None if info is None else letterbox_rows(info, self.batch)
         self._prepare(flat)
         self._kind = "plain"
         if any(t.dtype != self._head_dtype for t in flat):
             raise ValueError(f"this processor was set up for {self._head_dtype} heads, got {sorted({str(t.dtype) for t in flat})}")
         self._check_layout(head_layout(self.family, flat))
-        return self._submit(flat, events, sync_input)
+        return self._submit(flat, events, sync_input, rows)
 
     def _check_layout(self, kind):
         if kind != self._layout:
             raise ValueError(f"this processor was set up for {_LAYOUT_NAMES[self._layout]} heads, got "
                              f"{_LAYOUT_NAMES[kind]} ones")
 
-    def submit_tta(self, passes, events=None, sync_input=True):
+    def submit_tta(self, passes, events=None, sync_input=True, info=None):
         """Enqueue one test-time-augmented batch: ``passes`` = [(heads, img_h, img_w, scale, flip_axis), ...] as for
         PostProcessor.run_tta, undone against the constructor's (img_h, img_w).  The passes' filter kernels append to one
         key list per image and one NMS kernel selects over all of them; rows are in un-augmented network-input pixels and
-        the local det_idx counts through the passes in order.  ``events`` / ``sync_input`` as for ``submit``."""
-        from .engine import flatten_heads
+        the local det_idx counts through the passes in order.  With ``info`` (as for ``submit``) the letterbox undo
+        follows the TTA undo, as in run_tta(info=...): rows in original-picture pixels.  ``events`` / ``sync_input`` as
+        for ``submit``."""
+        from .engine import flatten_heads, letterbox_rows
         if self._kind == "plain":
             raise ValueError("this processor was set up for plain batches: use submit")
         passes = list(passes)
@@ -402,6 +426,7 @@ class ShardedPostProcessor:
         for k, flat in enumerate(flats):
             if flat[0].shape[0] != self.batch:
                 raise ValueError(f"expected {self.batch} images per rank, got {flat[0].shape[0]} in pass {k}")
+        rows = None if info is None else letterbox_rows(info, self.batch)
         geom = tuple((int(h), int(w), float(s), int(f or 0)) for _, h, w, s, f in passes)
         dtypes = {t.dtype for flat in flats for t in flat}
         if len(dtypes) != 1:
@@ -419,61 +444,66 @@ class ShardedPostProcessor:
         self._check_layout(ents[0][1]["params"].input_kind)
         if any(e is not k for (_, e), k in zip(ents, self._tta["ents"])):
             raise ValueError("the head shapes differ from those of the first submit_tta")
-        return self._submit([t for flat in flats for t in flat], events, sync_input)
+        return self._submit([t for flat in flats for t in flat], events, sync_input, rows)
 
-    def _submit(self, flat, events, sync_input):
-        """Lane choice, plain launches / graph capture / replay and the NCCL all-gather of one batch whose heads (all
-        passes' for TTA) are ``flat``."""
+    def _submit(self, flat, events, sync_input, lb_rows):
+        """Lane choice, letterbox upload, plain launches / graph capture / replay and the NCCL all-gather of one batch
+        whose heads (all passes' for TTA) are ``flat``; ``lb_rows``: letterbox_rows of its info, or None."""
         lane = self._next % self.lanes
         self._next += 1
         st = self.streams[lane]
         if sync_input:
             st.wait_stream(torch.cuda.current_stream(self.device))
         with torch.cuda.device(self.device):
-            key = (lane,) + tuple(t.data_ptr() for t in flat)
+            sl = self._slots[lane]
+            # the lane's previous batch (its "done" event) ended after the previous copy out of the staging buffer; a
+            # graph captures the table's address and the copy, so a replay copies in the rows staged here
+            lb = None if lb_rows is None else sl["lb"].stage(lb_rows, sl["done"])
+            key = (lane, lb is not None) + tuple(t.data_ptr() for t in flat)
             if self.graph and events is None and not self._warmed:
                 # the very first batch runs as plain launches (lazy module load, function attributes) and counts as a
                 # normal step; graphs are captured from the second submission on
-                self._enqueue(_lib.head_pointer_array(flat), len(flat), lane, st, None)
+                self._enqueue(_lib.head_pointer_array(flat), len(flat), lane, st, None, lb)
                 torch.cuda.synchronize(self.device)
                 self._warmed = True
             elif self.graph and events is None:
                 gr = self._graphs.get(key)
                 if gr is None:
-                    gr = self._capture(flat, lane, st)
+                    gr = self._capture(flat, lane, st, lb)
                     self._graphs[key] = gr
                 with torch.cuda.stream(st):
                     gr.replay()
             else:
-                self._enqueue(_lib.head_pointer_array(flat), len(flat), lane, st, events)
+                self._enqueue(_lib.head_pointer_array(flat), len(flat), lane, st, events, lb)
             if self.mode == "nccl":
                 with torch.cuda.stream(st):
-                    sl = self._slots[lane]
                     dist.all_gather_into_tensor(sl["recv"].view(-1), sl["send"], group=self.group)
-        self._slots[lane]["done"].record(st)
+        sl["done"].record(st)
         if sync_input:
             for t in flat:
                 t.record_stream(st)
         return lane
 
-    def _capture(self, flat, lane, st):
+    def _capture(self, flat, lane, st, lb):
         ptrs = _lib.head_pointer_array(flat)
         torch.cuda.synchronize(self.device)
         g = torch.cuda.CUDAGraph()
         with torch.cuda.graph(g, stream=st, capture_error_mode="thread_local"):
-            self._enqueue(ptrs, len(flat), lane, st)
+            self._enqueue(ptrs, len(flat), lane, st, None, lb)
         g._ysb_keep = (ptrs, flat, self._tta)   # pointer arrays, heads and (TTA) the params / heads-per-pass arrays
         return g
 
     def gathered(self, ticket):
         """Device views (rows (world, batch, max_det, 6), counts (world, batch)); the caller's current stream is made to
-        wait for the batch (and, p2p, for every peer's rows)."""
+        wait for the batch (and, p2p, for every peer's rows).  Rank r's rows are in original-picture pixels when rank r
+        submitted the batch with ``info``, otherwise in network-input pixels."""
         sl = self._slots[ticket]
         torch.cuda.current_stream(self.device).wait_event(sl["done"])
         return sl["rows"], sl["cnt"]
 
     def result(self, ticket):
-        """list over the world*batch images in rank order: CPU float32 (K, 6) tensors, or None (a4.3 contract)."""
+        """list over the world*batch images in rank order: CPU float32 (K, 6) tensors, or None (a4.3 contract); pixels as
+        for ``gathered``."""
         rows, cnt = self.gathered(ticket)
         cnt_h = cnt.cpu()
         kmax = max(int(cnt_h.max().item()), 1)

@@ -234,6 +234,39 @@ def letterbox_table(info):
              float(d["org_shape"][1])] for d in info]
 
 
+def letterbox_rows(info, batch):
+    """letterbox_table(info); raises ValueError unless there is one dict per image of a ``batch``-image batch."""
+    if len(info) != batch:
+        raise ValueError(f"need one info dict per image: {len(info)} != {batch}")
+    return letterbox_table(info)
+
+
+class LetterboxStaging:
+    """One pipeline lane's letterbox table: the (batch, 5) float32 device table the NMS kernel's row write reads, and the
+    pinned staging buffer it is copied from with cudaMemcpyAsync on the lane's stream, so an upload never makes the host
+    wait for the lane's earlier work.  Construct it under the lane's stream; the table's address never changes (CUDA
+    graphs capture it, and may capture the copy as well)."""
+
+    def __init__(self, batch, device):
+        self.table = torch.empty((batch, 5), dtype=torch.float32, device=device)
+        self.host = torch.empty((batch, 5), dtype=torch.float32, pin_memory=True)
+        self._host_np = self.host.numpy()
+
+    def stage(self, rows, after):
+        """Write ``rows`` (letterbox_rows) into the staging buffer; returns the table's address.  ``after``: an event
+        recorded after the previous copy out of the buffer (None: there was none).  That copy may still be queued behind
+        the lane's earlier work -- in a detection gather, behind the flow control that waits for the peers -- and
+        overwriting the buffer before it ran would map that earlier batch with these rows."""
+        if after is not None:
+            after.synchronize()
+        self._host_np[...] = rows   # float32, rounded to nearest like torch.tensor(rows, dtype=torch.float32)
+        return self.table.data_ptr()
+
+    def enqueue_copy(self):
+        """The copy of the staged rows into the table on the current stream (capturable into a CUDA graph)."""
+        self.table.copy_(self.host, non_blocking=True)
+
+
 class DetectionList(list):
     """The evaluator's output list (CPU rows, the reference's contract) that also remembers the device rows it was read
     from, so that preds_postprocess can map them without staging them back to the GPU."""
@@ -443,32 +476,39 @@ class PostProcessor:
         preds_postprocess, val_yolov5.py:166-172); ``info`` None switches the undo off."""
         ptr = None
         if info is not None:
-            if len(info) != batch:
-                raise ValueError(f"need one info dict per image: {len(info)} != {batch}")
+            rows = torch.tensor(letterbox_rows(info, batch), dtype=torch.float32)
             if "lb" not in holder:
                 holder["lb"] = torch.empty((batch, 5), dtype=torch.float32, device=dev)
-            holder["lb"].copy_(torch.tensor(letterbox_table(info), dtype=torch.float32), non_blocking=False)
+            holder["lb"].copy_(rows, non_blocking=False)
             ptr = holder["lb"].data_ptr()
         for p in params_list:
             p.d_letterbox = ptr
 
+    def _run_entry(self, heads, img_h, img_w, decoded):
+        """(flat heads, cache entry) of one run; the entry is None for a batch of zero images."""
+        flat = [heads] if decoded else flatten_heads(self.family, heads)
+        if flat[0].shape[0] == 0:
+            return flat, None
+        kind = _lib.INPUT_DECODED_ROWS if decoded else _lib.INPUT_RAW_HEADS
+        return flat, self._prepare(flat, flat[0].shape[0], img_h, img_w, kind)
+
+    def _launch(self, flat, ent):
+        """The whole path for an entry whose params (letterbox pointer included) are set."""
+        out = ent["out"]
+        # through the torch extension (csrc/torch_adapter.cpp): tensor checks, device guard, torch's current stream
+        self._ops.postprocess(flat, ent["params_t"], ent["workspace"], out.dets, out.det_idx, out.det_cnt)
+        return out
+
     def run(self, heads, img_h, img_w, decoded=False, info=None):
         """Whole path on the device.  Returns DetectionBuffers (views into reused storage).  ``info``: optional list of
         the reference's letterbox dicts (scale, pad_top, pad_left, org_shape): rows come out in original-picture pixels."""
-        flat = [heads] if decoded else flatten_heads(self.family, heads)
-        batch = flat[0].shape[0]
-        if batch == 0:  # the reference loops over zero images and returns []
+        flat, ent = self._run_entry(heads, img_h, img_w, decoded)
+        if ent is None:  # the reference loops over zero images and returns []
             return DetectionBuffers(0, int(self.hyp["max_predictions_per_img"]), flat[0].device)
-        kind = _lib.INPUT_DECODED_ROWS if decoded else _lib.INPUT_RAW_HEADS
-        ent = self._prepare(flat, batch, img_h, img_w, kind)
-        out = ent["out"]
-        ws = ent["workspace"]
         dev = flat[0].device
         with torch.cuda.device(dev):
-            self._letterbox(ent, [ent["params"]], info, batch, dev)
-        # through the torch extension (csrc/torch_adapter.cpp): tensor checks, device guard, torch's current stream
-        self._ops.postprocess(flat, ent["params_t"], ws, out.dets, out.det_idx, out.det_cnt)
-        return out
+            self._letterbox(ent, [ent["params"]], info, flat[0].shape[0], dev)
+        return self._launch(flat, ent)
 
     # ---- test-time augmentation (trainer/eval_yolov5.py:152-179 and the same method of every evaluator) ------------
     def _tta_entries(self, passes, org_hw):
@@ -616,15 +656,18 @@ class PipelinedPostProcessor:
         dets = ppp.result(t)             # list[Tensor(K,6) | None], blocks on that batch only
 
     A ticket's buffers are reused ``lanes`` submissions later: fetch results before submitting that many new batches.
+    With ``info`` (as for PostProcessor.run) a batch's rows come out in original-picture pixels; each lane uploads its
+    own letterbox table on its stream (LetterboxStaging).
     """
 
     def __init__(self, family, hyp, anchors=None, compute_metric=False, lanes=4):
         self._pps = [PostProcessor(family, hyp, anchors, compute_metric) for _ in range(lanes)]
         self._streams = None
+        self._done = [None] * lanes   # per lane: the event recorded after its last batch
         self._next = 0
         self._layout = None   # contiguous or channels-last raw heads: fixed by the first submission
 
-    def submit(self, heads, img_h, img_w, decoded=False):
+    def submit(self, heads, img_h, img_w, decoded=False, info=None):
         flat = [heads] if decoded else flatten_heads(self._pps[0].family, heads)
         if not decoded:
             kind = head_layout(self._pps[0].family, flat)
@@ -633,6 +676,7 @@ class PipelinedPostProcessor:
             elif kind != self._layout:
                 names = {_lib.INPUT_RAW_HEADS: "contiguous", _lib.INPUT_RAW_HEADS_NHWC: "channels-last"}
                 raise ValueError(f"this processor was set up for {names[self._layout]} heads, got {names[kind]} ones")
+        rows = None if info is None else letterbox_rows(info, flat[0].shape[0])
         dev = flat[0].device
         if self._streams is None:
             self._streams = [torch.cuda.Stream(device=dev) for _ in self._pps]
@@ -641,9 +685,22 @@ class PipelinedPostProcessor:
         st = self._streams[i]
         st.wait_stream(torch.cuda.current_stream(dev))  # the heads were produced on the caller's stream
         with torch.cuda.stream(st):
-            out = self._pps[i].run(heads, img_h, img_w, decoded=decoded)
+            pp = self._pps[i]
+            flat, ent = pp._run_entry(heads, img_h, img_w, decoded)
+            if ent is None:   # zero images
+                out = DetectionBuffers(0, int(pp.hyp["max_predictions_per_img"]), dev)
+            else:
+                ent["params"].d_letterbox = None
+                if rows is not None:
+                    if "staging" not in ent:   # allocated under the lane's stream, like the entry's other buffers
+                        ent["staging"] = LetterboxStaging(flat[0].shape[0], dev)
+                    # the lane's previous batch ended after any earlier copy out of this staging buffer
+                    ent["params"].d_letterbox = ent["staging"].stage(rows, self._done[i])
+                    ent["staging"].enqueue_copy()
+                out = pp._launch(flat, ent)
             done = torch.cuda.Event()
             done.record(st)
+            self._done[i] = done
         for t in flat:
             t.record_stream(st)
         return (i, done, out)
