@@ -58,6 +58,7 @@ extern "C" {
 #define YSB_MAX_CLASSES 2048             /* class id must fit 11 bits of the wide sort key */
 #define YSB_MAX_PEERS 16            /* ranks (GPUs of one NVLink domain) in a detection gather */
 #define YSB_IPC_HANDLE_BYTES 64     /* sizeof(cudaIpcMemHandle_t) */
+#define YSB_CNT_ABSENT (-2)         /* gathered count of an image a rank did not have in a partial step */
 
 typedef enum ysb_status {
     YSB_OK = 0,
@@ -352,7 +353,13 @@ int ysb_undo_letterbox(float *d_dets, const int32_t *d_det_cnt, int batch, int m
  *                            whole filter + NMS pass earlier -- then rows + counts -> every peer's slot, then arrival counts)
  *     ysb_gather_wait        wait until the rows of every rank have landed in MY slot
  *   Every rank must run the same sequence of (slot) steps.  Spins are bounded (~20 s); a timeout sets `err`, which
- *   ysb_gather_error reads back (host sync). */
+ *   ysb_gather_error reads back (host sync).
+ *   Partial steps (the tail of a dataset that is not a multiple of world * batch): a rank that holds n < g->batch images
+ *   in a step calls ysb_select_nms_gather_partial (or ysb_select_nms_tta_gather_partial) with a plan of batch n, 0
+ *   included, in place of the strict entry; the rest of its step is unchanged.  The NMS kernel runs for images [0, n)
+ *   (no launch for n = 0), then one small kernel waits for every peer's ack of the slot, stores YSB_CNT_ABSENT into
+ *   every rank's count words of images [n, g->batch) and adds g->batch - n to the arrival counters, so every rank still
+ *   arrives with g->batch images per step and ysb_gather_wait works unchanged.  Rows of absent images are unspecified. */
 typedef struct ysb_gather {
     int32_t world, rank, slots, batch, max_det;
     void *d_buf[YSB_MAX_PEERS];   /* d_buf[rank] = own buffer (ysb_gather_alloc), the others = ysb_gather_open mappings */
@@ -377,6 +384,16 @@ int ysb_select_nms_gather(const ysb_params *p, const void *const *d_heads, int n
 int ysb_select_nms_tta_gather(const ysb_params *passes, int num_passes, const void *const *d_heads,
                               const int32_t *heads_per_pass, const uint64_t *d_keys, int64_t key_capacity,
                               const int32_t *d_counts, const ysb_gather *g, int slot, int32_t *d_det_idx, void *stream);
+/* Partial steps: the arguments of ysb_select_nms_gather / ysb_select_nms_tta_gather, but the plan may hold
+ * 0 <= batch <= g->batch images (max_det must still match); images [batch, g->batch) of this rank read YSB_CNT_ABSENT in
+ * every rank's slot.  Every refusal returns before any CUDA call. */
+int ysb_select_nms_gather_partial(const ysb_params *p, const void *const *d_heads, int num_heads, const uint64_t *d_keys,
+                                  int64_t key_capacity, const int32_t *d_counts, const ysb_gather *g, int slot,
+                                  int32_t *d_det_idx, void *stream);
+int ysb_select_nms_tta_gather_partial(const ysb_params *passes, int num_passes, const void *const *d_heads,
+                                      const int32_t *heads_per_pass, const uint64_t *d_keys, int64_t key_capacity,
+                                      const int32_t *d_counts, const ysb_gather *g, int slot, int32_t *d_det_idx,
+                                      void *stream);
 int ysb_gather_wait(const ysb_gather *g, int slot, void *stream);
 int ysb_gather_error(const ysb_gather *g, uint32_t *err_out);
 

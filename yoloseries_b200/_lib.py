@@ -33,6 +33,7 @@ ABI_VERSION = 6
 YSB_MAX_PASSES = 4
 YSB_MAX_PEERS = 16
 YSB_IPC_HANDLE_BYTES = 64
+YSB_CNT_ABSENT = -2   # gathered count of an image a rank did not have in a partial step
 YSB_OK, YSB_ERR_BAD_ARG, YSB_ERR_UNSUPPORTED, YSB_ERR_WORKSPACE, YSB_ERR_CUDA, YSB_ERR_LIMIT = 0, -1, -2, -3, -4, -5
 
 
@@ -175,6 +176,15 @@ _SIGNATURES = {
     "ysb_select_nms_gather": (ctypes.c_int, [ctypes.POINTER(YsbParams), ctypes.POINTER(ctypes.c_void_p), ctypes.c_int,
                                              ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p, ctypes.POINTER(YsbGather),
                                              ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p]),
+    "ysb_select_nms_gather_partial": (ctypes.c_int, [ctypes.POINTER(YsbParams), ctypes.POINTER(ctypes.c_void_p),
+                                                     ctypes.c_int, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p,
+                                                     ctypes.POINTER(YsbGather), ctypes.c_int, ctypes.c_void_p,
+                                                     ctypes.c_void_p]),
+    "ysb_select_nms_tta_gather_partial": (ctypes.c_int, [ctypes.POINTER(YsbParams), ctypes.c_int,
+                                                         ctypes.POINTER(ctypes.c_void_p), ctypes.POINTER(ctypes.c_int32),
+                                                         ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p,
+                                                         ctypes.POINTER(YsbGather), ctypes.c_int, ctypes.c_void_p,
+                                                         ctypes.c_void_p]),
     "ysb_gather_wait": (ctypes.c_int, [ctypes.POINTER(YsbGather), ctypes.c_int, ctypes.c_void_p]),
     "ysb_gather_error": (ctypes.c_int, [ctypes.POINTER(YsbGather), ctypes.POINTER(ctypes.c_uint32)]),
 }

@@ -19,6 +19,7 @@ bool make_gather_sink(const ysb_gather *g, int slot, GatherSink *out);
 bool gather_valid(const ysb_gather *g, int slot);
 cudaError_t launch_gather_begin(const ysb_gather *g, int slot, int32_t *d_counts, int64_t n_counts, cudaStream_t stream);
 cudaError_t launch_gather_wait(const ysb_gather *g, int slot, cudaStream_t stream);
+cudaError_t launch_gather_absent(const GatherSink &sink, int first, int batch, cudaStream_t stream);
 cudaError_t launch_select_nms_tta(const Plan &P, const ExtraPasses &X, const uint64_t *d_keys, int64_t key_cap,
                                   const int32_t *d_counts, float *d_dets, int32_t *d_det_idx, int32_t *d_det_cnt,
                                   cudaStream_t stream, const GatherSink *sink, int dtype);
@@ -468,9 +469,29 @@ int ysb_gather_begin(const ysb_gather *g, int slot, int32_t *d_counts, int64_t n
     return cuda_status(launch_gather_begin(g, slot, d_counts, n_counts, static_cast<cudaStream_t>(stream)));
 }
 
-int ysb_select_nms_gather(const ysb_params *p, const void *const *d_heads, int num_heads, const uint64_t *d_keys,
-                          int64_t key_capacity, const int32_t *d_counts, const ysb_gather *g, int slot,
-                          int32_t *d_det_idx, void *stream)
+// The plan's images against the gather's: a full step has exactly g->batch of them, a partial step 0..g->batch.
+static bool gather_matches(const ysb_gather *g, const Plan &P, bool partial)
+{
+    return (partial ? P.batch <= g->batch : P.batch == g->batch) && P.max_det == g->max_det;
+}
+
+// The NMS kernel for the plan's images (none for a plan of 0), then, for a partial step, the absent marks and arrival
+// counts of images [plan batch, g->batch).
+static int nms_gather(const Plan &P, const ExtraPasses *X, const uint64_t *d_keys, int64_t key_capacity,
+                      const int32_t *d_counts, const GatherSink &sink, int g_batch, int32_t *d_det_idx, int dtype,
+                      cudaStream_t s)
+{
+    const int e = cuda_status(X ? launch_select_nms_tta(P, *X, d_keys, key_capacity, d_counts, nullptr, d_det_idx, nullptr, s,
+                                                        &sink, dtype)
+                                : launch_select_nms(P, d_keys, key_capacity, d_counts, nullptr, d_det_idx, nullptr, s, &sink,
+                                                    dtype));
+    if (e != YSB_OK) return e;
+    return cuda_status(launch_gather_absent(sink, P.batch, g_batch, s));
+}
+
+static int select_nms_gather(const ysb_params *p, const void *const *d_heads, int num_heads, const uint64_t *d_keys,
+                             int64_t key_capacity, const int32_t *d_counts, const ysb_gather *g, int slot,
+                             int32_t *d_det_idx, void *stream, bool partial)
 {
     if (!d_heads || !d_keys || !d_counts) return YSB_ERR_BAD_ARG;
     Built b;
@@ -479,9 +500,23 @@ int ysb_select_nms_gather(const ysb_params *p, const void *const *d_heads, int n
     if (key_capacity < key_slots(b.plan)) return YSB_ERR_WORKSPACE;
     GatherSink sink;
     if (!make_gather_sink(g, slot, &sink)) return YSB_ERR_BAD_ARG;
-    if (g->batch != b.plan.batch || g->max_det != b.plan.max_det) return YSB_ERR_BAD_ARG;
-    return cuda_status(launch_select_nms(b.plan, d_keys, key_capacity, d_counts, nullptr, d_det_idx, nullptr,
-                                         static_cast<cudaStream_t>(stream), &sink, b.dtype));
+    if (!gather_matches(g, b.plan, partial)) return YSB_ERR_BAD_ARG;
+    return nms_gather(b.plan, nullptr, d_keys, key_capacity, d_counts, sink, g->batch, d_det_idx, b.dtype,
+                      static_cast<cudaStream_t>(stream));
+}
+
+int ysb_select_nms_gather(const ysb_params *p, const void *const *d_heads, int num_heads, const uint64_t *d_keys,
+                          int64_t key_capacity, const int32_t *d_counts, const ysb_gather *g, int slot,
+                          int32_t *d_det_idx, void *stream)
+{
+    return select_nms_gather(p, d_heads, num_heads, d_keys, key_capacity, d_counts, g, slot, d_det_idx, stream, false);
+}
+
+int ysb_select_nms_gather_partial(const ysb_params *p, const void *const *d_heads, int num_heads, const uint64_t *d_keys,
+                                  int64_t key_capacity, const int32_t *d_counts, const ysb_gather *g, int slot,
+                                  int32_t *d_det_idx, void *stream)
+{
+    return select_nms_gather(p, d_heads, num_heads, d_keys, key_capacity, d_counts, g, slot, d_det_idx, stream, true);
 }
 
 int ysb_gather_wait(const ysb_gather *g, int slot, void *stream)
@@ -630,9 +665,10 @@ int ysb_select_nms_tta(const ysb_params *passes, int num_passes, const void *con
                                              static_cast<cudaStream_t>(stream), nullptr, bp.b[0].dtype));
 }
 
-int ysb_select_nms_tta_gather(const ysb_params *passes, int num_passes, const void *const *d_heads,
-                              const int32_t *heads_per_pass, const uint64_t *d_keys, int64_t key_capacity,
-                              const int32_t *d_counts, const ysb_gather *g, int slot, int32_t *d_det_idx, void *stream)
+static int select_nms_tta_gather(const ysb_params *passes, int num_passes, const void *const *d_heads,
+                                 const int32_t *heads_per_pass, const uint64_t *d_keys, int64_t key_capacity,
+                                 const int32_t *d_counts, const ysb_gather *g, int slot, int32_t *d_det_idx, void *stream,
+                                 bool partial)
 {
     if (!d_heads || !heads_per_pass || !d_keys || !d_counts) return YSB_ERR_BAD_ARG;
     BuiltPasses bp;
@@ -641,10 +677,27 @@ int ysb_select_nms_tta_gather(const ysb_params *passes, int num_passes, const vo
     if (key_capacity < bp.slots) return YSB_ERR_WORKSPACE;
     GatherSink sink;
     if (!make_gather_sink(g, slot, &sink)) return YSB_ERR_BAD_ARG;
-    if (g->batch != bp.b[0].plan.batch || g->max_det != bp.b[0].plan.max_det) return YSB_ERR_BAD_ARG;
+    if (!gather_matches(g, bp.b[0].plan, partial)) return YSB_ERR_BAD_ARG;
     const ExtraPasses X = extra_passes(bp, num_passes);
-    return cuda_status(launch_select_nms_tta(bp.b[0].plan, X, d_keys, key_capacity, d_counts, nullptr, d_det_idx, nullptr,
-                                             static_cast<cudaStream_t>(stream), &sink, bp.b[0].dtype));
+    return nms_gather(bp.b[0].plan, &X, d_keys, key_capacity, d_counts, sink, g->batch, d_det_idx, bp.b[0].dtype,
+                      static_cast<cudaStream_t>(stream));
+}
+
+int ysb_select_nms_tta_gather(const ysb_params *passes, int num_passes, const void *const *d_heads,
+                              const int32_t *heads_per_pass, const uint64_t *d_keys, int64_t key_capacity,
+                              const int32_t *d_counts, const ysb_gather *g, int slot, int32_t *d_det_idx, void *stream)
+{
+    return select_nms_tta_gather(passes, num_passes, d_heads, heads_per_pass, d_keys, key_capacity, d_counts, g, slot,
+                                 d_det_idx, stream, false);
+}
+
+int ysb_select_nms_tta_gather_partial(const ysb_params *passes, int num_passes, const void *const *d_heads,
+                                      const int32_t *heads_per_pass, const uint64_t *d_keys, int64_t key_capacity,
+                                      const int32_t *d_counts, const ysb_gather *g, int slot, int32_t *d_det_idx,
+                                      void *stream)
+{
+    return select_nms_tta_gather(passes, num_passes, d_heads, heads_per_pass, d_keys, key_capacity, d_counts, g, slot,
+                                 d_det_idx, stream, true);
 }
 
 int ysb_postprocess_tta(const ysb_params *passes, int num_passes, const void *const *d_heads, const int32_t *heads_per_pass,

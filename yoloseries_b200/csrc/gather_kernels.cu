@@ -3,10 +3,12 @@
 //
 // Every rank owns one symmetric receive buffer, mapped by its peers through CUDA IPC (NVLink P2P).  The producer side
 // lives in the NMS kernel (nms_kernel.cu: the ordered row write stores into every peer's slot and then adds one
-// system-scope arrival count per image); this file holds the buffer management and the two flow-control kernels:
+// system-scope arrival count per image); this file holds the buffer management and the flow-control kernels:
 //   k_gather_begin  zero the filter counters of the step; publish "I am done reading the previous use of this slot"
 //                   (ack) to every peer.  The NMS kernel waits for the peers' acks before it overwrites their slots.
 //   k_gather_wait   wait until all images of every rank have landed in my slot; bump the slot's use counter
+//   k_gather_absent (partial steps) mark this rank's images beyond the ones it had as absent in every slot, and count
+//                   them as arrived
 // Spins are volatile loads of LOCAL memory that peers write remotely (the L2 is the point of coherence for incoming
 // NVLink writes), bounded by a wall-clock limit: a timeout sets the buffer's err word instead of hanging the GPU.
 #include <cstring>
@@ -52,6 +54,22 @@ __global__ void __launch_bounds__(32) k_gather_wait(const __grid_constant__ Wait
     __threadfence_system();   // the rows behind the counters are visible to everything that follows on this stream
     __syncwarp();
     if (r == 0) *a.use = u + 1u;
+}
+
+// Images [first, batch) of this rank are absent from this step (a partial step, ysb_select_nms_gather_partial): the
+// M <= 0 branch of k_select_nms for a range of images, with the absent mark instead of -1.  Once per peer: wait for its
+// ack of this slot, then YSB_CNT_ABSENT into every rank's count words of those images, then one arrival increment of
+// batch - first, so k_gather_wait's target (use + 1) * batch and the ack protocol of later steps hold unchanged.
+__global__ void __launch_bounds__(256) k_gather_absent(const __grid_constant__ GatherSink G, int first, int batch)
+{
+    const int tid = threadIdx.x;
+    if (tid < G.world && tid != G.rank && !spin_until_reached(G.my_ack + tid, *G.use)) atomicExch(G.err, 1u);
+    __syncthreads();
+    const int n = batch - first;
+    for (int e = tid; e < G.world * n; e += blockDim.x) G.cnt[e / n][first + e % n] = YSB_CNT_ABSENT;
+    __threadfence_system();   // release: the marks are ordered before the arrival counts the peers wait for
+    __syncthreads();
+    if (tid < G.world) atomicAdd_system(G.arrived[tid], static_cast<unsigned int>(n));
 }
 
 static bool gather_ok(const ysb_gather *g, int slot)
@@ -114,6 +132,13 @@ cudaError_t launch_gather_wait(const ysb_gather *g, int slot, cudaStream_t strea
     a.use = reinterpret_cast<unsigned int *>(at(mine, L.use)) + slot;
     a.err = reinterpret_cast<unsigned int *>(at(mine, L.err));
     k_gather_wait<<<1, 32, 0, stream>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_gather_absent(const GatherSink &sink, int first, int batch, cudaStream_t stream)
+{
+    if (first >= batch) return cudaSuccess;
+    k_gather_absent<<<1, 256, 0, stream>>>(sink, first, batch);
     return cudaGetLastError();
 }
 

@@ -235,6 +235,17 @@ class ShardedPostProcessor:
 
     ``info`` is decided per submission (None: network-input pixels); one dict per image, otherwise ValueError.
 
+    Partial steps (the tail of a dataset that is not a multiple of world * batch): with ``partial=True`` a rank may
+    submit any 0 <= n <= batch images, and ranks may differ within the step.  Every rank still submits once per step,
+    with zero images if it has none (a rank that skips a step makes its peers time out).  The images a rank did not have
+    read count -2 in ``gathered`` and are left out of ``result``.  Partial steps run as plain launches, never as graphs;
+    their heads must have the per-image shapes, dtype and layout of the set-up.  The first submission must hold at least
+    one image.  Without ``partial=True`` any count but ``batch`` raises ValueError: mid-run, a short batch is usually a
+    sharding bug.
+
+        lo, hi = shard_bounds(len(tail), rank, world)                  # the last, short step
+        t = spp.submit([h[lo:hi] for h in heads], info=info[lo:hi], partial=True)   # hi - lo may be 0
+
     Lanes, graphs and the gather work as for ``submit``.  The first submission fixes the kind (plain or TTA): a processor
     takes only ``submit`` or only ``submit_tta`` calls.  For TTA it also fixes the number of passes, each pass's
     (img_h, img_w, scale, flip_axis) and the head shapes, and sizes the key buffers to the passes' summed key slots; a
@@ -285,10 +296,18 @@ class ShardedPostProcessor:
     def _prepare(self, flat):
         if self._ent is not None:
             return
+        self._need_images(flat[0].shape[0])
         self._ent = self.pp._prepare(flat, self.batch, self.img_h, self.img_w, _lib.INPUT_RAW_HEADS)
         self._head_dtype = flat[0].dtype
         self._layout = self._ent["params"].input_kind
+        self._set_shapes(flat)
         self._alloc_lanes(self._ent["N"] * self._slots_per_candidate())
+
+    @staticmethod
+    def _need_images(n):
+        if n == 0:
+            raise ValueError("the first submission must hold at least one image: it fixes the head shapes, dtype and "
+                             "layout of the processor")
 
     def _slots_per_candidate(self):
         return int(self.pp.hyp["num_class"]) if self.pp.hyp["mutil_label"] else 1
@@ -301,6 +320,7 @@ class ShardedPostProcessor:
                          per_pass=(ctypes.c_int32 * n)(*[len(flat) for flat, _ in ents]))
         self._head_dtype = ents[0][0][0].dtype
         self._layout = ents[0][1]["params"].input_kind
+        self._set_shapes([t for flat, _ in ents for t in flat])
         self._alloc_lanes(sum(e["N"] for _, e in ents) * self._slots_per_candidate())
 
     def _alloc_lanes(self, n):
@@ -327,6 +347,7 @@ class ShardedPostProcessor:
                     sl["rows"], sl["cnt"] = self.dg.views(s)
                 elif self.mode == "nccl":
                     sl["send"] = torch.zeros(b * d * 6 + b, dtype=torch.float32, device=dev)
+                    sl["send_cnt"] = sl["send"][b * d * 6:].view(torch.int32)
                     sl["recv"] = torch.empty((self.world, b * d * 6 + b), dtype=torch.float32, device=dev)
                     sl["rows"] = sl["recv"][:, : b * d * 6].view(self.world, b, d, 6)
                     sl["cnt"] = sl["recv"][:, b * d * 6:].view(torch.int32)
@@ -335,25 +356,35 @@ class ShardedPostProcessor:
                     sl["cnt"] = torch.zeros((1, b), dtype=torch.int32, device=dev)
             self._slots.append(sl)
 
-    def _enqueue(self, ptrs, nheads, lane, st, events=None, lb=None):
+    def _enqueue(self, ptrs, nheads, lane, st, events=None, lb=None, n=None):
         """The launch sequence of one batch on stream ``st`` (plain C-ABI calls and a copy: capturable into a CUDA
         graph).  ``lb``: address of the lane's letterbox table, whose staged rows the sequence copies in first, or None
-        for rows in network-input pixels."""
+        for rows in network-input pixels.  ``n``: the image count of a partial step (fewer than ``batch``), else None."""
         lib, sl = self.lib, self._slots[lane]
         sp = ctypes.c_void_p(st.cuda_stream)
         # the plain and the TTA entry points take the same arguments after the heads; the params are shared by the lanes,
-        # and every call copies them, so the lane's table pointer is set right before the calls
+        # and every call copies them, so the lane's table pointer is set right before the calls.  A partial step gets its
+        # own copy with batch = n: captured graphs and the other lanes read the shared ones.
         if self._kind == "tta":
             tta, sfx = self._tta, "_tta"
-            for p in tta["params"]:
+            params = tta["params"]
+            if n is not None:
+                params = (_lib.YsbParams * len(params))(*params)
+                for p in params:
+                    p.batch = n
+            for p in params:
                 p.d_letterbox = lb
-            head = (tta["params"], len(tta["params"]), ptrs, tta["per_pass"])
+            head = (params, len(params), ptrs, tta["per_pass"])
         else:
             sfx = ""
-            self._ent["params"].d_letterbox = lb
-            head = (ctypes.byref(self._ent["params"]), ptrs, nheads)
+            params = self._ent["params"]
+            if n is not None:
+                params = _lib.YsbParams.from_buffer_copy(params)
+                params.batch = n
+            params.d_letterbox = lb
+            head = (ctypes.byref(params), ptrs, nheads)
         filt, nms = getattr(lib, "ysb_filter_candidates" + sfx), getattr(lib, "ysb_select_nms" + sfx)
-        nms_gather = getattr(lib, "ysb_select_nms" + sfx + "_gather")
+        nms_gather = getattr(lib, "ysb_select_nms" + sfx + ("_gather" if n is None else "_gather_partial"))
         if self.mode == "p2p":
             # first thing of the step: tell the peers this slot's previous contents have been consumed (they check it
             # right before storing into it, a filter + NMS pass from now)
@@ -370,7 +401,7 @@ class ShardedPostProcessor:
             events[1].record(st)
         if self.mode == "p2p":
             _lib.check(nms_gather(*head, sl["keys"].data_ptr(), self._key_cap, sl["counts"].data_ptr(), g, lane,
-                                  sl["idx"].data_ptr(), sp), "ysb_select_nms" + sfx + "_gather")
+                                  sl["idx"].data_ptr(), sp), nms_gather.__name__)
             if events:
                 events[2].record(st)
             _lib.check(lib.ysb_gather_wait(g, lane, sp), "ysb_gather_wait")
@@ -381,52 +412,84 @@ class ShardedPostProcessor:
                 rows_ptr, cnt_ptr = sl["rows"].data_ptr(), sl["cnt"].data_ptr()
             _lib.check(nms(*head, sl["keys"].data_ptr(), self._key_cap, sl["counts"].data_ptr(), rows_ptr,
                            sl["idx"].data_ptr(), cnt_ptr, sp), "ysb_select_nms" + sfx)
+            if n is not None:   # the images this rank did not have in a partial step
+                with torch.cuda.stream(st):
+                    (sl["send_cnt"] if self.mode == "nccl" else sl["cnt"][0])[n:].fill_(_lib.YSB_CNT_ABSENT)
             if events:
                 events[2].record(st)
 
     # ---- public ----------------------------------------------------------------------------------------------------
-    def submit(self, heads, events=None, sync_input=True, info=None):
+    def submit(self, heads, events=None, sync_input=True, info=None, partial=False):
         """Enqueue one batch.  ``events``: optional 3 timing events (start, filter done, NMS done) recorded on the lane's
         stream.  ``sync_input=False`` skips the wait on the caller's current stream (heads known to be ready).  ``info``:
         this rank's letterbox dicts (scale, pad_top, pad_left, org_shape), one per image as for PostProcessor.run: its
-        rows are then stored in original-picture pixels, into every rank's slot; None keeps network-input pixels."""
+        rows are then stored in original-picture pixels, into every rank's slot; None keeps network-input pixels.
+        ``partial=True``: this rank may hold any 0 <= n <= batch images in this step (see the class docstring)."""
         from .engine import flatten_heads, head_layout, letterbox_rows
         if self._kind == "tta":
             raise ValueError("this processor was set up for test-time-augmented batches: use submit_tta")
         flat = flatten_heads(self.family, heads)
-        if flat[0].shape[0] != self.batch:
-            raise ValueError(f"expected {self.batch} images per rank, got {flat[0].shape[0]}")
-        rows = None if info is None else letterbox_rows(info, self.batch)
+        n = flat[0].shape[0]
+        if n != self.batch:
+            self._check_count(n, partial)
+        rows = None if info is None else letterbox_rows(info, n)
         self._prepare(flat)
         self._kind = "plain"
         if any(t.dtype != self._head_dtype for t in flat):
             raise ValueError(f"this processor was set up for {self._head_dtype} heads, got {sorted({str(t.dtype) for t in flat})}")
-        self._check_layout(head_layout(self.family, flat))
-        return self._submit(flat, events, sync_input, rows)
+        if n:   # zero-image tensors count as contiguous whatever their strides: nothing of them is read
+            self._check_layout(head_layout(self.family, flat))
+        self._check_shapes(flat, n)
+        return self._submit(flat, events, sync_input, rows, n)
+
+    def _check_count(self, n, partial, where=""):
+        if partial:
+            if n > self.batch:
+                raise ValueError(f"expected at most {self.batch} images per rank, got {n}{where}")
+        elif n != self.batch:
+            raise ValueError(f"expected {self.batch} images per rank, got {n}{where}")
+
+    def _set_shapes(self, flat):
+        """Cache the set-up's head shapes as torch.Size objects: per image, and of a full batch."""
+        self._shapes = [t.shape[1:] for t in flat]
+        self._full_shapes = [torch.Size((self.batch,) + tuple(s)) for s in self._shapes]
+
+    def _check_shapes(self, flat, n):
+        """Per-image head shapes against the set-up's.  submit is on the host's critical path at small batches, so a full
+        batch compares one list of shapes with the cached one (the batch dimension matches by then)."""
+        if n == self.batch:
+            same = [t.shape for t in flat] == self._full_shapes
+        else:
+            same = [t.shape[1:] for t in flat] == self._shapes
+        if not same:
+            raise ValueError(f"the head shapes differ from those of the first submission: per image "
+                             f"{[tuple(s) for s in self._shapes]}, got {[tuple(t.shape[1:]) for t in flat]}")
 
     def _check_layout(self, kind):
         if kind != self._layout:
             raise ValueError(f"this processor was set up for {_LAYOUT_NAMES[self._layout]} heads, got "
                              f"{_LAYOUT_NAMES[kind]} ones")
 
-    def submit_tta(self, passes, events=None, sync_input=True, info=None):
+    def submit_tta(self, passes, events=None, sync_input=True, info=None, partial=False):
         """Enqueue one test-time-augmented batch: ``passes`` = [(heads, img_h, img_w, scale, flip_axis), ...] as for
         PostProcessor.run_tta, undone against the constructor's (img_h, img_w).  The passes' filter kernels append to one
         key list per image and one NMS kernel selects over all of them; rows are in un-augmented network-input pixels and
         the local det_idx counts through the passes in order.  With ``info`` (as for ``submit``) the letterbox undo
-        follows the TTA undo, as in run_tta(info=...): rows in original-picture pixels.  ``events`` / ``sync_input`` as
-        for ``submit``."""
-        from .engine import flatten_heads, letterbox_rows
+        follows the TTA undo, as in run_tta(info=...): rows in original-picture pixels.  ``events`` / ``sync_input`` /
+        ``partial`` as for ``submit``; every pass holds the same images."""
+        from .engine import flatten_heads, head_layout, letterbox_rows
         if self._kind == "plain":
             raise ValueError("this processor was set up for plain batches: use submit")
         passes = list(passes)
         if not 1 <= len(passes) <= _lib.YSB_MAX_PASSES:
             raise ValueError(f"1..{_lib.YSB_MAX_PASSES} passes, got {len(passes)}")
         flats = [flatten_heads(self.family, p[0]) for p in passes]
+        n = flats[0][0].shape[0]
         for k, flat in enumerate(flats):
-            if flat[0].shape[0] != self.batch:
-                raise ValueError(f"expected {self.batch} images per rank, got {flat[0].shape[0]} in pass {k}")
-        rows = None if info is None else letterbox_rows(info, self.batch)
+            self._check_count(flat[0].shape[0], partial, f" in pass {k}")
+            if flat[0].shape[0] != n:
+                raise ValueError(f"every pass must hold the same images: {n} in pass 0, {flat[0].shape[0]} in pass {k}")
+        rows = None if info is None else letterbox_rows(info, n)
         geom = tuple((int(h), int(w), float(s), int(f or 0)) for _, h, w, s, f in passes)
         dtypes = {t.dtype for flat in flats for t in flat}
         if len(dtypes) != 1:
@@ -437,18 +500,28 @@ class ShardedPostProcessor:
                                  f"{list(self._tta['geom'])}, got {list(geom)}")
             if dtypes != {self._head_dtype}:
                 raise ValueError(f"this processor was set up for {self._head_dtype} heads, got {sorted(map(str, dtypes))}")
-        ents = self.pp._tta_entries(passes, (self.img_h, self.img_w))
+        flat_all = [t for flat in flats for t in flat]
+        if self._tta is not None and n != self.batch:
+            # a partial step: no cache entries of its own (its params are a copy of the set-up's with batch = n)
+            if n:
+                self._check_layout(head_layout(self.family, flat_all))
+            self._check_shapes(flat_all, n)
+            return self._submit(flat_all, events, sync_input, rows, n)
+        if self._tta is None:
+            self._need_images(n)
+        ents = self.pp._tta_entries(passes, (self.img_h, self.img_w), batch=self.batch)
         if self._tta is None:
             self._prepare_tta(ents, geom)
             self._kind = "tta"
         self._check_layout(ents[0][1]["params"].input_kind)
         if any(e is not k for (_, e), k in zip(ents, self._tta["ents"])):
             raise ValueError("the head shapes differ from those of the first submit_tta")
-        return self._submit([t for flat in flats for t in flat], events, sync_input, rows)
+        return self._submit(flat_all, events, sync_input, rows, n)
 
-    def _submit(self, flat, events, sync_input, lb_rows):
+    def _submit(self, flat, events, sync_input, lb_rows, n):
         """Lane choice, letterbox upload, plain launches / graph capture / replay and the NCCL all-gather of one batch
-        whose heads (all passes' for TTA) are ``flat``; ``lb_rows``: letterbox_rows of its info, or None."""
+        whose heads (all passes' for TTA) are ``flat``; ``lb_rows``: letterbox_rows of its info, or None; ``n``: its
+        image count (a partial step when below ``batch``: plain launches, never a graph)."""
         lane = self._next % self.lanes
         self._next += 1
         st = self.streams[lane]
@@ -458,15 +531,17 @@ class ShardedPostProcessor:
             sl = self._slots[lane]
             # the lane's previous batch (its "done" event) ended after the previous copy out of the staging buffer; a
             # graph captures the table's address and the copy, so a replay copies in the rows staged here
-            lb = None if lb_rows is None else sl["lb"].stage(lb_rows, sl["done"])
-            key = (lane, lb is not None) + tuple(t.data_ptr() for t in flat)
-            if self.graph and events is None and not self._warmed:
+            lb = None if not lb_rows else sl["lb"].stage(lb_rows, sl["done"])
+            if n != self.batch:
+                self._enqueue(_lib.head_pointer_array(flat), len(flat), lane, st, events, lb, n)
+            elif self.graph and events is None and not self._warmed:
                 # the very first batch runs as plain launches (lazy module load, function attributes) and counts as a
                 # normal step; graphs are captured from the second submission on
                 self._enqueue(_lib.head_pointer_array(flat), len(flat), lane, st, None, lb)
                 torch.cuda.synchronize(self.device)
                 self._warmed = True
             elif self.graph and events is None:
+                key = (lane, lb is not None) + tuple(t.data_ptr() for t in flat)
                 gr = self._graphs.get(key)
                 if gr is None:
                     gr = self._capture(flat, lane, st, lb)
@@ -496,14 +571,16 @@ class ShardedPostProcessor:
     def gathered(self, ticket):
         """Device views (rows (world, batch, max_det, 6), counts (world, batch)); the caller's current stream is made to
         wait for the batch (and, p2p, for every peer's rows).  Rank r's rows are in original-picture pixels when rank r
-        submitted the batch with ``info``, otherwise in network-input pixels."""
+        submitted the batch with ``info``, otherwise in network-input pixels.  After a partial step the images a rank
+        did not have read count YSB_CNT_ABSENT (-2), and their rows are unspecified."""
         sl = self._slots[ticket]
         torch.cuda.current_stream(self.device).wait_event(sl["done"])
         return sl["rows"], sl["cnt"]
 
     def result(self, ticket):
-        """list over the world*batch images in rank order: CPU float32 (K, 6) tensors, or None (a4.3 contract); pixels as
-        for ``gathered``."""
+        """list over the images every rank had in this step, in rank order: CPU float32 (K, 6) tensors, or None (a4.3
+        contract); pixels as for ``gathered``.  A full step gives world*batch entries; after a partial step the absent
+        images are skipped, so with per-rank shard_bounds slices of a step's images the list is in their global order."""
         rows, cnt = self.gathered(ticket)
         cnt_h = cnt.cpu()
         kmax = max(int(cnt_h.max().item()), 1)
@@ -512,7 +589,8 @@ class ShardedPostProcessor:
         for r in range(rows_h.shape[0]):
             for i in range(self.batch):
                 c = int(cnt_h[r, i])
-                out.append(None if c < 0 else rows_h[r, i, :c].clone())
+                if c != _lib.YSB_CNT_ABSENT:
+                    out.append(None if c < 0 else rows_h[r, i, :c].clone())
         return out
 
     def drain(self):

@@ -253,13 +253,14 @@ class LetterboxStaging:
         self._host_np = self.host.numpy()
 
     def stage(self, rows, after):
-        """Write ``rows`` (letterbox_rows) into the staging buffer; returns the table's address.  ``after``: an event
+        """Write ``rows`` (letterbox_rows, up to ``batch`` of them) into the first rows of the staging buffer; returns the
+        table's address.  ``after``: an event
         recorded after the previous copy out of the buffer (None: there was none).  That copy may still be queued behind
         the lane's earlier work -- in a detection gather, behind the flow control that waits for the peers -- and
         overwriting the buffer before it ran would map that earlier batch with these rows."""
         if after is not None:
             after.synchronize()
-        self._host_np[...] = rows   # float32, rounded to nearest like torch.tensor(rows, dtype=torch.float32)
+        self._host_np[:len(rows)] = rows   # float32, rounded to nearest like torch.tensor(rows, dtype=torch.float32)
         return self.table.data_ptr()
 
     def enqueue_copy(self):
@@ -511,15 +512,17 @@ class PostProcessor:
         return self._launch(flat, ent)
 
     # ---- test-time augmentation (trainer/eval_yolov5.py:152-179 and the same method of every evaluator) ------------
-    def _tta_entries(self, passes, org_hw):
-        """passes: [(heads, img_h, img_w, scale, flip_axis), ...] -> [(flat heads, cache entry), ...]."""
+    def _tta_entries(self, passes, org_hw, batch=None):
+        """passes: [(heads, img_h, img_w, scale, flip_axis), ...] -> [(flat heads, cache entry), ...].  ``batch``: the
+        entries' image count when it is not the heads' (a sharded processor set up by a partial step)."""
         if not 1 <= len(passes) <= _lib.YSB_MAX_PASSES:
             raise ValueError(f"1..{_lib.YSB_MAX_PASSES} passes, got {len(passes)}")
         ents = []
         for heads, img_h, img_w, scale, flip in passes:
             flat = flatten_heads(self.family, heads)
             tta = (float(scale), int(flip or 0), int(org_hw[0]), int(org_hw[1]))
-            ents.append((flat, self._prepare(flat, flat[0].shape[0], int(img_h), int(img_w), _lib.INPUT_RAW_HEADS, tta)))
+            b = flat[0].shape[0] if batch is None else batch
+            ents.append((flat, self._prepare(flat, b, int(img_h), int(img_w), _lib.INPUT_RAW_HEADS, tta)))
         if len({e["params"].batch for _, e in ents}) != 1:
             raise ValueError("every pass must hold the same images")
         if len({e["params"].input_kind for _, e in ents}) != 1:
