@@ -23,6 +23,7 @@
  *   ysb_wbf, ysb_wbf_collect  weighted_fusion_bbox / do_wfb   utils/weighted_fusion_bbox.py:41-96, trainer/eval_yolov5.py:44-92
  *   ysb_map_iou           utils.mAP.iou                    utils/mAP.py:18-42
  *   ysb_compute_tp        mAP_v2.compute_tp                utils/mAP.py:70-100
+ *   ysb_match_tp, ysb_match_compact  the same on the post-processors' own row blocks, + the per-run concatenation
  *   ysb_nms               utils.numba_nms / utils.gpu_nms  utils/nms.py:10-27 / 30-65
  *   ysb_pairwise_iou      utils.numba_iou / utils.gpu_iou  utils/bbox_tools.py:12-35 / 164-190
  *   ysb_elementwise_iou   utils.gpu_Giou/gpu_DIoU/gpu_CIoU utils/bbox_tools.py:193-339
@@ -85,7 +86,8 @@ typedef enum ysb_family {
 typedef enum ysb_dtype {
     YSB_F32 = 0,
     YSB_F16 = 1,   /* IEEE binary16 (torch.float16) */
-    YSB_BF16 = 2   /* bfloat16 (torch.bfloat16) */
+    YSB_BF16 = 2,  /* bfloat16 (torch.bfloat16) */
+    YSB_F64 = 3    /* float64: ground truth of ysb_match_step only (heads refuse it) */
 } ysb_dtype;
 
 /* What d_heads point to.  RAW_HEADS_NHWC (added in ABI version 6 without a layout change of ysb_params; an older library
@@ -316,6 +318,43 @@ int ysb_compute_tp_workspace_bytes(int64_t total_gt, size_t *bytes_out);
 int ysb_compute_tp(const void *d_gt, const int64_t *d_gt_offsets, int64_t total_gt, const void *d_pred,
                    const int64_t *d_pred_offsets, int64_t total_pred, int batch, int is_f64, const double *iou_thresholds,
                    void *d_workspace, size_t workspace_bytes, uint8_t *d_tp, void *stream);
+
+/* The same matching on the rows where the post-processors keep them: a (world, batch, max_det, 6) float32 block (the
+ * rows of DetectionBuffers with world = 1, or one gather slot, ysb_gather_slot_views / ysb_gather_strides) and its
+ * (world, batch) counts, against padded ground truth.  Image k = rank * batch + i; one step = one such block.
+ *   count c >= 0: c rows;  -1 (the reference's None): no rows, the image's ground truth still counts as targets;
+ *   YSB_CNT_ABSENT: the image is not part of the step (partial gather steps): skipped, its tp rows are left untouched.
+ * Ground truth rows (x1, y1, x2, y2, cls) are gt_dtype, one type per call: YSB_F32 matches in float32, YSB_F64 in
+ * float64 with the float32 rows widened exactly -- what ysb_compute_tp computes on the promoted arrays.  Counts above
+ * max_gt (or max_det) are clamped to it. */
+typedef struct ysb_match_step {
+    int32_t world, batch, max_det, max_gt;
+    const float *d_rows;         /* rank r's (batch, max_det, 6) rows start r * rows_rank_bytes after d_rows */
+    int64_t rows_rank_bytes;     /* >= batch * max_det * 24 */
+    const int32_t *d_cnt;        /* rank r's (batch) counts start r * cnt_rank_bytes after d_cnt */
+    int64_t cnt_rank_bytes;      /* >= batch * 4 */
+    const void *d_gt;            /* (world, batch, max_gt, 5) gt_dtype, dense */
+    const int32_t *d_gt_cnt;     /* (world, batch) int32, dense: ground-truth rows of every image */
+    int32_t gt_dtype;            /* YSB_F32 or YSB_F64 */
+} ysb_match_step;
+
+/* ysb_match_tp: d_tp (world, batch, max_det, 10) uint8 <- for every present image, ysb_compute_tp of its ground truth
+ * and its rows, bit for bit, aligned with the rows (rows past the count are not written).  iou_thresholds: 10 HOST
+ * doubles.  One launch, one CTA per image.  Workspace: one int32 per ground-truth slot (world * batch * max_gt).
+ * ysb_match_compact: appends the step's present images, in image order, to the caller's run-long arrays: per kept
+ * row d_conf[p] = score, d_pred_cls[p] = class (float32) and d_tp_out[p] (10 uint8, from d_tp of ysb_match_tp); per
+ * ground-truth row d_target_cls[g] = class (float64).  d_acc_in = {rows, targets} appended so far (int64, device), read;
+ * d_acc_out (another 2 int64) <- d_acc_in + the step's rows and targets: feed it to the next step as d_acc_in.  Rows
+ * or targets beyond the capacities are counted in d_acc_out but not written.  The result is the concatenation of
+ * mAP_v2.compute_tp over the images in order, the arrays the AP integration consumes.
+ * Both refuse, before any CUDA call: null pointers, negative sizes, world < 1 or > YSB_MAX_PEERS, strides smaller than
+ * a rank's rows / counts, max_det > YSB_MAX_DET_LIMIT (YSB_ERR_LIMIT), an unknown gt_dtype, d_acc_in == d_acc_out. */
+int ysb_match_tp_workspace_bytes(const ysb_match_step *step, size_t *bytes_out);
+int ysb_match_tp(const ysb_match_step *step, const double *iou_thresholds, void *d_workspace, size_t workspace_bytes,
+                 uint8_t *d_tp, void *stream);
+int ysb_match_compact(const ysb_match_step *step, const uint8_t *d_tp, const int64_t *d_acc_in, int64_t *d_acc_out,
+                      float *d_conf, float *d_pred_cls, uint8_t *d_tp_out, int64_t row_capacity, double *d_target_cls,
+                      int64_t target_capacity, void *stream);
 
 /* Soft-NMS (utils/nms.py:68-140; no caller in the reference, float32 GIoU/DIoU/CIoU flavours only -- 'iou' is broken
  * there).  Repeats: pick the first arg-max, record processed[idx] = its current score, decay every score whose IoU with

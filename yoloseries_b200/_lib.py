@@ -25,6 +25,7 @@ INPUT_RAW_HEADS, INPUT_DECODED_ROWS = 0, 1
 INPUT_RAW_HEADS_NHWC = 2   # raw heads in channels-last memory (YOLOv5, YOLOX, YOLOv8, FCOS)
 # enum ysb_dtype (element type of the raw heads)
 DTYPE_F32, DTYPE_F16, DTYPE_BF16 = 0, 1, 2
+DTYPE_F64 = 3   # ground truth of ysb_match_step only
 IOU_NUMBA_F64MIX, IOU_F32, GIOU, DIOU, CIOU = range(5)
 IOU_KIND_IDS = {"numba": IOU_NUMBA_F64MIX, "iou": IOU_F32, "giou": GIOU, "diou": DIOU, "ciou": CIOU}
 CMP_GE, CMP_GT = 0, 1
@@ -84,6 +85,23 @@ class YsbGather(ctypes.Structure):
         ("batch", ctypes.c_int32),
         ("max_det", ctypes.c_int32),
         ("d_buf", ctypes.c_void_p * YSB_MAX_PEERS),
+    ]
+
+
+class YsbMatchStep(ctypes.Structure):
+    """Mirror of ``struct ysb_match_step``."""
+    _fields_ = [
+        ("world", ctypes.c_int32),
+        ("batch", ctypes.c_int32),
+        ("max_det", ctypes.c_int32),
+        ("max_gt", ctypes.c_int32),
+        ("d_rows", ctypes.c_void_p),
+        ("rows_rank_bytes", ctypes.c_int64),
+        ("d_cnt", ctypes.c_void_p),
+        ("cnt_rank_bytes", ctypes.c_int64),
+        ("d_gt", ctypes.c_void_p),
+        ("d_gt_cnt", ctypes.c_void_p),
+        ("gt_dtype", ctypes.c_int32),
     ]
 
 
@@ -161,6 +179,12 @@ _SIGNATURES = {
     "ysb_compute_tp": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p,
                                       ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_double),
                                       ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p, ctypes.c_void_p]),
+    "ysb_match_tp_workspace_bytes": (ctypes.c_int, [ctypes.POINTER(YsbMatchStep), ctypes.POINTER(ctypes.c_size_t)]),
+    "ysb_match_tp": (ctypes.c_int, [ctypes.POINTER(YsbMatchStep), ctypes.POINTER(ctypes.c_double), ctypes.c_void_p,
+                                    ctypes.c_size_t, ctypes.c_void_p, ctypes.c_void_p]),
+    "ysb_match_compact": (ctypes.c_int, [ctypes.POINTER(YsbMatchStep), ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+                                         ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p,
+                                         ctypes.c_int64, ctypes.c_void_p]),
     "ysb_gather_buffer_bytes": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                                ctypes.POINTER(ctypes.c_size_t)]),
     "ysb_gather_alloc": (ctypes.c_int, [ctypes.c_size_t, ctypes.POINTER(ctypes.c_void_p), ctypes.c_char_p]),

@@ -1,6 +1,6 @@
 """Loader of the thin PyTorch C++ extension (csrc/torch_adapter.cpp -> _lib/libysb_torch.so, TORCH_LIBRARY namespace
 ``ysb``): the binding the hot entry points go through -- torch.ops.ysb.postprocess / filter_candidates / select_nms /
-decode / decode_into / nms / pairwise_iou(_backward) / elementwise_iou(_backward).
+decode / decode_into / nms / pairwise_iou(_backward) / elementwise_iou(_backward) / match_tp / match_compact.
 
 The extension checks tensors, picks torch's current stream on the tensors' device, allocates outputs from the caching
 allocator and raises the reference's exception types; the arithmetic lives in libysb_postproc.so behind the C ABI

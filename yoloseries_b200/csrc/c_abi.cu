@@ -51,6 +51,11 @@ cudaError_t launch_map_iou(const void *b1, int64_t n, int w1, const void *b2, in
                            cudaStream_t stream);
 cudaError_t launch_compute_tp(const void *gt, const int64_t *gt_off, const void *pred, const int64_t *pred_off, int batch,
                               int f64, const double *thr10, int32_t *first_pred, uint8_t *tp, cudaStream_t stream);
+cudaError_t launch_match_tp(const ysb_match_step &s, const double *thr10, int32_t *first_pred, uint8_t *tp,
+                            cudaStream_t stream);
+cudaError_t launch_match_compact(const ysb_match_step &s, const uint8_t *tp, const int64_t *acc_in, int64_t *acc_out,
+                                 float *conf, float *pred_cls, uint8_t *tp_out, int64_t row_cap, double *target_cls,
+                                 int64_t target_cap, cudaStream_t stream);
 cudaError_t launch_pairwise_iou_backward(const float *b1, int64_t n, const float *b2, int64_t m, const float *grad_out,
                                          float *g1, float *g2, cudaStream_t stream);
 cudaError_t launch_soft_nms(const float *boxes, const float *scores, int64_t m, float thr, int kind, int mode, float sigma,
@@ -846,6 +851,64 @@ int ysb_compute_tp(const void *d_gt, const int64_t *d_gt_offsets, int64_t total_
         if (!(iou_thresholds[t] == iou_thresholds[t])) return YSB_ERR_BAD_ARG;
     return cuda_status(launch_compute_tp(d_gt, d_gt_offsets, d_pred, d_pred_offsets, batch, is_f64 != 0, iou_thresholds,
                                          static_cast<int32_t *>(d_workspace), d_tp, static_cast<cudaStream_t>(stream)));
+}
+
+// The block description of a match step; every refusal of ysb_match_tp / ysb_match_compact except their own pointers.
+static int match_step_status(const ysb_match_step *s)
+{
+    if (!s) return YSB_ERR_BAD_ARG;
+    if (s->world < 1 || s->world > YSB_MAX_PEERS || s->batch < 0 || s->max_det < 0 || s->max_gt < 0) return YSB_ERR_BAD_ARG;
+    if (s->gt_dtype != YSB_F32 && s->gt_dtype != YSB_F64) return YSB_ERR_BAD_ARG;
+    if (s->max_det > YSB_MAX_DET_LIMIT) return YSB_ERR_LIMIT;
+    if (static_cast<int64_t>(s->world) * s->batch * s->max_gt > 0x7fffffffll) return YSB_ERR_LIMIT;   // first_pred index
+    if (s->batch == 0) return YSB_OK;
+    if (!s->d_rows || !s->d_cnt || !s->d_gt_cnt || (s->max_gt > 0 && !s->d_gt)) return YSB_ERR_BAD_ARG;
+    if (s->rows_rank_bytes < static_cast<int64_t>(s->batch) * s->max_det * 6 * static_cast<int64_t>(sizeof(float)) ||
+        s->cnt_rank_bytes < static_cast<int64_t>(s->batch) * static_cast<int64_t>(sizeof(int32_t)))
+        return YSB_ERR_BAD_ARG;
+    return YSB_OK;
+}
+
+static size_t match_workspace_bytes(const ysb_match_step *s)
+{
+    const size_t slots = static_cast<size_t>(s->world) * static_cast<size_t>(s->batch) * static_cast<size_t>(s->max_gt);
+    return sizeof(int32_t) * (slots > 0 ? slots : 1);
+}
+
+int ysb_match_tp_workspace_bytes(const ysb_match_step *step, size_t *bytes_out)
+{
+    const int st = match_step_status(step);
+    if (st != YSB_OK) return st;
+    if (!bytes_out) return YSB_ERR_BAD_ARG;
+    *bytes_out = match_workspace_bytes(step);
+    return YSB_OK;
+}
+
+int ysb_match_tp(const ysb_match_step *step, const double *iou_thresholds, void *d_workspace, size_t workspace_bytes,
+                 uint8_t *d_tp, void *stream)
+{
+    const int st = match_step_status(step);
+    if (st != YSB_OK) return st;
+    if (!iou_thresholds) return YSB_ERR_BAD_ARG;
+    for (int t = 0; t < 10; ++t)
+        if (!(iou_thresholds[t] == iou_thresholds[t])) return YSB_ERR_BAD_ARG;
+    if (step->batch == 0) return YSB_OK;
+    if (!d_tp) return YSB_ERR_BAD_ARG;
+    if (!d_workspace || workspace_bytes < match_workspace_bytes(step)) return YSB_ERR_WORKSPACE;
+    return cuda_status(launch_match_tp(*step, iou_thresholds, static_cast<int32_t *>(d_workspace), d_tp,
+                                       static_cast<cudaStream_t>(stream)));
+}
+
+int ysb_match_compact(const ysb_match_step *step, const uint8_t *d_tp, const int64_t *d_acc_in, int64_t *d_acc_out,
+                      float *d_conf, float *d_pred_cls, uint8_t *d_tp_out, int64_t row_capacity, double *d_target_cls,
+                      int64_t target_capacity, void *stream)
+{
+    const int st = match_step_status(step);
+    if (st != YSB_OK) return st;
+    if (!d_acc_in || !d_acc_out || d_acc_in == d_acc_out || row_capacity < 0 || target_capacity < 0) return YSB_ERR_BAD_ARG;
+    if (step->batch > 0 && (!d_tp || !d_conf || !d_pred_cls || !d_tp_out || !d_target_cls)) return YSB_ERR_BAD_ARG;
+    return cuda_status(launch_match_compact(*step, d_tp, d_acc_in, d_acc_out, d_conf, d_pred_cls, d_tp_out, row_capacity,
+                                            d_target_cls, target_capacity, static_cast<cudaStream_t>(stream)));
 }
 
 int ysb_soft_nms(const float *d_boxes, const float *d_scores, int64_t m, float iou_thr, int iou_kind, int mode,

@@ -1,5 +1,6 @@
 // eval_kernels.cu -- the consumers right after the kept rows (SURVEY.md 8f "next" rows):
-//   * mAP_v2.compute_tp and its pairwise IoU        utils/mAP.py:18-42, 70-100   (k_compute_tp, k_map_iou)
+//   * mAP_v2.compute_tp and its pairwise IoU        utils/mAP.py:18-42, 70-100   (k_compute_tp, k_map_iou; k_match_tp
+//                                                   and k_match_compact on the post-processors' own row blocks)
 //   * weighted-box-fusion                           utils/weighted_fusion_bbox.py:41-96, trainer/eval_yolov5.py:44-92
 //                                                   (k_wbf)
 // Small, latency-bound problems (<= max_det predictions x a few dozen ground-truth boxes per image; a few thousand boxes
@@ -13,13 +14,14 @@ namespace ysb {
 // ---- utils/mAP.py:18-42 ------------------------------------------------------------------------------------------------
 // numpy, in the arrays' own precision T: areas = w*h, inter = max(0, .) * max(0, .), iou = inter / clip(a1 + a2 - inter,
 // 1e-6, 1e7).  a = ground truth row (x1, y1, x2, y2, ...), b = prediction row.
-template <typename T>
-__device__ __forceinline__ T map_iou(const T *a, const T *b)
+// B: element type of b's storage, widened exactly to T on load (float32 rows against float64 ground truth).
+template <typename T, typename B = T>
+__device__ __forceinline__ T map_iou(const T *a, const B *b)
 {
     const T a1 = (a[2] - a[0]) * (a[3] - a[1]);
-    const T a2 = (b[2] - b[0]) * (b[3] - b[1]);
-    const T xmin = a[0] > b[0] ? a[0] : b[0], ymin = a[1] > b[1] ? a[1] : b[1];   // np.maximum / np.minimum
-    const T xmax = a[2] < b[2] ? a[2] : b[2], ymax = a[3] < b[3] ? a[3] : b[3];
+    const T a2 = (T(b[2]) - T(b[0])) * (T(b[3]) - T(b[1]));
+    const T xmin = a[0] > T(b[0]) ? a[0] : T(b[0]), ymin = a[1] > T(b[1]) ? a[1] : T(b[1]);   // np.maximum / np.minimum
+    const T xmax = a[2] < T(b[2]) ? a[2] : T(b[2]), ymax = a[3] < T(b[3]) ? a[3] : T(b[3]);
     T w = xmax - xmin, h = ymax - ymin;
     w = w > T(0) ? w : T(0);
     h = h > T(0) ? h : T(0);
@@ -46,15 +48,16 @@ struct TpThresholds {
 // The best ground-truth box of prediction j under the reference's ordering (utils/mAP.py:88-96): pairs with
 // iou >= thr[0] and equal label, sorted by IoU descending; np.unique(pred) keeps the first pair of every prediction.
 // Equal IoUs: argsort()[::-1] of a stable sort visits the LATER pair first, i.e. the larger ground-truth index.
-template <typename T>
-__device__ __forceinline__ int best_gt(const T *gt, int n, const T *p, double thr0, T &best_iou)
+// P: element type of the prediction rows (T, or float32 rows widened to float64).
+template <typename T, typename P>
+__device__ __forceinline__ int best_gt(const T *gt, int n, const P *p, double thr0, T &best_iou)
 {
     int bi = -1;
     T bv = T(0);
     for (int i = 0; i < n; ++i) {
         const T *g = gt + static_cast<int64_t>(i) * 5;
-        const T v = map_iou<T>(g, p);
-        if (static_cast<double>(v) >= thr0 && g[4] == p[5] && (bi < 0 || v >= bv)) {
+        const T v = map_iou<T, P>(g, p);
+        if (static_cast<double>(v) >= thr0 && g[4] == static_cast<T>(p[5]) && (bi < 0 || v >= bv)) {
             bi = i;
             bv = v;
         }
@@ -63,12 +66,40 @@ __device__ __forceinline__ int best_gt(const T *gt, int n, const T *p, double th
     return bi;
 }
 
-// One CTA per image.  gt rows (x1, y1, x2, y2, cls), pred rows (x1, y1, x2, y2, score, cls); images are concatenated,
-// gt_off / pred_off (batch + 1) are row offsets.  first_pred: one int per ground-truth row (workspace).
+// The matching of one image, run by one CTA.  Its n ground-truth rows (x1, y1, x2, y2, cls) are gt[g0 ..], its m kept
+// rows (x1, y1, x2, y2, score, cls) pred[p0 ..], its tp rows (10 bytes) tp[t0 ..]; first_pred[g0 ..]: one int per
+// ground-truth row (workspace).
 //   phase 1: every prediction finds its best ground-truth box and bids for it with atomicMin(pred index): the second
 //            np.unique (over the ground-truth column of the pred-ordered list) keeps the LOWEST prediction index of
 //            every ground-truth box -- not the highest IoU; that is the reference's behaviour and it is kept.
 //   phase 2: the winning prediction of every ground-truth box gets tp[j, t] = iou >= thr[t] (float64 comparison).
+// The kernels below differ only in where an image's rows live (the addressing); all of them match through this body.
+template <typename T, typename P>
+__device__ __forceinline__ void match_image(const T *__restrict__ gt, int64_t g0, int n, const P *__restrict__ pred,
+                                            int64_t p0, int m, const TpThresholds &thr, int32_t *__restrict__ first_pred,
+                                            uint8_t *__restrict__ tp, int64_t t0)
+{
+    for (int i = threadIdx.x; i < n; i += blockDim.x) first_pred[g0 + i] = INT_MAX;
+    for (int e = threadIdx.x; e < m * 10; e += blockDim.x) tp[t0 * 10 + e] = 0;
+    __syncthreads();
+    const T *g = gt + g0 * 5;
+    for (int j = threadIdx.x; j < m; j += blockDim.x) {
+        T v;
+        const int bi = best_gt<T, P>(g, n, pred + (p0 + j) * 6, thr.v[0], v);
+        if (bi >= 0) atomicMin(first_pred + g0 + bi, j);
+    }
+    __syncthreads();
+    for (int j = threadIdx.x; j < m; j += blockDim.x) {
+        T v;
+        const int bi = best_gt<T, P>(g, n, pred + (p0 + j) * 6, thr.v[0], v);
+        if (bi >= 0 && first_pred[g0 + bi] == j) {
+#pragma unroll
+            for (int t = 0; t < 10; ++t) tp[(t0 + j) * 10 + t] = static_cast<double>(v) >= thr.v[t] ? 1 : 0;
+        }
+    }
+}
+
+// ysb_compute_tp: one CTA per image; images are concatenated, gt_off / pred_off (batch + 1) are row offsets.
 template <typename T>
 __global__ void __launch_bounds__(256) k_compute_tp(const T *__restrict__ gt, const int64_t *__restrict__ gt_off,
                                                     const T *__restrict__ pred, const int64_t *__restrict__ pred_off,
@@ -78,23 +109,108 @@ __global__ void __launch_bounds__(256) k_compute_tp(const T *__restrict__ gt, co
     const int img = blockIdx.x;
     const int64_t g0 = gt_off[img], p0 = pred_off[img];
     const int n = static_cast<int>(gt_off[img + 1] - g0), m = static_cast<int>(pred_off[img + 1] - p0);
-    for (int i = threadIdx.x; i < n; i += blockDim.x) first_pred[g0 + i] = INT_MAX;
-    for (int e = threadIdx.x; e < m * 10; e += blockDim.x) tp[p0 * 10 + e] = 0;
+    match_image<T, T>(gt, g0, n, pred, p0, m, thr, first_pred, tp, p0);
+}
+
+// ---- matching in the post-processors' own layouts (ysb_match_tp, ysb_match_compact) ---------------------------------
+// Image k = rank * batch + i of a step.  Rows and counts of a rank start rows_rank_bytes / cnt_rank_bytes after those
+// of the previous one (the 256-byte padded regions of a gather slot); ground truth and its counts are dense.
+__device__ __forceinline__ int step_count(const ysb_match_step &s, int k)
+{
+    const int r = k / s.batch, i = k - r * s.batch;
+    return reinterpret_cast<const int32_t *>(reinterpret_cast<const unsigned char *>(s.d_cnt) + r * s.cnt_rank_bytes)[i];
+}
+
+__device__ __forceinline__ const float *step_rows(const ysb_match_step &s, int k)
+{
+    const int r = k / s.batch, i = k - r * s.batch;
+    return reinterpret_cast<const float *>(reinterpret_cast<const unsigned char *>(s.d_rows) + r * s.rows_rank_bytes) +
+           static_cast<int64_t>(i) * s.max_det * 6;
+}
+
+// rows of image k that take part (a count of -1 -- the reference's None -- has none; absent images are not asked)
+__device__ __forceinline__ int step_preds(const ysb_match_step &s, int c) { return c < 0 ? 0 : (c < s.max_det ? c : s.max_det); }
+
+__device__ __forceinline__ int step_targets(const ysb_match_step &s, int k)
+{
+    const int n = s.d_gt_cnt[k];
+    return n < 0 ? 0 : (n < s.max_gt ? n : s.max_gt);
+}
+
+// One CTA per image of the step; absent images (YSB_CNT_ABSENT) keep their tp rows.  Rows are float32 and are widened
+// to T (the ground truth's type) on load, as ysb_compute_tp matches float32 rows promoted to float64.
+template <typename T>
+__global__ void __launch_bounds__(256) k_match_tp(const __grid_constant__ ysb_match_step s,
+                                                  const __grid_constant__ TpThresholds thr, int32_t *__restrict__ first_pred,
+                                                  uint8_t *__restrict__ tp)
+{
+    const int k = blockIdx.x;
+    const int c = step_count(s, k);
+    if (c == YSB_CNT_ABSENT) return;
+    match_image<T, float>(static_cast<const T *>(s.d_gt), static_cast<int64_t>(k) * s.max_gt, step_targets(s, k),
+                          step_rows(s, k), 0, step_preds(s, c), thr, first_pred, tp, static_cast<int64_t>(k) * s.max_det);
+}
+
+// The sum over the CTA of one value per thread (blockDim.x a multiple of 32, <= 1024).
+__device__ __forceinline__ long long block_sum(long long v, long long *red)
+{
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
     __syncthreads();
-    const T *g = gt + g0 * 5;
-    for (int j = threadIdx.x; j < m; j += blockDim.x) {
-        T v;
-        const int bi = best_gt<T>(g, n, pred + (p0 + j) * 6, thr.v[0], v);
-        if (bi >= 0) atomicMin(first_pred + g0 + bi, j);
+    long long t = 0;
+    for (int w = 0; w < static_cast<int>(blockDim.x >> 5); ++w) t += red[w];
+    __syncthreads();
+    return t;
+}
+
+// One CTA per image of the step: its place among the step's present images (a prefix sum over the counts before it),
+// then a scatter of its kept rows' score, class and tp row and of its targets' classes after what earlier steps
+// appended (acc_in = {rows, targets} so far).  The last CTA writes acc_in + the step's totals to acc_out.  Writes beyond
+// the capacities are dropped; the totals still count them.
+template <typename T>
+__global__ void __launch_bounds__(256) k_match_compact(const __grid_constant__ ysb_match_step s, const uint8_t *__restrict__ tp,
+                                                       const long long *__restrict__ acc_in, long long *__restrict__ acc_out,
+                                                       float *__restrict__ conf, float *__restrict__ pred_cls,
+                                                       uint8_t *__restrict__ tp_out, long long row_cap,
+                                                       double *__restrict__ target_cls, long long target_cap)
+{
+    __shared__ long long red[2][32];
+    const int k = blockIdx.x;
+    long long rows = 0, tgts = 0;
+    for (int q = threadIdx.x; q < k; q += blockDim.x) {
+        const int c = step_count(s, q);
+        if (c == YSB_CNT_ABSENT) continue;
+        rows += step_preds(s, c);
+        tgts += step_targets(s, q);
     }
-    __syncthreads();
+    rows = block_sum(rows, red[0]);
+    tgts = block_sum(tgts, red[1]);
+    const int c = step_count(s, k);
+    const bool present = c != YSB_CNT_ABSENT;
+    const int m = present ? step_preds(s, c) : 0, n = present ? step_targets(s, k) : 0;
+    const long long r0 = acc_in[0] + rows, g0 = acc_in[1] + tgts;
+    if (k == static_cast<int>(gridDim.x) - 1 && threadIdx.x == 0) {
+        acc_out[0] = r0 + m;
+        acc_out[1] = g0 + n;
+    }
+    const float *pr = step_rows(s, k);
+    const uint8_t *t = tp + static_cast<int64_t>(k) * s.max_det * 10;
     for (int j = threadIdx.x; j < m; j += blockDim.x) {
-        T v;
-        const int bi = best_gt<T>(g, n, pred + (p0 + j) * 6, thr.v[0], v);
-        if (bi >= 0 && first_pred[g0 + bi] == j) {
-#pragma unroll
-            for (int t = 0; t < 10; ++t) tp[(p0 + j) * 10 + t] = static_cast<double>(v) >= thr.v[t] ? 1 : 0;
-        }
+        const long long at = r0 + j;
+        if (at >= row_cap) break;
+        conf[at] = pr[j * 6 + 4];
+        pred_cls[at] = pr[j * 6 + 5];
+    }
+    for (int e = threadIdx.x; e < m * 10; e += blockDim.x) {
+        const long long at = r0 * 10 + e;
+        if (at >= row_cap * 10) break;
+        tp_out[at] = t[e];
+    }
+    const T *g = static_cast<const T *>(s.d_gt) + static_cast<int64_t>(k) * s.max_gt * 5;
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+        const long long at = g0 + i;
+        if (at >= target_cap) break;
+        target_cls[at] = static_cast<double>(g[static_cast<int64_t>(i) * 5 + 4]);
     }
 }
 
@@ -129,6 +245,37 @@ cudaError_t launch_compute_tp(const void *gt, const int64_t *gt_off, const void 
     else
         k_compute_tp<float><<<batch, 256, 0, stream>>>(static_cast<const float *>(gt), gt_off,
                                                        static_cast<const float *>(pred), pred_off, t, first_pred, tp);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_match_tp(const ysb_match_step &s, const double *thr10, int32_t *first_pred, uint8_t *tp,
+                            cudaStream_t stream)
+{
+    const int images = s.world * s.batch;
+    if (images == 0) return cudaSuccess;
+    TpThresholds t;
+    for (int i = 0; i < 10; ++i) t.v[i] = thr10[i];
+    if (s.gt_dtype == YSB_F64)
+        k_match_tp<double><<<images, 256, 0, stream>>>(s, t, first_pred, tp);
+    else
+        k_match_tp<float><<<images, 256, 0, stream>>>(s, t, first_pred, tp);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_match_compact(const ysb_match_step &s, const uint8_t *tp, const int64_t *acc_in, int64_t *acc_out,
+                                 float *conf, float *pred_cls, uint8_t *tp_out, int64_t row_cap, double *target_cls,
+                                 int64_t target_cap, cudaStream_t stream)
+{
+    const int images = s.world * s.batch;
+    if (images == 0) return cudaMemcpyAsync(acc_out, acc_in, 2 * sizeof(int64_t), cudaMemcpyDeviceToDevice, stream);
+    const long long *ai = reinterpret_cast<const long long *>(acc_in);
+    long long *ao = reinterpret_cast<long long *>(acc_out);
+    if (s.gt_dtype == YSB_F64)
+        k_match_compact<double><<<images, 256, 0, stream>>>(s, tp, ai, ao, conf, pred_cls, tp_out, row_cap, target_cls,
+                                                            target_cap);
+    else
+        k_match_compact<float><<<images, 256, 0, stream>>>(s, tp, ai, ao, conf, pred_cls, tp_out, row_cap, target_cls,
+                                                           target_cap);
     return cudaGetLastError();
 }
 

@@ -305,6 +305,88 @@ std::tuple<at::Tensor, at::Tensor> elementwise_iou_backward(const at::Tensor &b1
     return {g1, g2};
 }
 
+// ---- mAP hand-off on the post-processors' row blocks (ysb_match_tp, ysb_match_compact) -----------------------------------
+// rows (world, batch, max_det, 6) float32 whose ranks may lie any distance apart (a gather slot), dense within a rank;
+// counts (world, batch) int32 likewise; ground truth (world, batch, max_gt, 5) float32 / float64 and its counts dense.
+ysb_match_step match_step(const at::Tensor &rows, const at::Tensor &cnt, const at::Tensor &gt, const at::Tensor &gt_cnt)
+{
+    const c10::Device dev = rows.device();
+    check_cuda(rows, at::kFloat, dev, "rows", false);
+    check_cuda(cnt, at::kInt, dev, "counts", false);
+    TORCH_CHECK_VALUE(gt.is_cuda() && gt.device() == dev && gt.is_contiguous() &&
+                          (gt.scalar_type() == at::kFloat || gt.scalar_type() == at::kDouble),
+                      "gt: expected a contiguous float32 or float64 CUDA tensor on the rows' device");
+    check_cuda(gt_cnt, at::kInt, dev, "gt_counts");
+    TORCH_CHECK_VALUE(rows.dim() == 4 && rows.size(3) == 6, "rows must be (world, batch, max_det, 6)");
+    const int64_t W = rows.size(0), B = rows.size(1), D = rows.size(2);
+    TORCH_CHECK_VALUE((B == 0 || D == 0 || (rows.stride(3) == 1 && rows.stride(2) == 6 && rows.stride(1) == D * 6)) &&
+                          (W == 1 || rows.stride(0) >= B * D * 6),
+                      "rows: every rank's (batch, max_det, 6) rows must be dense");
+    TORCH_CHECK_VALUE(cnt.dim() == 2 && cnt.size(0) == W && cnt.size(1) == B && (B <= 1 || cnt.stride(1) == 1) &&
+                          (W == 1 || cnt.stride(0) >= B),
+                      "counts must be (world, batch) with every rank's counts dense");
+    TORCH_CHECK_VALUE(gt.dim() == 4 && gt.size(0) == W && gt.size(1) == B && gt.size(3) == 5,
+                      "gt must be (world, batch, max_gt, 5)");
+    TORCH_CHECK_VALUE(gt_cnt.dim() == 2 && gt_cnt.size(0) == W && gt_cnt.size(1) == B, "gt_counts must be (world, batch)");
+    ysb_match_step s{};
+    s.world = static_cast<int32_t>(W);
+    s.batch = static_cast<int32_t>(B);
+    s.max_det = static_cast<int32_t>(D);
+    s.max_gt = static_cast<int32_t>(gt.size(2));
+    s.d_rows = rows.data_ptr<float>();
+    s.rows_rank_bytes = (W == 1 ? B * D * 6 : rows.stride(0)) * static_cast<int64_t>(sizeof(float));
+    s.d_cnt = cnt.data_ptr<int32_t>();
+    s.cnt_rank_bytes = (W == 1 ? B : cnt.stride(0)) * static_cast<int64_t>(sizeof(int32_t));
+    s.d_gt = gt.data_ptr();
+    s.d_gt_cnt = gt_cnt.data_ptr<int32_t>();
+    s.gt_dtype = gt.scalar_type() == at::kDouble ? YSB_F64 : YSB_F32;
+    return s;
+}
+
+void match_tp(const at::Tensor &rows, const at::Tensor &cnt, const at::Tensor &gt, const at::Tensor &gt_cnt,
+              at::ArrayRef<double> iou_thr, at::Tensor tp)
+{
+    const ysb_match_step s = match_step(rows, cnt, gt, gt_cnt);
+    const c10::Device dev = rows.device();
+    check_cuda(tp, at::kByte, dev, "tp");
+    TORCH_CHECK_VALUE(tp.dim() == 4 && tp.size(0) == s.world && tp.size(1) == s.batch && tp.size(2) == s.max_det &&
+                          tp.size(3) == 10,
+                      "tp must be (world, batch, max_det, 10) uint8");
+    TORCH_CHECK_VALUE(iou_thr.size() == 10, "iou_thr must hold 10 thresholds");
+    c10::cuda::CUDAGuard guard(dev);
+    size_t ws_bytes = 0;
+    check_status(ysb_match_tp_workspace_bytes(&s, &ws_bytes), "ysb_match_tp_workspace_bytes");
+    at::Tensor ws = at::empty({static_cast<int64_t>(ws_bytes)}, at::TensorOptions().dtype(at::kByte).device(dev));
+    check_status(ysb_match_tp(&s, iou_thr.data(), ws.data_ptr(), ws_bytes, tp.data_ptr<uint8_t>(), current_stream(dev)),
+                 "ysb_match_tp");
+}
+
+void match_compact(const at::Tensor &rows, const at::Tensor &cnt, const at::Tensor &gt, const at::Tensor &gt_cnt,
+                   const at::Tensor &tp, const at::Tensor &acc_in, at::Tensor acc_out, at::Tensor conf, at::Tensor pred_cls,
+                   at::Tensor tp_out, at::Tensor target_cls)
+{
+    const ysb_match_step s = match_step(rows, cnt, gt, gt_cnt);
+    const c10::Device dev = rows.device();
+    check_cuda(tp, at::kByte, dev, "tp");
+    TORCH_CHECK_VALUE(tp.numel() == static_cast<int64_t>(s.world) * s.batch * s.max_det * 10,
+                      "tp must be (world, batch, max_det, 10) uint8");
+    check_cuda(acc_in, at::kLong, dev, "acc_in");
+    check_cuda(acc_out, at::kLong, dev, "acc_out");
+    TORCH_CHECK_VALUE(acc_in.numel() == 2 && acc_out.numel() == 2, "acc_in / acc_out must hold 2 int64 each");
+    check_cuda(conf, at::kFloat, dev, "conf");
+    check_cuda(pred_cls, at::kFloat, dev, "pred_cls");
+    check_cuda(tp_out, at::kByte, dev, "tp_out");
+    check_cuda(target_cls, at::kDouble, dev, "target_cls");
+    const int64_t cap = conf.numel();
+    TORCH_CHECK_VALUE(pred_cls.numel() == cap && tp_out.numel() == cap * 10,
+                      "conf, pred_cls (P,) and tp_out (P, 10) must share one capacity");
+    c10::cuda::CUDAGuard guard(dev);
+    check_status(ysb_match_compact(&s, tp.data_ptr<uint8_t>(), acc_in.data_ptr<int64_t>(), acc_out.data_ptr<int64_t>(),
+                                   conf.data_ptr<float>(), pred_cls.data_ptr<float>(), tp_out.data_ptr<uint8_t>(), cap,
+                                   target_cls.data_ptr<double>(), target_cls.numel(), current_stream(dev)),
+                 "ysb_match_compact");
+}
+
 int64_t abi_version() { return ysb_abi_version(); }
 int64_t params_bytes() { return static_cast<int64_t>(sizeof(ysb_params)); }
 
@@ -326,6 +408,11 @@ TORCH_LIBRARY(ysb, m)
     m.def("elementwise_iou(Tensor bbox1, Tensor bbox2, int kind) -> Tensor", &elementwise_iou);
     m.def("elementwise_iou_backward(Tensor bbox1, Tensor bbox2, int kind, Tensor grad_out, bool need1, bool need2) -> "
           "(Tensor, Tensor)", &elementwise_iou_backward);
+    m.def("match_tp(Tensor rows, Tensor counts, Tensor gt, Tensor gt_counts, float[] iou_thr, Tensor(a!) tp) -> ()",
+          &match_tp);
+    m.def("match_compact(Tensor rows, Tensor counts, Tensor gt, Tensor gt_counts, Tensor tp, Tensor acc_in, "
+          "Tensor(a!) acc_out, Tensor(b!) conf, Tensor(c!) pred_cls, Tensor(d!) tp_out, Tensor(e!) target_cls) -> ()",
+          &match_compact);
     m.def("abi_version() -> int", &abi_version);
     m.def("params_bytes() -> int", &params_bytes);
 }

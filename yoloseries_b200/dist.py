@@ -246,15 +246,25 @@ class ShardedPostProcessor:
         lo, hi = shard_bounds(len(tail), rank, world)                  # the last, short step
         t = spp.submit([h[lo:hi] for h in heads], info=info[lo:hi], partial=True)   # hi - lo may be 0
 
-    Lanes, graphs and the gather work as for ``submit``.  The first submission fixes the kind (plain or TTA): a processor
+    Lanes, graphs and the gather work as for ``submit``.
+
+    Matching against ground truth for mAP (mAP_v2.compute_tp, val_yolov5.py:388) runs where the rows landed: ``match``
+    enqueues it on the lane after the gather, and every rank matches all world*batch images of the step, so no ground
+    truth or tp crosses ranks (each rank holds the dataset's labels, as YOLO datasets do):
+
+        m = spp.match(t, targets)              # targets: one (n_i, 5) array per image, in result() order
+        stats.add(m)                           # utils.mAP.MatchStats: the run's tp / conf / pred_cls / target_cls
+
+    The first submission fixes the kind (plain or TTA): a processor
     takes only ``submit`` or only ``submit_tta`` calls.  For TTA it also fixes the number of passes, each pass's
     (img_h, img_w, scale, flip_axis) and the head shapes, and sizes the key buffers to the passes' summed key slots; a
     later submission that differs raises ValueError.
     """
 
     def __init__(self, family, hyp, batch, img_h, img_w, anchors=None, lanes=None, group=None, gather="auto", graph=None,
-                 compute_metric=False, device=None):
-        from .engine import PostProcessor
+                 compute_metric=False, device=None, max_targets=1024):
+        from .engine import PostProcessor, check_max_targets
+        self.max_targets = check_max_targets(max_targets)
         self.family, self.batch, self.img_h, self.img_w = family, int(batch), int(img_h), int(img_w)
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         self.group = group
@@ -592,6 +602,30 @@ class ShardedPostProcessor:
                 if c != _lib.YSB_CNT_ABSENT:
                     out.append(None if c < 0 else rows_h[r, i, :c].clone())
         return out
+
+    def match(self, ticket, targets, iou_thr=None):
+        """mAP_v2.compute_tp for every image of the step, on the gathered rows, enqueued on the ticket's lane after the
+        rows of every rank have landed (outside any captured graph).  ``targets``: one (n_i, 5) array or tensor per
+        image (x1, y1, x2, y2, cls; float32 or float64, one type per step, at most ``max_targets`` rows), in ``result()``
+        order, in the pixels of the rows.  Returns engine.Matches (tp (world, batch, max_det, 10) on the device) for
+        utils.mAP.MatchStats.add; no host wait -- except after a partial step (fewer arrays than world * batch), where
+        which images are absent is read back from the gathered counts once.  Raises ValueError for a wrong count of
+        arrays, a wrong shape or dtype, mixed dtypes, or more than ``max_targets`` rows in an image."""
+        from .engine import StepMatcher
+        sl = self._slots[ticket]
+        images = self.world * self.batch
+        if len(targets) == images:
+            positions = range(images)
+        elif len(targets) > images:
+            raise ValueError(f"need one target array per image of the step: {len(targets)} > {images}")
+        else:
+            sl["done"].synchronize()
+            cnt = sl["cnt"].cpu().reshape(-1).tolist()
+            positions = [k for k, c in enumerate(cnt) if c != _lib.YSB_CNT_ABSENT]
+        with torch.cuda.device(self.device), torch.cuda.stream(self.streams[ticket]):
+            if "matcher" not in sl:
+                sl["matcher"] = StepMatcher(self.world, self.batch, self.max_det, self.max_targets, self.device)
+            return sl["matcher"].run(sl["rows"], sl["cnt"], targets, positions, iou_thr)
 
     def drain(self):
         """The caller's current stream waits for everything submitted so far."""

@@ -268,6 +268,126 @@ class LetterboxStaging:
         self.table.copy_(self.host, non_blocking=True)
 
 
+# ---- mAP hand-off: ground truth matched against the kept rows where they are (ysb_match_tp) -----------------------------
+MATCH_DTYPES = (np.float32, np.float64)   # ground-truth element types the match kernel reads (one per step)
+
+
+def _target_array(t, i):
+    a = t.detach().cpu().numpy() if isinstance(t, torch.Tensor) else np.asarray(t)
+    if a.size == 0:
+        return a.reshape(0, 5)
+    if a.ndim != 2 or a.shape[1] != 5:
+        raise ValueError(f"targets[{i}]: expected an (n, 5) array (x1, y1, x2, y2, cls), got shape {a.shape}")
+    if a.dtype not in MATCH_DTYPES:
+        raise ValueError(f"targets[{i}]: expected float32 or float64, got {a.dtype}")
+    return a
+
+
+def pack_targets(targets, positions, images, capacity):
+    """Host half of ``match``: one (n_i, 5) ground-truth array or tensor per image of a step, in ``result()`` order, ->
+    (arrays, dtype, max_n): image ``positions[i]`` of the step's ``images`` (rank * batch + image) receives
+    ``targets[i]``.  dtype is the step's one element type (float32 or float64; empty arrays take any), max_n its largest
+    count (at least 1), the padded stride of the block the kernel reads.  Raises ValueError for a wrong count of arrays,
+    a wrong shape or dtype, mixed dtypes, or more than ``capacity`` rows in one image."""
+    if len(targets) != len(positions):
+        raise ValueError(f"need one target array per image of the step: {len(targets)} != {len(positions)}")
+    arrs = [_target_array(t, i) for i, t in enumerate(targets)]
+    for i, a in enumerate(arrs):
+        if a.shape[0] > capacity:
+            raise ValueError(f"targets[{i}] has {a.shape[0]} boxes, more than the processor's max_targets = {capacity}")
+    dtypes = {a.dtype for a in arrs if a.shape[0]}
+    if len(dtypes) > 1:
+        raise ValueError(f"every target array of a step must have one dtype, got {sorted(map(str, dtypes))}")
+    if any(not 0 <= k < images for k in positions):
+        raise ValueError(f"image positions outside 0..{images - 1}")
+    dtype = np.dtype(dtypes.pop() if dtypes else np.float32)
+    max_n = max([1] + [a.shape[0] for a in arrs])
+    return arrs, dtype, max_n
+
+
+class TargetStaging:
+    """The padded ground truth of one lane's ``match``: a pinned host buffer and a device buffer holding the (images)
+    int32 counts followed by the (images, max_n, 5) rows, uploaded with one cudaMemcpyAsync on the current stream (the
+    lane's), so the upload never makes the host wait for the lane's earlier work.  Both grow (powers of two) to the
+    largest step seen; a step's max_n is its largest count, so a COCO step uploads tens of KB."""
+
+    def __init__(self, images, device):
+        self.images, self.device = int(images), torch.device(device)
+        self._cnt_bytes = (4 * self.images + 15) // 16 * 16
+        self._host = self._dev = None
+        self._copied = None   # event after the last copy out of the pinned buffer
+
+    def stage(self, arrs, positions, dtype, max_n):
+        """Fill the buffer and enqueue its upload; returns device views (gt (images, max_n, 5), counts (images,))."""
+        nbytes = self._cnt_bytes + self.images * max_n * 5 * dtype.itemsize
+        if self._copied is not None:
+            self._copied.synchronize()   # the previous upload may still be queued behind the lane's earlier work
+        if self._host is None or self._host.numel() < nbytes:
+            size = 1 << max(12, (nbytes - 1).bit_length())
+            self._host = torch.empty(size, dtype=torch.uint8, pin_memory=True)
+            self._dev = torch.empty(size, dtype=torch.uint8, device=self.device)
+        raw = self._host.numpy()
+        cnt = raw[:4 * self.images].view(np.int32)
+        cnt[:] = 0
+        vals = raw[self._cnt_bytes:nbytes].view(dtype).reshape(self.images, max_n, 5)
+        for k, a in zip(positions, arrs):
+            cnt[k] = a.shape[0]
+            vals[k, :a.shape[0]] = a
+        self._dev[:nbytes].copy_(self._host[:nbytes], non_blocking=True)
+        self._copied = torch.cuda.Event()
+        self._copied.record(torch.cuda.current_stream(self.device))
+        gt = self._dev[self._cnt_bytes:nbytes].view(torch.float64 if dtype == np.float64 else torch.float32)
+        return gt.view(self.images, max_n, 5), self._dev[:4 * self.images].view(torch.int32)
+
+
+class Matches:
+    """What ``match`` enqueued for one step, all device tensors ordered on ``stream`` (the lane's): the step's rows
+    (world, batch, max_det, 6) and counts (world, batch) as the processor keeps them, the staged ground truth
+    (world, batch, max_n, 5) and its counts, and ``tp`` (world, batch, max_det, 10) uint8 -- the reference's bool matrix
+    of every present image, aligned with its rows (world = 1 for PostProcessor and PipelinedPostProcessor).  Valid until
+    the lane's buffers are reused, like the ticket.  MatchStats.add appends it to a run's arrays."""
+
+    def __init__(self, rows, cnt, gt, gt_cnt, tp, stream, n_targets):
+        self.rows, self.cnt, self.gt, self.gt_cnt, self.tp = rows, cnt, gt, gt_cnt, tp
+        self.stream, self.n_targets = stream, n_targets
+
+    def to_list(self):
+        """Host copy: list over the step's present images in ``result()`` order of (K, 10) bool arrays (K = 0 for the
+        reference's None).  Synchronises the lane."""
+        self.stream.synchronize()
+        cnt = self.cnt.cpu().reshape(-1).tolist()
+        tp = self.tp.cpu().numpy().reshape(len(cnt), self.tp.shape[2], 10).astype(bool)
+        return [tp[k, :max(c, 0)] for k, c in enumerate(cnt) if c != _lib.YSB_CNT_ABSENT]
+
+
+class StepMatcher:
+    """The device state of ``match`` for one output buffer (a PostProcessor entry, a pipeline lane, a gather slot):
+    the ground-truth staging and the tp rows.  Construct and run it under the buffer's stream."""
+
+    def __init__(self, world, batch, max_det, capacity, device):
+        self.world, self.batch, self.capacity = int(world), int(batch), int(capacity)
+        self.staging = TargetStaging(self.world * self.batch, device)
+        self.tp = torch.empty((self.world, self.batch, int(max_det), 10), dtype=torch.uint8, device=device)
+
+    def run(self, rows, cnt, targets, positions, iou_thr=None):
+        from .utils.mAP import IOU_THRESHOLDS
+        thr = [float(v) for v in np.asarray(IOU_THRESHOLDS if iou_thr is None else iou_thr, dtype=np.float64).reshape(-1)]
+        if len(thr) != 10:
+            raise ValueError("iou_thr must hold 10 thresholds (np.linspace(0.5, 0.95, 10) in the reference)")
+        arrs, dtype, max_n = pack_targets(targets, positions, self.world * self.batch, self.capacity)
+        gt, gt_cnt = self.staging.stage(arrs, positions, dtype, max_n)
+        gt, gt_cnt = gt.view(self.world, self.batch, max_n, 5), gt_cnt.view(self.world, self.batch)
+        _ops.load().match_tp(rows, cnt, gt, gt_cnt, thr, self.tp)
+        return Matches(rows, cnt, gt, gt_cnt, self.tp, torch.cuda.current_stream(self.tp.device),
+                       sum(a.shape[0] for a in arrs))
+
+
+def check_max_targets(max_targets):
+    if int(max_targets) < 1:
+        raise ValueError(f"max_targets must be at least 1, got {max_targets}")
+    return int(max_targets)
+
+
 class DetectionList(list):
     """The evaluator's output list (CPU rows, the reference's contract) that also remembers the device rows it was read
     from, so that preds_postprocess can map them without staging them back to the GPU."""
@@ -394,15 +514,18 @@ class DetectionBuffers:
         self.dets = torch.empty((batch, max_det, 6), dtype=torch.float32, device=device)
         self.det_idx = torch.empty((batch, max_det), dtype=torch.int32, device=device)
         self.det_cnt = torch.empty((batch,), dtype=torch.int32, device=device)
+        self.matcher = None   # StepMatcher of PostProcessor.match, made on first use
 
 
 class PostProcessor:
     """decode -> filter -> top-k -> class-aware NMS -> post-filter for one family / one head geometry.
 
     Buffers are allocated once per (batch, geometry) and reused; every call enqueues on torch's current stream.
+    ``max_targets``: ground-truth boxes per image that ``match`` accepts.
     """
 
-    def __init__(self, family, hyp, anchors=None, compute_metric=False):
+    def __init__(self, family, hyp, anchors=None, compute_metric=False, max_targets=1024):
+        self.max_targets = check_max_targets(max_targets)
         self.family = family
         self.hyp = dict(hyp)
         self.anchors = anchors
@@ -626,6 +749,18 @@ class PostProcessor:
                        "ysb_undo_letterbox")
         return out
 
+    def match(self, out, targets, iou_thr=None):
+        """mAP_v2.compute_tp for every image of a ``run`` / ``run_tta`` output, on the device rows, in one launch on the
+        current stream: ``targets`` holds one (n_i, 5) array or tensor (x1, y1, x2, y2, cls; float32 or float64, one
+        type per call, at most ``max_targets`` rows) per image.  Float32 ground truth matches in float32, float64 in
+        float64 -- bit for bit what utils.mAP.compute_tp_batch returns for the images' rows.  Returns Matches (tp on
+        the device, for MatchStats.add); its buffers are reused by the next match on the same output."""
+        b, dev = out.dets.shape[0], out.dets.device
+        with torch.cuda.device(dev):
+            if out.matcher is None:
+                out.matcher = StepMatcher(1, b, out.dets.shape[1], self.max_targets, dev)
+            return out.matcher.run(out.dets.unsqueeze(0), out.det_cnt.unsqueeze(0), targets, range(b), iou_thr)
+
     @staticmethod
     def to_list(out, as_numpy=False, with_index=False):
         """DetectionBuffers -> the reference's output contract: list of CPU float32 (K, 6) tensors or None."""
@@ -661,10 +796,12 @@ class PipelinedPostProcessor:
     A ticket's buffers are reused ``lanes`` submissions later: fetch results before submitting that many new batches.
     With ``info`` (as for PostProcessor.run) a batch's rows come out in original-picture pixels; each lane uploads its
     own letterbox table on its stream (LetterboxStaging).
+
+        m = ppp.match(t, targets)        # tp of the batch on the device, on its lane; MatchStats.add(m) accumulates
     """
 
-    def __init__(self, family, hyp, anchors=None, compute_metric=False, lanes=4):
-        self._pps = [PostProcessor(family, hyp, anchors, compute_metric) for _ in range(lanes)]
+    def __init__(self, family, hyp, anchors=None, compute_metric=False, lanes=4, max_targets=1024):
+        self._pps = [PostProcessor(family, hyp, anchors, compute_metric, max_targets) for _ in range(lanes)]
         self._streams = None
         self._done = [None] * lanes   # per lane: the event recorded after its last batch
         self._next = 0
@@ -713,3 +850,10 @@ class PipelinedPostProcessor:
         done.synchronize()
         with torch.cuda.stream(self._streams[i]):
             return PostProcessor.to_list(out, as_numpy=as_numpy, with_index=with_index)
+
+    def match(self, ticket, targets, iou_thr=None):
+        """PostProcessor.match for a submitted batch, enqueued on its lane after its rows: ``targets`` holds one (n_i, 5)
+        array per image, in ``result()`` order.  Returns Matches; no host wait."""
+        i, _, out = ticket
+        with torch.cuda.stream(self._streams[i]):
+            return self._pps[i].match(out, targets, iou_thr)

@@ -3,6 +3,7 @@
     iou(box1, box2)                     utils/mAP.py:18-42   (M,4), (N,4) ndarrays -> (M,N), the arrays' own precision
     compute_tp(gt, pred)                utils/mAP.py:70-100  (N,5), (M,6) ndarrays -> (M,10) bool
     compute_tp_batch(gts, preds)        the loop of utils/mAP.py:102-108 (compute_ap_per_class) as ONE launch
+    MatchStats                          that loop's outputs accumulated on the device from the post-processors' match()
 
 The AP integration / plotting half of mAP_v2 is bookkeeping on a few thousand numbers and stays with the caller;
 dropin.install() rebinds ``mAP_v2.compute_tp`` so the reference's class keeps working unchanged.  Compute runs in
@@ -13,10 +14,10 @@ import ctypes
 import numpy as np
 import torch
 
-from .. import _lib
+from .. import _lib, _ops
 from ._common import cuda_device, stream_ptr
 
-__all__ = ["iou", "compute_tp", "compute_tp_batch", "IOU_THRESHOLDS"]
+__all__ = ["iou", "compute_tp", "compute_tp_batch", "MatchStats", "IOU_THRESHOLDS"]
 
 IOU_THRESHOLDS = np.linspace(0.5, 0.95, 10)   # mAP_v2.__init__, utils/mAP.py:64
 
@@ -82,6 +83,80 @@ def compute_tp_batch(gts, preds, iou_thr=None):
 def compute_tp(gt, pred, iou_thr=None):
     """mAP_v2.compute_tp(gt, pred), utils/mAP.py:70-100 -> (M, 10) bool."""
     return compute_tp_batch([gt], [pred], iou_thr)[0]
+
+
+class MatchStats:
+    """The per-image results of a validation run's matching, accumulated on the device: ``add`` appends a step's
+    ``match`` result (PostProcessor, PipelinedPostProcessor or dist.ShardedPostProcessor) with one launch on the step's
+    lane (ysb_match_compact), and ``arrays`` returns, at the end, what the AP integration of mAP_v2 consumes:
+
+        tp (P, 10) bool, conf (P,) float32, pred_cls (P,) float32, target_cls (G,) float64
+
+    equal to concatenating compute_tp(gt_i, pred_i), pred_i[:, 4], pred_i[:, 5] and gt_i[:, 4] over the images in the
+    order ``result()`` lists them, step after step in ``add`` order (absent images of a partial step are skipped; an
+    image whose rows are None adds its targets only).  AP sorts by confidence, so that order matters for equal scores.
+    Storage grows with the rows the steps could hold (world * batch * max_det per step), without a host wait."""
+
+    def __init__(self):
+        self.device = None
+        self._acc = None       # (2, 2) int64: {rows, targets} so far, ping-pong between the steps
+        self._cur = 0
+        self._rows_bound = self._targets = 0
+        self._buf = None       # conf, pred_cls, tp (cap, 10), target_cls (cap_t)
+        self._last = None      # event after the last compaction
+
+    def _grow(self, rows, targets, dev, st):
+        cap_r = self._buf[0].numel() if self._buf else 0
+        cap_t = self._buf[3].numel() if self._buf else 0
+        if self._buf is not None and rows <= cap_r and targets <= cap_t:
+            return
+        new_r, new_t = max(rows, 2 * cap_r, 4096), max(targets, 2 * cap_t, 4096)
+        buf = (torch.empty(new_r, dtype=torch.float32, device=dev), torch.empty(new_r, dtype=torch.float32, device=dev),
+               torch.empty((new_r, 10), dtype=torch.uint8, device=dev), torch.empty(new_t, dtype=torch.float64, device=dev))
+        if self._buf is not None:
+            for new, old in zip(buf, self._buf):
+                new[:old.shape[0]].copy_(old)
+                old.record_stream(st)
+        self._buf = buf
+
+    def add(self, matches):
+        """Append one step (engine.Matches); enqueued on its lane after the previous add, no host wait."""
+        st = matches.stream
+        dev = matches.tp.device
+        if self.device is None:
+            self.device = dev
+            with torch.cuda.device(dev), torch.cuda.stream(st):
+                self._acc = torch.zeros((2, 2), dtype=torch.int64, device=dev)
+        elif dev != self.device:
+            raise ValueError(f"this MatchStats accumulates on {self.device}, got matches on {dev}")
+        with torch.cuda.device(dev), torch.cuda.stream(st):
+            if self._last is not None:
+                st.wait_event(self._last)
+            w, b, d = matches.tp.shape[:3]
+            self._rows_bound += w * b * d
+            self._targets += matches.n_targets
+            self._grow(self._rows_bound, self._targets, dev, st)
+            conf, cls, tp, tcls = self._buf
+            _ops.load().match_compact(matches.rows, matches.cnt, matches.gt, matches.gt_cnt, matches.tp,
+                                      self._acc[self._cur], self._acc[1 - self._cur], conf, cls, tp, tcls)
+            self._cur = 1 - self._cur
+            for t in (self._acc, *self._buf):   # used on several lanes: freed only after this one's work
+                t.record_stream(st)
+            self._last = torch.cuda.Event()
+            self._last.record(st)
+
+    def arrays(self):
+        """(tp (P, 10) bool, conf (P,) float32, pred_cls (P,) float32, target_cls (G,) float64) on the host."""
+        if self._last is None:
+            return (np.zeros((0, 10), dtype=bool), np.zeros(0, dtype=np.float32), np.zeros(0, dtype=np.float32),
+                    np.zeros(0, dtype=np.float64))
+        with torch.cuda.device(self.device):
+            cur = torch.cuda.current_stream(self.device)
+            cur.wait_event(self._last)
+            p, g = self._acc[self._cur].cpu().tolist()
+            conf, cls, tp, tcls = self._buf
+            return (tp[:p].cpu().numpy().astype(bool), conf[:p].cpu().numpy(), cls[:p].cpu().numpy(),
+                    tcls[:g].cpu().numpy())
 
 
 def _compute_tp_method(self, gt, pred):
